@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the Bi-Mamba backend hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 Workload at N = 1 is BASELINE.json configs[1]: the 4-layer Bi-Mamba backend (4 x
 PN_BiMambas_Encoder, d_model 144, d_state 16) fwd + bwd (+ AdamW step), 201 frames, batch 64,
@@ -15,6 +15,11 @@ public API with the step's input coming from pinned HOST memory and the loss rea
 every step.  `--impl reference` times the CPU oracle port of the reference's own path
 (oracle/bimamba_oracle.py; the reference is a Python package whose /root/reference tree does not
 exist on the GPU box) on all host threads.
+
+`--dump-outputs DIR` writes what the last device-timed training step handed back to its caller, as
+DIR/<name>.npy: `loss` (float64) and, for every backbone parameter, `param.<name>` (after that step's
+AdamW update) and `grad.<name>` (the gradient it applied), float32, about 10 MB in all.  Inputs and
+weights are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -30,6 +35,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True     # the benchmark may run from a read-only tree; it writes nothing into it
 
 import torch  # noqa: E402
 
@@ -58,7 +64,14 @@ def parse():
     ap.add_argument("--comm", default="overlap", choices=["overlap", "graph", "eager"],
                     help="N > 1: gradient all-reduce per encoder layer inside the step graph, overlapping the remaining "
                          "backward (default); one all-reduce inside the graph; or launched after the graph (round 1)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write the loss, parameters and gradients of the last timed step as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
+    return args
 
 
 def workload_config(args, world):
@@ -124,7 +137,7 @@ def run_reference(args, rank, world):
     step = oracle_step_fn(sample_batch, args.frames)
     for _ in range(max(1, min(args.warmup, 2))):
         step()
-    steps = max(1, min(args.steps, 30))           # each step is ~2-4 s of CPU work on 8-16 threads
+    steps = args.steps
     t0 = time.perf_counter()
     for _ in range(steps):
         step()
@@ -237,6 +250,19 @@ def load_peaks():
         with open(path) as f:
             return json.load(f).get("hbm_gbs", 6650.0), "measured (MEASURED_PEAKS.json hbm_gbs)"
     return 6650.0, "fallback (B200_PROFILING.md 6.65 TB/s)"
+
+
+def dump_step_outputs(directory, model, loss):
+    """What a caller of the training step holds once it returns: the loss, every backbone parameter after the AdamW
+    update and the gradient that update applied."""
+    import numpy as np
+    out = {"loss": loss.detach().double().cpu().numpy()}
+    for name, p in model.backbone_layers.named_parameters(prefix="backbone_layers"):
+        out["param." + name] = p.detach().float().cpu().numpy()
+        out["grad." + name] = p.grad.detach().float().cpu().numpy()
+    os.makedirs(directory, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
 
 
 def scan_bytes(frames, ndir, esize, backward):
@@ -465,11 +491,13 @@ def run_ours(args, rank, world, local_rank):
     for s, e in evs:
         flush.zero_()
         s.record()
-        step()
+        loss = step()
         e.record()
     barrier()
     w1 = time.perf_counter()
     dev_ms = sum(s.elapsed_time(e) for s, e in evs)
+    if rank == 0 and args.dump_outputs:
+        dump_step_outputs(args.dump_outputs, model, loss)
 
     # ---- end to end: pinned host input -> H2D -> step -> loss.item() every step ----
     pipelined = use_graph and (world == 1 or args.comm != "eager")
