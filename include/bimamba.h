@@ -28,6 +28,9 @@
  *   bimamba_block_fwd/bwd            <- the whole block, both directions, one call each way
  *                                       (mamba_block.py:41-63 + DualStreamSEMamba.py:473-481)
  *
+ *   bimamba_*_fwd_varlen              <- scoring of right-padded batches of utterances of different lengths
+ *                                       (per-utterance frame counts; see "Variable-length scoring" below)
+ *
  * Ownership: the library never allocates or frees device memory.  All tensors and
  * workspaces are caller-allocated; pointers are borrowed for the duration of the
  * enqueue.  Calls only enqueue work on `stream` (no device sync, CUDA-graph safe).
@@ -44,7 +47,7 @@
 extern "C" {
 #endif
 
-#define BIMAMBA_ABI_VERSION 11
+#define BIMAMBA_ABI_VERSION 12
 
 /* element types of activation operands */
 #define BIMAMBA_F32 0
@@ -146,6 +149,15 @@ int bimamba_scan_plan(int seqlen, int dim, int rows, int backward, int* group_ch
 int bimamba_selective_scan_fwd(const bimamba_scan_desc* d, bimamba_stream_t stream);
 int bimamba_selective_scan_bwd(const bimamba_scan_desc* d, bimamba_stream_t stream);
 
+/* ---- Variable-length scoring.  `seqlens` is a DEVICE pointer to `batch` int32 frame counts: utterance b is frames
+ * 0 .. seqlens[b]-1 of a right-padded batch of `seqlen` frames, and every valid output equals what the utterance gives
+ * when it runs alone at its own length.  Kernels clamp seqlens[b] to [0, seqlen]; frames at or past it are never read
+ * by the conv, the scan or the head, so the padding may hold anything (NaN included).  Outputs a call owns per frame
+ * (conv out, scan out / ypre) are written as zeros at padded frames; a zero-length utterance yields zeros.  A NULL
+ * seqlens is the fixed-length call: bimamba_X(...) is bimamba_X_varlen(..., NULL, ...).  Forward only: the scan rejects
+ * checkpoints (d->ckpt != NULL) and the block / layer reject save_for_backward != 0 with a negative code. */
+int bimamba_selective_scan_fwd_varlen(const bimamba_scan_desc* d, const int32_t* seqlens, bimamba_stream_t stream);
+
 /* Time-parallel forward scan for long sequences at small batches (the scan as an associative operator on pairs,
  * (a2, b2) o (a1, b1) = (a2 a1, a2 b1 + b2); mamba_block.py:92-117 is the serial loop).  Scan time is cut into nseg
  * segments of seg_len steps: a carry pass computes every segment's end state from zero and its decay exponent
@@ -168,6 +180,11 @@ int bimamba_causal_conv1d_fwd(const void* x, const float* weight, const float* b
                               int batch, int ndir, int dim, int seqlen, int width,
                               int64_t x_bs, int64_t x_ts, int64_t out_bs, int64_t out_ds, int64_t out_ts,
                               int dtype, int flags, bimamba_stream_t stream);
+/* Per-utterance frame counts (see bimamba_selective_scan_fwd_varlen): dir 1's taps t + k >= seqlens[b] read as zero. */
+int bimamba_causal_conv1d_fwd_varlen(const void* x, const float* weight, const float* bias, void* out,
+                                     const int32_t* seqlens, int batch, int ndir, int dim, int seqlen, int width,
+                                     int64_t x_bs, int64_t x_ts, int64_t out_bs, int64_t out_ds, int64_t out_ts,
+                                     int dtype, int flags, bimamba_stream_t stream);
 
 /* dout: (batch, ndir, L, dim) grads w.r.t. the conv output of each direction.
  * dx: (batch, L, dim), summed over directions.  dz_in (optional, may be NULL): per-direction
@@ -207,6 +224,12 @@ int bimamba_gemm_tn(const void* A, int64_t lda, const void* B, int64_t ldb, floa
 int bimamba_head_fwd(const void* x, const float* gamma, const float* beta, const float* w_att, const float* b_att,
                      const float* w_cls, const float* b_cls, float* features, float* logits, int batch, int seqlen,
                      int channels, int nclasses, float eps, int dtype, bimamba_stream_t stream);
+/* Per-utterance frame counts (see bimamba_selective_scan_fwd_varlen): norm, softmax and pooling over t < seqlens[b];
+ * a zero-length utterance gets zero features and logits = b_cls. */
+int bimamba_head_fwd_varlen(const void* x, const float* gamma, const float* beta, const float* w_att, const float* b_att,
+                            const float* w_cls, const float* b_cls, float* features, float* logits,
+                            const int32_t* seqlens, int batch, int seqlen, int channels, int nclasses, float eps,
+                            int dtype, bimamba_stream_t stream);
 
 /* Backward of the pooled features of bimamba_head_fwd (the training head: norm_f + attention pooling under autograd,
  * DualStreamSEMamba.py:759-763; call bimamba_head_fwd with nclasses = 0 for the forward - dropout and the classifier
@@ -382,6 +405,9 @@ size_t bimamba_block_fwd_workspace_bytes(int batch, int seqlen, int d_model, int
 size_t bimamba_block_bwd_workspace_bytes(int batch, int seqlen, int d_model, int d_inner, int d_conv, int ndir,
                                          int io_dtype);
 int bimamba_block_fwd(const bimamba_block_desc* d, bimamba_stream_t stream);
+/* Per-utterance frame counts (see bimamba_selective_scan_fwd_varlen); d->save_for_backward must be 0.  Output rows at
+ * padded frames are unspecified. */
+int bimamba_block_fwd_varlen(const bimamba_block_desc* d, const int32_t* seqlens, bimamba_stream_t stream);
 /* `d` is the descriptor the forward ran with (same workspace, save_for_backward != 0). */
 int bimamba_block_bwd(const bimamba_block_desc* d, const bimamba_block_grads* g, bimamba_stream_t stream);
 
@@ -431,6 +457,9 @@ size_t bimamba_layer_fwd_workspace_bytes(int batch, int seqlen, int d_model, int
 size_t bimamba_layer_bwd_workspace_bytes(int batch, int seqlen, int d_model, int d_inner, int d_ff, int d_conv, int ndir,
                                          int io_dtype);
 int bimamba_layer_fwd(const bimamba_layer_desc* d, bimamba_stream_t stream);
+/* Per-utterance frame counts (see bimamba_selective_scan_fwd_varlen); d->block.save_for_backward must be 0.  Output
+ * rows at padded frames are unspecified. */
+int bimamba_layer_fwd_varlen(const bimamba_layer_desc* d, const int32_t* seqlens, bimamba_stream_t stream);
 int bimamba_layer_bwd(const bimamba_layer_desc* d, const bimamba_layer_grads* g, bimamba_stream_t stream);
 
 #ifdef __cplusplus

@@ -16,7 +16,7 @@ F32, BF16, F16 = 0, 1, 2
 FLAG_SOFTPLUS = 1
 FLAG_DTR_PADDED = 2
 FLAG_SILU = 1
-ABI_VERSION = 11
+ABI_VERSION = 12
 CHUNK = 16
 
 EXPORTS = (
@@ -30,6 +30,8 @@ EXPORTS = (
     "bimamba_scan_fwd_split_plan", "bimamba_scan_fwd_split_workspace_bytes", "bimamba_selective_scan_fwd_split",
     "bimamba_block_fwd_workspace_bytes", "bimamba_block_bwd_workspace_bytes", "bimamba_block_fwd", "bimamba_block_bwd",
     "bimamba_layer_fwd_workspace_bytes", "bimamba_layer_bwd_workspace_bytes", "bimamba_layer_fwd", "bimamba_layer_bwd",
+    "bimamba_causal_conv1d_fwd_varlen", "bimamba_selective_scan_fwd_varlen", "bimamba_head_fwd_varlen",
+    "bimamba_block_fwd_varlen", "bimamba_layer_fwd_varlen",
 )
 
 
@@ -125,6 +127,11 @@ def load() -> C.CDLL:
         lib.bimamba_causal_conv1d_fwd.restype = i32
         lib.bimamba_causal_conv1d_fwd.argtypes = [vp, vp, vp, vp, i32, i32, i32, i32, i32,
                                                   i64, i64, i64, i64, i64, i32, i32, vp]
+        lib.bimamba_selective_scan_fwd_varlen.restype = i32
+        lib.bimamba_selective_scan_fwd_varlen.argtypes = [C.POINTER(ScanDesc), vp, vp]
+        lib.bimamba_causal_conv1d_fwd_varlen.restype = i32
+        lib.bimamba_causal_conv1d_fwd_varlen.argtypes = [vp, vp, vp, vp, vp, i32, i32, i32, i32, i32,
+                                                         i64, i64, i64, i64, i64, i32, i32, vp]
         lib.bimamba_causal_conv1d_bwd.restype = i32
         lib.bimamba_causal_conv1d_bwd.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, i32, i32, i32, i32, i32,
                                                   i64, i64, i64, i64, i64, i64, i64, i32, i32, vp]
@@ -153,6 +160,8 @@ def load() -> C.CDLL:
         lib.bimamba_gemm_nt_block_n_k.argtypes = [i32, i32]
         lib.bimamba_head_fwd.restype = i32
         lib.bimamba_head_fwd.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, vp, i32, i32, i32, i32, C.c_float, i32, vp]
+        lib.bimamba_head_fwd_varlen.restype = i32
+        lib.bimamba_head_fwd_varlen.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, i32, i32, i32, i32, C.c_float, i32, vp]
         lib.bimamba_adamw_chunk.restype = i32
         lib.bimamba_adamw_chunk.argtypes = []
         lib.bimamba_adamw_step.restype = i32
@@ -197,6 +206,8 @@ def load() -> C.CDLL:
         lib.bimamba_block_bwd_workspace_bytes.argtypes = [i32] * 7
         lib.bimamba_block_fwd.restype = i32
         lib.bimamba_block_fwd.argtypes = [C.POINTER(BlockDesc), vp]
+        lib.bimamba_block_fwd_varlen.restype = i32
+        lib.bimamba_block_fwd_varlen.argtypes = [C.POINTER(BlockDesc), vp, vp]
         lib.bimamba_block_bwd.restype = i32
         lib.bimamba_block_bwd.argtypes = [C.POINTER(BlockDesc), C.POINTER(BlockGrads), vp]
         lib.bimamba_scan_fwd_split_plan.restype = i32
@@ -211,6 +222,8 @@ def load() -> C.CDLL:
         lib.bimamba_layer_bwd_workspace_bytes.argtypes = [i32] * 8
         lib.bimamba_layer_fwd.restype = i32
         lib.bimamba_layer_fwd.argtypes = [C.POINTER(LayerDesc), vp]
+        lib.bimamba_layer_fwd_varlen.restype = i32
+        lib.bimamba_layer_fwd_varlen.argtypes = [C.POINTER(LayerDesc), vp, vp]
         lib.bimamba_layer_bwd.restype = i32
         lib.bimamba_layer_bwd.argtypes = [C.POINTER(LayerDesc), C.POINTER(LayerGrads), vp]
         got = lib.bimamba_abi_version()

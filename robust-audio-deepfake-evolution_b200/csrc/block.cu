@@ -140,6 +140,17 @@ extern "C" size_t bimamba_block_bwd_workspace_bytes(int batch, int seqlen, int d
 }
 
 extern "C" int bimamba_block_fwd(const bimamba_block_desc* d, bimamba_stream_t stream) {
+  return bimamba_block_fwd_varlen(d, nullptr, stream);
+}
+
+// seqlens != NULL: scoring of right-padded utterances of different lengths.  The products run on every row (a row of a
+// product depends on that row only); the conv and the scan walk each utterance's own frames and write zeros to the
+// padded ones, so valid outputs do not depend on what the padding holds.
+extern "C" int bimamba_block_fwd_varlen(const bimamba_block_desc* d, const int32_t* seqlens, bimamba_stream_t stream) {
+  if (d && seqlens && d->save_for_backward) {
+    set_err("block_fwd_varlen: variable-length batches are forward-only (save_for_backward must be 0)");
+    return -9;
+  }
   int rc = check_block(d);
   if (rc) return rc;
   if (d->batch == 0 || d->seqlen == 0) return 0;
@@ -155,8 +166,8 @@ extern "C" int bimamba_block_fwd(const bimamba_block_desc* d, bimamba_stream_t s
   rc = bimamba_gemm_nt(d->x, dm, d->Wi, dm, xz, 2 * D, nullptr, nullptr, M, 2 * D, dm, dt, dt, stream);
   if (rc) return rc;
   // causal conv + SiLU of the x half, direction 0 and the flipped direction from one read (:52-55)
-  rc = bimamba_causal_conv1d_fwd(xz, d->conv_w, d->conv_b, xc, (int)B, nd, D, (int)L, d->d_conv, L * 2 * D, 2 * D,
-                                 L * nd * D, D, (int64_t)nd * D, dt, BIMAMBA_FLAG_SILU, stream);
+  rc = bimamba_causal_conv1d_fwd_varlen(xz, d->conv_w, d->conv_b, xc, seqlens, (int)B, nd, D, (int)L, d->d_conv, L * 2 * D,
+                                        2 * D, L * nd * D, D, (int64_t)nd * D, dt, BIMAMBA_FLAG_SILU, stream);
   if (rc) return rc;
   // x_proj against the repacked (48, D) weight: rows [B | C | dt_r | 0] of both directions in one product (:73)
   rc = bimamba_gemm_nt(xc, D, d->Wxp, D, xdbl, kXW, nullptr, nullptr, M * nd, kXW, D, dt, dt, stream);
@@ -170,7 +181,7 @@ extern "C" int bimamba_block_fwd(const bimamba_block_desc* d, bimamba_stream_t s
   int G = 0, ng = 0;
   bimamba_scan_plan((int)L, D, (int)(B * nd), 0, &G, &ng);
   s.group_channels = G;
-  rc = bimamba_selective_scan_fwd(&s, stream);
+  rc = bimamba_selective_scan_fwd_varlen(&s, seqlens, stream);
   if (rc) return rc;
   // out_proj of the sum of the directions as one product over [y_fwd | y_rev] (:62, DualStreamSEMamba.py:481)
   return bimamba_gemm_nt(y, (int64_t)nd * D, d->Wo2, (int64_t)nd * D, d->out, dm, nullptr, nullptr, M, dm, nd * D, dt, dt, stream);
@@ -362,6 +373,16 @@ extern "C" size_t bimamba_layer_bwd_workspace_bytes(int batch, int seqlen, int d
 }
 
 extern "C" int bimamba_layer_fwd(const bimamba_layer_desc* d, bimamba_stream_t stream) {
+  return bimamba_layer_fwd_varlen(d, nullptr, stream);
+}
+
+// seqlens != NULL: the block walks each utterance's own frames (bimamba_block_fwd_varlen); the norms and the feed-forward
+// are per row.
+extern "C" int bimamba_layer_fwd_varlen(const bimamba_layer_desc* d, const int32_t* seqlens, bimamba_stream_t stream) {
+  if (d && seqlens && d->block.save_for_backward) {
+    set_err("layer_fwd_varlen: variable-length batches are forward-only (save_for_backward must be 0)");
+    return -9;
+  }
   int rc = check_layer(d);
   if (rc) return rc;
   bimamba_block_desc k = d->block;
@@ -385,7 +406,7 @@ extern "C" int bimamba_layer_fwd(const bimamba_layer_desc* d, bimamba_stream_t s
   k.out = mo;
   k.workspace = ws + c.block;
   k.workspace_bytes = d->workspace_bytes - c.block;
-  BIMAMBA_TRY(bimamba_block_fwd(&k, stream));
+  BIMAMBA_TRY(bimamba_block_fwd_varlen(&k, seqlens, stream));
   // norm2 (:482)
   BIMAMBA_TRY(bimamba_layernorm_fwd(mo, d->norm2_w, d->norm2_b, mn, mean2, rstd2, M, dm, d->eps2, cd, cd, stream));
   // feed-forward + residual (:483-485): weights cast (and transposed for the backward), two products with the bias and

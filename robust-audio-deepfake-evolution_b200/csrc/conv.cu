@@ -51,11 +51,14 @@ __device__ __forceinline__ float silu_grad(float pre) {
   return sg * (1.f + pre * (1.f - sg));
 }
 
-template <typename T, int V, int K>
+// kVar: per-utterance frame counts (seqlens, clamped to [0, L]).  Frames t >= len_b read as zero - the window is never
+// loaded from them, so whatever the padding holds (NaN included) cannot reach a valid output - and the kernel writes zeros
+// to both directions' padded output frames.
+template <typename T, int V, int K, bool kVar>
 __global__ void __launch_bounds__(kConvThreads)
 conv_fwd_kernel(const T* __restrict__ x, const float* __restrict__ w, const float* __restrict__ bias, T* __restrict__ out,
                 int batch, int ndir, int dim, int L, int64_t x_bs, int64_t x_ts, int64_t o_bs, int64_t o_ds,
-                int64_t o_ts, int silu) {
+                int64_t o_ts, int silu, const int32_t* __restrict__ seqlens) {
   pdl_prologue();
   const int nvec = (dim + V - 1) / V;
   const int nseg = (L + kSeg - 1) / kSeg;
@@ -67,6 +70,7 @@ conv_fwd_kernel(const T* __restrict__ x, const float* __restrict__ w, const floa
   const int b = (int)(gid / ((int64_t)nvec * nseg));
   const int d = v * V, t0 = s * kSeg;
   constexpr int H = K - 1;
+  const int Lv = kVar ? min(max(__ldg(seqlens + b), 0), L) : L;   // frames that exist
 
   float wk[V][K], bs[V];
 #pragma unroll
@@ -81,7 +85,7 @@ conv_fwd_kernel(const T* __restrict__ x, const float* __restrict__ w, const floa
 #pragma unroll
   for (int j = 0; j < 2 * H; ++j) {
     const int t = t0 - H + j;
-    if (t >= 0 && t < L) {
+    if (t >= 0 && t < Lv) {
       load_row<T, V>(xb + (int64_t)t * x_ts, win[j + 1]);
     } else {
 #pragma unroll
@@ -97,7 +101,7 @@ conv_fwd_kernel(const T* __restrict__ x, const float* __restrict__ w, const floa
 #pragma unroll
       for (int i = 0; i < V; ++i) win[j][i] = win[j + 1][i];
     const int tn = t + H;
-    if (tn < L) {
+    if (tn < Lv) {
       load_row<T, V>(xb + (int64_t)tn * x_ts, win[2 * H]);
     } else {
 #pragma unroll
@@ -116,8 +120,8 @@ conv_fwd_kernel(const T* __restrict__ x, const float* __restrict__ w, const floa
         a0 *= sigmoid_f(a0);
         a1 *= sigmoid_f(a1);
       }
-      o0[i] = a0;
-      o1[i] = a1;
+      o0[i] = (kVar && t >= Lv) ? 0.f : a0;
+      o1[i] = (kVar && t >= Lv) ? 0.f : a1;
     }
     T* ob = out + (int64_t)b * o_bs + (int64_t)t * o_ts + d;
     store_row<T, V>(ob, o0);
@@ -466,19 +470,19 @@ conv_bwd_seg_kernel(const T* __restrict__ x, const float* __restrict__ w, const 
 
 static int conv_bwd_time_tiles(int seqlen) { return seqlen > 0 ? (seqlen + kBwdT - 1) / kBwdT : 1; }
 
-template <typename T, int V>
+template <typename T, int V, bool kVar>
 static void launch_conv_fwd(const void* x, const float* w, const float* bias, void* out, int batch, int ndir, int dim,
                             int L, int width, int64_t x_bs, int64_t x_ts, int64_t o_bs, int64_t o_ds, int64_t o_ts,
-                            int silu, cudaStream_t st) {
+                            int silu, const int32_t* seqlens, cudaStream_t st) {
   const int nvec = (dim + V - 1) / V, nseg = (L + kSeg - 1) / kSeg;
   const int64_t total = (int64_t)batch * nseg * nvec;
   const unsigned blocks = (unsigned)((total + kConvThreads - 1) / kConvThreads);
   const T* xp = reinterpret_cast<const T*>(x);
   T* op = reinterpret_cast<T*>(out);
   switch (width) {
-    case 2: launch_k(conv_fwd_kernel<T, V, 2>, blocks, kConvThreads, 0, st, xp, w, bias, op, batch, ndir, dim, L, x_bs, x_ts, o_bs, o_ds, o_ts, silu); break;
-    case 3: launch_k(conv_fwd_kernel<T, V, 3>, blocks, kConvThreads, 0, st, xp, w, bias, op, batch, ndir, dim, L, x_bs, x_ts, o_bs, o_ds, o_ts, silu); break;
-    default: launch_k(conv_fwd_kernel<T, V, 4>, blocks, kConvThreads, 0, st, xp, w, bias, op, batch, ndir, dim, L, x_bs, x_ts, o_bs, o_ds, o_ts, silu); break;
+    case 2: launch_k(conv_fwd_kernel<T, V, 2, kVar>, blocks, kConvThreads, 0, st, xp, w, bias, op, batch, ndir, dim, L, x_bs, x_ts, o_bs, o_ds, o_ts, silu, seqlens); break;
+    case 3: launch_k(conv_fwd_kernel<T, V, 3, kVar>, blocks, kConvThreads, 0, st, xp, w, bias, op, batch, ndir, dim, L, x_bs, x_ts, o_bs, o_ds, o_ts, silu, seqlens); break;
+    default: launch_k(conv_fwd_kernel<T, V, 4, kVar>, blocks, kConvThreads, 0, st, xp, w, bias, op, batch, ndir, dim, L, x_bs, x_ts, o_bs, o_ds, o_ts, silu, seqlens); break;
   }
 }
 
@@ -519,6 +523,14 @@ extern "C" int bimamba_causal_conv1d_fwd(const void* x, const float* weight, con
                                          int ndir, int dim, int seqlen, int width, int64_t x_bs, int64_t x_ts,
                                          int64_t out_bs, int64_t out_ds, int64_t out_ts, int dtype, int flags,
                                          bimamba_stream_t stream) {
+  return bimamba_causal_conv1d_fwd_varlen(x, weight, bias, out, nullptr, batch, ndir, dim, seqlen, width, x_bs, x_ts,
+                                          out_bs, out_ds, out_ts, dtype, flags, stream);
+}
+
+extern "C" int bimamba_causal_conv1d_fwd_varlen(const void* x, const float* weight, const float* bias, void* out,
+                                                const int32_t* seqlens, int batch, int ndir, int dim, int seqlen,
+                                                int width, int64_t x_bs, int64_t x_ts, int64_t out_bs, int64_t out_ds,
+                                                int64_t out_ts, int dtype, int flags, bimamba_stream_t stream) {
   if (batch == 0 || seqlen == 0) return 0;
   if (!x || !weight || !out) { set_err("conv fwd: null operand"); return -1; }
   if (width < 2 || width > kMaxK) { set_err("conv width must be 2, 3 or 4"); return -2; }
@@ -526,7 +538,11 @@ extern "C" int bimamba_causal_conv1d_fwd(const void* x, const float* weight, con
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   const int silu = flags & BIMAMBA_FLAG_SILU;
   const bool v4 = vec4_ok(dtype, dim, {x, out}, {x_bs, x_ts, out_bs, out_ds, out_ts});
-#define CONV_FWD(T, V) launch_conv_fwd<T, V>(x, weight, bias, out, batch, ndir, dim, seqlen, width, x_bs, x_ts, out_bs, out_ds, out_ts, silu, st)
+#define CONV_FWD(T, V)                                                                                                     \
+  do {                                                                                                                     \
+    if (seqlens) launch_conv_fwd<T, V, true>(x, weight, bias, out, batch, ndir, dim, seqlen, width, x_bs, x_ts, out_bs, out_ds, out_ts, silu, seqlens, st); \
+    else launch_conv_fwd<T, V, false>(x, weight, bias, out, batch, ndir, dim, seqlen, width, x_bs, x_ts, out_bs, out_ds, out_ts, silu, nullptr, st); \
+  } while (0)
   if (dtype == BIMAMBA_F32) { if (v4) CONV_FWD(float, 4); else CONV_FWD(float, 1); }
   else if (dtype == BIMAMBA_BF16) { if (v4) CONV_FWD(__nv_bfloat16, 4); else CONV_FWD(__nv_bfloat16, 1); }
   else { if (v4) CONV_FWD(__half, 4); else CONV_FWD(__half, 1); }

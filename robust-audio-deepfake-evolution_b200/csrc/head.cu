@@ -21,12 +21,14 @@ __device__ __forceinline__ float warp_sum_h(float v) {
   return v;
 }
 
-template <typename T, int NPL>
+// kVar: norm, softmax and pooling over the frames t < clamp(seqlens[b], 0, L) only; a zero-length utterance pools to
+// zero features (its logits are the classifier bias).
+template <typename T, int NPL, bool kVar>
 __global__ void __launch_bounds__(kHeadThreads)
 head_fwd_kernel(const T* __restrict__ x, const float* __restrict__ gamma, const float* __restrict__ beta,
                 const float* __restrict__ w_att, const float* __restrict__ b_att, const float* __restrict__ w_cls,
                 const float* __restrict__ b_cls, float* __restrict__ features, float* __restrict__ logits, int L, int C,
-                int ncls, float eps) {
+                int ncls, float eps, const int32_t* __restrict__ seqlens) {
   pdl_prologue();
   __shared__ float s_m[kHeadWarps], s_l[kHeadWarps];
   __shared__ float s_acc[kHeadWarps][32 * NPL];
@@ -44,8 +46,9 @@ head_fwd_kernel(const T* __restrict__ x, const float* __restrict__ gamma, const 
     acc[i] = 0.f;
   }
   const float ba = b_att ? __ldg(b_att) : 0.f;
+  const int Lb = kVar ? min(max(__ldg(seqlens + b), 0), L) : L;
   float m = -INFINITY, l = 0.f;
-  for (int t = warp; t < L; t += kHeadWarps) {
+  for (int t = warp; t < Lb; t += kHeadWarps) {
     const T* xr = xb + (int64_t)t * C;
     float v[NPL];
     float s = 0.f;
@@ -99,7 +102,7 @@ head_fwd_kernel(const T* __restrict__ x, const float* __restrict__ gamma, const 
 #pragma unroll
     for (int w = 0; w < kHeadWarps; ++w)
       num += s_m[w] == -INFINITY ? 0.f : s_acc[w][c] * ex2_approx((s_m[w] - M) * kLog2e);
-    const float f = num / den;
+    const float f = (kVar && !(den > 0.f)) ? 0.f : num / den;
     s_feat[c] = f;
     features[(int64_t)b * C + c] = f;
   }
@@ -272,13 +275,18 @@ head_bwd_kernel(const T* __restrict__ x, const float* __restrict__ gamma, const 
 
 template <typename T>
 static void launch_head(const void* x, const float* gamma, const float* beta, const float* w_att, const float* b_att,
-                        const float* w_cls, const float* b_cls, float* features, float* logits, int batch, int L, int C,
-                        int ncls, float eps, cudaStream_t st) {
+                        const float* w_cls, const float* b_cls, float* features, float* logits, const int32_t* seqlens,
+                        int batch, int L, int C, int ncls, float eps, cudaStream_t st) {
   const T* xp = reinterpret_cast<const T*>(x);
-  if (C <= 160)
-    launch_k(head_fwd_kernel<T, 5>, batch, kHeadThreads, 0, st, xp, gamma, beta, w_att, b_att, w_cls, b_cls, features, logits, L, C, ncls, eps);
-  else
-    launch_k(head_fwd_kernel<T, 8>, batch, kHeadThreads, 0, st, xp, gamma, beta, w_att, b_att, w_cls, b_cls, features, logits, L, C, ncls, eps);
+#define HEAD_FWD(NPL, VAR) launch_k(head_fwd_kernel<T, NPL, VAR>, batch, kHeadThreads, 0, st, xp, gamma, beta, w_att, b_att, w_cls, b_cls, features, logits, L, C, ncls, eps, seqlens)
+  if (C <= 160) {
+    if (seqlens) HEAD_FWD(5, true);
+    else HEAD_FWD(5, false);
+  } else {
+    if (seqlens) HEAD_FWD(8, true);
+    else HEAD_FWD(8, false);
+  }
+#undef HEAD_FWD
 }
 
 }  // namespace bimamba
@@ -289,14 +297,22 @@ extern "C" int bimamba_head_fwd(const void* x, const float* gamma, const float* 
                                 const float* b_att, const float* w_cls, const float* b_cls, float* features,
                                 float* logits, int batch, int seqlen, int channels, int nclasses, float eps, int dtype,
                                 bimamba_stream_t stream) {
+  return bimamba_head_fwd_varlen(x, gamma, beta, w_att, b_att, w_cls, b_cls, features, logits, nullptr, batch, seqlen,
+                                 channels, nclasses, eps, dtype, stream);
+}
+
+extern "C" int bimamba_head_fwd_varlen(const void* x, const float* gamma, const float* beta, const float* w_att,
+                                       const float* b_att, const float* w_cls, const float* b_cls, float* features,
+                                       float* logits, const int32_t* seqlens, int batch, int seqlen, int channels,
+                                       int nclasses, float eps, int dtype, bimamba_stream_t stream) {
   if (batch == 0) return 0;
   if (!x || !gamma || !beta || !w_att || !features || (nclasses > 0 && (!w_cls || !logits))) { set_err("head: null operand"); return -1; }
   if (batch < 0 || seqlen < 1 || channels < 1 || channels > 256 || nclasses < 0) { set_err("head: seqlen >= 1, channels 1..256"); return -3; }
   if (dtype < 0 || dtype > 2) { set_err("head: bad dtype"); return -6; }
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  if (dtype == BIMAMBA_F32) launch_head<float>(x, gamma, beta, w_att, b_att, w_cls, b_cls, features, logits, batch, seqlen, channels, nclasses, eps, st);
-  else if (dtype == BIMAMBA_BF16) launch_head<__nv_bfloat16>(x, gamma, beta, w_att, b_att, w_cls, b_cls, features, logits, batch, seqlen, channels, nclasses, eps, st);
-  else launch_head<__half>(x, gamma, beta, w_att, b_att, w_cls, b_cls, features, logits, batch, seqlen, channels, nclasses, eps, st);
+  if (dtype == BIMAMBA_F32) launch_head<float>(x, gamma, beta, w_att, b_att, w_cls, b_cls, features, logits, seqlens, batch, seqlen, channels, nclasses, eps, st);
+  else if (dtype == BIMAMBA_BF16) launch_head<__nv_bfloat16>(x, gamma, beta, w_att, b_att, w_cls, b_cls, features, logits, seqlens, batch, seqlen, channels, nclasses, eps, st);
+  else launch_head<__half>(x, gamma, beta, w_att, b_att, w_cls, b_cls, features, logits, seqlens, batch, seqlen, channels, nclasses, eps, st);
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) { set_err(cudaGetErrorString(e)); return (int)e; }
   return 0;

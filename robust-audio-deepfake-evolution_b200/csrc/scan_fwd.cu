@@ -33,8 +33,9 @@ namespace bimamba {
 constexpr int kFwdMaxThreads = 128;
 
 // kMode: 0 = delta given; 1 = fused dt projection with dt_rank <= 12; 2 = dt_rank <= 16.
-template <typename T, int kMode, bool kGate>
-__global__ void __launch_bounds__(kFwdMaxThreads) scan_fwd_kernel(const bimamba_scan_desc p) {
+// kVar: per-utterance frame counts, as in scan_fwd_warp_kernel (scan_fwd1.cu).
+template <typename T, int kMode, bool kGate, bool kVar>
+__global__ void __launch_bounds__(kFwdMaxThreads) scan_fwd_kernel(const bimamba_scan_desc p, const int32_t* __restrict__ seqlens) {
   pdl_prologue();
   extern __shared__ __align__(16) unsigned char smem_raw[];
   constexpr bool expl = kMode == 0;
@@ -42,7 +43,8 @@ __global__ void __launch_bounds__(kFwdMaxThreads) scan_fwd_kernel(const bimamba_
   const int G = blockDim.x, tid = threadIdx.x;
   const int b = blockIdx.z, dir = blockIdx.y, d0 = blockIdx.x * G, d = d0 + tid;
   const bool ok = d < p.dim;
-  const int L = p.seqlen, nck = (L + kT - 1) / kT, nckpt = (L + BIMAMBA_CKPT - 1) / BIMAMBA_CKPT;
+  const int L = kVar ? min(max(__ldg(seqlens + b), 0), p.seqlen) : p.seqlen;
+  const int nck = (L + kT - 1) / kT, nckpt = (L + BIMAMBA_CKPT - 1) / BIMAMBA_CKPT;
   const bool softplus = (p.flags & BIMAMBA_FLAG_SOFTPLUS) != 0;
   const int R = expl ? 0 : p.dt_rank;
 
@@ -52,6 +54,13 @@ __global__ void __launch_bounds__(kFwdMaxThreads) scan_fwd_kernel(const bimamba_
   const T* gbc = reinterpret_cast<const T*>(p.bc) + (int64_t)b * p.bc_bs + (int64_t)dir * p.bc_ds;
   const T* gdtr = expl ? nullptr : reinterpret_cast<const T*>(p.dtr) + (int64_t)b * p.dtr_bs + (int64_t)dir * p.dtr_ds;
   const int64_t obase = (int64_t)b * p.out_bs + (int64_t)dir * p.out_ds;
+  if (kVar && ok) {   // padded frames (the variable-length entry takes no checkpoints)
+    for (int t = L; t < p.seqlen; ++t) {
+      const int64_t o = obase + (int64_t)t * p.out_ts + d;
+      reinterpret_cast<T*>(p.out)[o] = from_f<T>(0.f);
+      if (p.ypre) reinterpret_cast<T*>(p.ypre)[o] = from_f<T>(0.f);
+    }
+  }
 
   // shared memory: [2][nact][kT*G] T | [2][kT*kXW] T | [kT*kXW] float
   constexpr int nact = 1 + (kGate ? 1 : 0) + (expl ? 1 : 0);
@@ -198,42 +207,53 @@ static size_t fwd_smem_bytes(int G, int esize, bool has_z, bool expl) {
   return (size_t)2 * nact * kT * G * esize + (size_t)2 * kT * kXW * esize + (size_t)kT * kXW * 4;
 }
 
-template <typename T, int kMode, bool kGate>
-static void launch_fwd2(const bimamba_scan_desc* d, cudaStream_t st) {
+template <typename T, int kMode, bool kGate, bool kVar>
+static void launch_fwd3(const bimamba_scan_desc* d, const int32_t* seqlens, cudaStream_t st) {
   const int G = d->group_channels;
   const size_t smem = fwd_smem_bytes(G, (int)sizeof(T), kGate, kMode == 0);
   dim3 grid((d->dim + G - 1) / G, d->ndir, d->batch);
   if (smem > 48 * 1024)
-    cudaFuncSetAttribute(scan_fwd_kernel<T, kMode, kGate>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  launch_k(scan_fwd_kernel<T, kMode, kGate>, grid, G, smem, st, *d);
+    cudaFuncSetAttribute(scan_fwd_kernel<T, kMode, kGate, kVar>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  launch_k(scan_fwd_kernel<T, kMode, kGate, kVar>, grid, G, smem, st, *d, seqlens);
+}
+
+template <typename T, int kMode, bool kGate>
+static void launch_fwd2(const bimamba_scan_desc* d, const int32_t* seqlens, cudaStream_t st) {
+  if (seqlens) launch_fwd3<T, kMode, kGate, true>(d, seqlens, st);
+  else launch_fwd3<T, kMode, kGate, false>(d, seqlens, st);
 }
 
 template <typename T>
-static void launch_fwd(const bimamba_scan_desc* d, cudaStream_t st) {
+static void launch_fwd(const bimamba_scan_desc* d, const int32_t* seqlens, cudaStream_t st) {
   const bool gate = d->z != nullptr;
   const int mode = d->delta ? 0 : (d->dt_rank <= 12 ? 1 : 2);
   if (gate) {
-    if (mode == 0) launch_fwd2<T, 0, true>(d, st);
-    else if (mode == 1) launch_fwd2<T, 1, true>(d, st);
-    else launch_fwd2<T, 2, true>(d, st);
+    if (mode == 0) launch_fwd2<T, 0, true>(d, seqlens, st);
+    else if (mode == 1) launch_fwd2<T, 1, true>(d, seqlens, st);
+    else launch_fwd2<T, 2, true>(d, seqlens, st);
   } else {
-    if (mode == 0) launch_fwd2<T, 0, false>(d, st);
-    else if (mode == 1) launch_fwd2<T, 1, false>(d, st);
-    else launch_fwd2<T, 2, false>(d, st);
+    if (mode == 0) launch_fwd2<T, 0, false>(d, seqlens, st);
+    else if (mode == 1) launch_fwd2<T, 1, false>(d, seqlens, st);
+    else launch_fwd2<T, 2, false>(d, seqlens, st);
   }
 }
 
 int check_desc(const bimamba_scan_desc* d, bool bwd);  // api.cu
-void launch_fwd_warp(const bimamba_scan_desc* d, cudaStream_t st);  // scan_fwd1.cu
+void launch_fwd_warp(const bimamba_scan_desc* d, const int32_t* seqlens, cudaStream_t st);  // scan_fwd1.cu
 
 }  // namespace bimamba
 
 using namespace bimamba;
 
 extern "C" int bimamba_selective_scan_fwd(const bimamba_scan_desc* d, bimamba_stream_t stream) {
+  return bimamba_selective_scan_fwd_varlen(d, nullptr, stream);
+}
+
+extern "C" int bimamba_selective_scan_fwd_varlen(const bimamba_scan_desc* d, const int32_t* seqlens, bimamba_stream_t stream) {
   if (d && (d->batch == 0 || d->seqlen == 0)) return 0;  // empty: nothing to do (pointers may be null)
   int rc = check_desc(d, false);
   if (rc) return rc;
+  if (seqlens && d->ckpt) { set_err("scan fwd: checkpoints feed the backward, which has no variable-length form"); return -9; }
   const int G = d->group_channels;
   if (G < 32 || G > kFwdMaxThreads || (G & 31)) { set_err("forward group_channels must be 32, 64, 96 or 128 (use bimamba_scan_plan)"); return -5; }
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
@@ -248,12 +268,12 @@ extern "C" int bimamba_selective_scan_fwd(const bimamba_scan_desc* d, bimamba_st
   const int force = g_tune[BIMAMBA_TUNE_SCAN_FWD];
   const int variant = force ? force : ((lanes < (int64_t)148 * 16 * 32 || d->io_dtype == BIMAMBA_F32) ? 3 : 1);
   if (variant == 3) {
-    launch_fwd_warp(d, st);
+    launch_fwd_warp(d, seqlens, st);
   } else {
     switch (d->io_dtype) {
-      case BIMAMBA_F32: launch_fwd<float>(d, st); break;
-      case BIMAMBA_BF16: launch_fwd<__nv_bfloat16>(d, st); break;
-      default: launch_fwd<__half>(d, st); break;
+      case BIMAMBA_F32: launch_fwd<float>(d, seqlens, st); break;
+      case BIMAMBA_BF16: launch_fwd<__nv_bfloat16>(d, seqlens, st); break;
+      default: launch_fwd<__half>(d, seqlens, st); break;
     }
   }
   cudaError_t e = cudaGetLastError();

@@ -10,8 +10,10 @@ namespace bimamba {
 
 constexpr int kF1G = 32;
 
-template <typename T, int kMode, bool kGate>
-__global__ void __launch_bounds__(kF1G) scan_fwd_warp_kernel(const bimamba_scan_desc p) {
+// kVar: utterance b walks its own len_b = clamp(seqlens[b], 0, seqlen) steps (direction 1 starts at len_b - 1) and the
+// padded frames len_b .. seqlen-1 of out (and ypre) are written as zeros.
+template <typename T, int kMode, bool kGate, bool kVar>
+__global__ void __launch_bounds__(kF1G) scan_fwd_warp_kernel(const bimamba_scan_desc p, const int32_t* __restrict__ seqlens) {
   pdl_prologue();
   extern __shared__ __align__(16) unsigned char smem_raw[];
   constexpr bool expl = kMode == 0;
@@ -22,7 +24,8 @@ __global__ void __launch_bounds__(kF1G) scan_fwd_warp_kernel(const bimamba_scan_
   const int tid = threadIdx.x;
   const int b = blockIdx.z, dir = blockIdx.y, d0 = blockIdx.x * G, d = d0 + tid;
   const bool ok = d < p.dim;
-  const int L = p.seqlen, nck = (L + kT - 1) / kT, nckpt = (L + BIMAMBA_CKPT - 1) / BIMAMBA_CKPT;
+  const int L = kVar ? min(max(__ldg(seqlens + b), 0), p.seqlen) : p.seqlen;
+  const int nck = (L + kT - 1) / kT, nckpt = (L + BIMAMBA_CKPT - 1) / BIMAMBA_CKPT;
   const bool softplus = (p.flags & BIMAMBA_FLAG_SOFTPLUS) != 0;
   const int R = expl ? 0 : p.dt_rank;
 
@@ -32,6 +35,13 @@ __global__ void __launch_bounds__(kF1G) scan_fwd_warp_kernel(const bimamba_scan_
   const T* gbc = reinterpret_cast<const T*>(p.bc) + (int64_t)b * p.bc_bs + (int64_t)dir * p.bc_ds;
   const T* gdtr = expl ? nullptr : reinterpret_cast<const T*>(p.dtr) + (int64_t)b * p.dtr_bs + (int64_t)dir * p.dtr_ds;
   const int64_t obase = (int64_t)b * p.out_bs + (int64_t)dir * p.out_ds;
+  if (kVar && ok) {   // padded frames (the variable-length entry takes no checkpoints)
+    for (int t = L; t < p.seqlen; ++t) {
+      const int64_t o = obase + (int64_t)t * p.out_ts + d;
+      reinterpret_cast<T*>(p.out)[o] = from_f<T>(0.f);
+      if (p.ypre) reinterpret_cast<T*>(p.ypre)[o] = from_f<T>(0.f);
+    }
+  }
 
   float* s_xf = reinterpret_cast<float*>(smem_raw);                 // [16][kXW] rows as fp32
   T* s_xr = reinterpret_cast<T*>(s_xf + kT * kXW);                  // [2][16][kXW] rows as staged
@@ -210,33 +220,34 @@ __global__ void __launch_bounds__(kF1G) scan_fwd_warp_kernel(const bimamba_scan_
 }
 
 template <typename T, int kMode, bool kGate>
-static void launch_warp2(const bimamba_scan_desc* d, cudaStream_t st) {
+static void launch_warp2(const bimamba_scan_desc* d, const int32_t* seqlens, cudaStream_t st) {
   const size_t smem = (size_t)kT * kXW * 4 + (size_t)2 * kT * kXW * sizeof(T) + (size_t)2 * 3 * kT * kF1G * sizeof(T);
   dim3 grid((d->dim + kF1G - 1) / kF1G, d->ndir, d->batch);
-  launch_k(scan_fwd_warp_kernel<T, kMode, kGate>, grid, kF1G, smem, st, *d);
+  if (seqlens) launch_k(scan_fwd_warp_kernel<T, kMode, kGate, true>, grid, kF1G, smem, st, *d, seqlens);
+  else launch_k(scan_fwd_warp_kernel<T, kMode, kGate, false>, grid, kF1G, smem, st, *d, seqlens);
 }
 
 template <typename T>
-static void launch_warp(const bimamba_scan_desc* d, cudaStream_t st) {
+static void launch_warp(const bimamba_scan_desc* d, const int32_t* seqlens, cudaStream_t st) {
   const bool gate = d->z != nullptr;
   const int mode = d->delta ? 0 : (d->dt_rank <= 12 ? 1 : 2);
   if (gate) {
-    if (mode == 0) launch_warp2<T, 0, true>(d, st);
-    else if (mode == 1) launch_warp2<T, 1, true>(d, st);
-    else launch_warp2<T, 2, true>(d, st);
+    if (mode == 0) launch_warp2<T, 0, true>(d, seqlens, st);
+    else if (mode == 1) launch_warp2<T, 1, true>(d, seqlens, st);
+    else launch_warp2<T, 2, true>(d, seqlens, st);
   } else {
-    if (mode == 0) launch_warp2<T, 0, false>(d, st);
-    else if (mode == 1) launch_warp2<T, 1, false>(d, st);
-    else launch_warp2<T, 2, false>(d, st);
+    if (mode == 0) launch_warp2<T, 0, false>(d, seqlens, st);
+    else if (mode == 1) launch_warp2<T, 1, false>(d, seqlens, st);
+    else launch_warp2<T, 2, false>(d, seqlens, st);
   }
 }
 
 // group_channels is ignored: this kernel always works on 32-channel groups (the forward has no per-group outputs).
-void launch_fwd_warp(const bimamba_scan_desc* d, cudaStream_t st) {
+void launch_fwd_warp(const bimamba_scan_desc* d, const int32_t* seqlens, cudaStream_t st) {
   switch (d->io_dtype) {
-    case BIMAMBA_F32: launch_warp<float>(d, st); break;
-    case BIMAMBA_BF16: launch_warp<__nv_bfloat16>(d, st); break;
-    default: launch_warp<__half>(d, st); break;
+    case BIMAMBA_F32: launch_warp<float>(d, seqlens, st); break;
+    case BIMAMBA_BF16: launch_warp<__nv_bfloat16>(d, seqlens, st); break;
+    default: launch_warp<__half>(d, seqlens, st); break;
   }
 }
 

@@ -7,7 +7,8 @@ import torch.nn as nn
 import torch.nn.functional as F
 
 from .mamba_simple import Mamba
-from .ops import encoder_layer_native, feed_forward_fn, head_fwd, head_pool_fn, layer_norm_fn, native_layer_ok
+from .ops import (_forward_only, encoder_layer_native, feed_forward_fn, head_fwd, head_pool_fn, layer_norm_fn,
+                  native_layer_ok, seqlens_tensor)
 
 
 class PN_BiMambas_Encoder(nn.Module):
@@ -26,15 +27,21 @@ class PN_BiMambas_Encoder(nn.Module):
             nn.Linear(d_model * 4, d_model),
         )
 
-    def forward(self, x):
+    def forward(self, x, lengths=None):
+        """x (B, T, d_model) -> (B, T, d_model).  lengths (B,) (list, CPU or CUDA tensor; scoring only): per-utterance
+        frame counts of a right-padded x; valid output frames equal the utterance's own, padded ones are unspecified."""
+        seqlens = None
+        if lengths is not None:
+            seqlens = seqlens_tensor(lengths, x.shape[0], x.shape[1], x.device)
+            _forward_only(seqlens, x, *self.parameters())
         if native_layer_ok(x, self):
             # eager mode: the whole layer in one native call each way (same kernels, same order, same bits; a captured
             # step keeps the sequenced Functions below, which overlap the weight-gradient products on a second stream)
-            return encoder_layer_native(x, self)
+            return encoder_layer_native(x, self, seqlens)
         # :471-472; the residual branch leaves the LayerNorm Function as its second output, so its gradient is added to dx
         # inside the LayerNorm backward kernel (no separate autograd add)
         x_norm, residual = layer_norm_fn(x, self.norm1.weight, self.norm1.bias, self.norm1.eps, with_residual=True)
-        mamba_out = self.mamba.forward_bidirectional(x_norm)                                         # :473-481 in one fused pass
+        mamba_out = self.mamba.forward_bidirectional(x_norm, seqlens)                                # :473-481 in one fused pass
         mamba_out = layer_norm_fn(mamba_out, self.norm2.weight, self.norm2.bias, self.norm2.eps)    # :482
         if isinstance(self.feed_forward[1], nn.GELU) and self.feed_forward[1].approximate == "none":
             l1, l2 = self.feed_forward[0], self.feed_forward[2]
@@ -55,18 +62,28 @@ class BiMambaBackend(nn.Module):
         self.dropout = nn.Dropout(0.1)
         self.classifier = nn.Linear(emb_size, 2)
 
-    def forward_features(self, f_fused):
+    def forward_features(self, f_fused, lengths=None):
+        """lengths (B,) (list, CPU or CUDA tensor; scoring only): per-utterance frame counts of the right-padded
+        f_fused.  Output frames at padded positions are unspecified."""
+        seqlens = seqlens_tensor(lengths, f_fused.shape[0], f_fused.shape[1], f_fused.device)
         for layer in self.backbone_layers:
-            f_fused = layer(f_fused)
+            f_fused = layer(f_fused, seqlens)
         return f_fused
 
-    def forward(self, f_fused):
-        return backend_head(self, self.forward_features(f_fused))
+    def forward(self, f_fused, lengths=None):
+        """f_fused (B, T, emb) -> (features, logits).  lengths (B,): see forward_features; every utterance is scored
+        as if it ran alone at its own length (net(x, lengths) with x padded on the right)."""
+        seqlens = seqlens_tensor(lengths, f_fused.shape[0], f_fused.shape[1], f_fused.device)
+        return backend_head(self, self.forward_features(f_fused, seqlens), seqlens)
 
 
-def backend_head(m, f_fused):
+def backend_head(m, f_fused, lengths=None):
     """norm_f -> attention pooling -> dropout -> classifier on a module that carries the reference's attribute names
-    (`norm_f`, `attention_pool`, `dropout`, `classifier`; DualStreamSEMamba.py:759-767).  Returns (features, logits)."""
+    (`norm_f`, `attention_pool`, `dropout`, `classifier`; DualStreamSEMamba.py:759-767).  Returns (features, logits).
+    lengths (B,) (list, CPU or CUDA tensor; scoring only): norm, softmax and pooling over each utterance's first
+    lengths[b] frames only."""
+    if lengths is not None:
+        return _backend_head_varlen(m, f_fused, lengths)
     if not torch.is_grad_enabled() and not m.training and f_fused.shape[-1] <= 256:
         # scoring (src/main.py:958-995): norm_f, attention pooling and the classifier in one launch
         feats, logits = head_fwd(f_fused, m.norm_f.weight, m.norm_f.bias, m.attention_pool.weight,
@@ -82,3 +99,23 @@ def backend_head(m, f_fused):
         features = torch.matmul(attn.transpose(1, 2), f_fused).squeeze(1)           # :763
     features = m.dropout(features)                                                  # :764
     return features, m.classifier(features)                                         # :767
+
+
+def _backend_head_varlen(m, f_fused, lengths):
+    seqlens = seqlens_tensor(lengths, f_fused.shape[0], f_fused.shape[1], f_fused.device)
+    _forward_only(seqlens, f_fused, *m.norm_f.parameters(), *m.attention_pool.parameters(), *m.classifier.parameters())
+    if f_fused.shape[-1] <= 256:
+        feats, logits = head_fwd(f_fused, m.norm_f.weight, m.norm_f.bias, m.attention_pool.weight,
+                                 m.attention_pool.bias, m.classifier.weight, m.classifier.bias, m.norm_f.eps, seqlens)
+        if not m.training:
+            return feats.to(f_fused.dtype), logits.to(f_fused.dtype)
+        features = feats.to(f_fused.dtype)
+    else:
+        # wider than the head kernel: the same three steps with the padded frames masked out of the softmax
+        f_fused = layer_norm_fn(f_fused, m.norm_f.weight, m.norm_f.bias, m.norm_f.eps, out_dtype=f_fused.dtype)
+        valid = torch.arange(f_fused.shape[1], device=f_fused.device).unsqueeze(0) < seqlens.unsqueeze(1)
+        scores = m.attention_pool(f_fused).masked_fill(~valid.unsqueeze(-1), float("-inf"))
+        attn = F.softmax(scores, dim=1).masked_fill(~valid.unsqueeze(-1), 0.0)   # zero-length: zero features
+        features = torch.matmul(attn.transpose(1, 2), f_fused.masked_fill(~valid.unsqueeze(-1), 0.0)).squeeze(1)
+    features = m.dropout(features)
+    return features, m.classifier(features)

@@ -10,7 +10,7 @@ from typing import Callable, Optional
 
 import torch
 
-from .ops import sequenced_block
+from .ops import seqlens_tensor, sequenced_block
 
 
 def _snapshot(optimizer):
@@ -130,24 +130,38 @@ class GraphedTrainStep:
 
 
 class GraphedForward:
-    """Captures a no-grad forward (scoring, src/main.py:958-995) for a fixed input shape."""
+    """Captures a no-grad forward (scoring, src/main.py:958-995) for a fixed input shape.
 
-    def __init__(self, fn: Callable[[torch.Tensor], torch.Tensor], example: torch.Tensor, warmup: int = 2):
+    With `lengths` (an example (B,) vector of frame counts, see ops.seqlens_tensor) `fn` is called as fn(x, lengths)
+    with the lengths in a static int32 device buffer, and run(x, lengths) copies both: one captured graph then scores
+    every mix of utterance lengths padded to the example's shape."""
+
+    def __init__(self, fn: Callable[..., torch.Tensor], example: torch.Tensor, warmup: int = 2, lengths=None):
         self.static_x = torch.empty_like(example, device="cuda")
         self.static_x.copy_(example)
+        self.static_lengths = None
+        args = (self.static_x,)
+        if lengths is not None:
+            self.static_lengths = seqlens_tensor(lengths, example.shape[0], example.shape[1], self.static_x.device).clone()
+            args = (self.static_x, self.static_lengths)
         side = torch.cuda.Stream()
         side.wait_stream(torch.cuda.current_stream())
         with torch.cuda.stream(side), torch.no_grad(), sequenced_block():
             for _ in range(max(1, warmup)):
-                fn(self.static_x)
+                fn(*args)
         torch.cuda.current_stream().wait_stream(side)
         torch.cuda.synchronize()
         self.graph = torch.cuda.CUDAGraph()
         with torch.cuda.graph(self.graph), torch.no_grad():
-            self.static_out = fn(self.static_x)
+            self.static_out = fn(*args)
 
-    def run(self, x: Optional[torch.Tensor] = None):
+    def run(self, x: Optional[torch.Tensor] = None, lengths=None):
         if x is not None:
             self.static_x.copy_(x, non_blocking=True)
+        if lengths is not None:
+            if self.static_lengths is None:
+                raise ValueError("this graph was captured without lengths")
+            B, T = self.static_x.shape[:2]
+            self.static_lengths.copy_(seqlens_tensor(lengths, B, T, self.static_x.device), non_blocking=True)
         self.graph.replay()
         return self.static_out

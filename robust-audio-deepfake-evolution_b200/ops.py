@@ -129,6 +129,31 @@ def _wants_grad(*ts) -> bool:
     return torch.is_grad_enabled() and any(isinstance(t, torch.Tensor) and t.requires_grad for t in ts)
 
 
+def seqlens_tensor(lengths, Bsz: int, T: int, device) -> Optional[torch.Tensor]:
+    """Per-utterance frame counts of a right-padded (B, T, ...) batch -> the (B,) int32 vector the kernels read on
+    `device` (None stays None: fixed length).  `lengths` may be a list, a CPU tensor or a CUDA tensor.  Host-side lengths
+    are checked here without a device sync: shape (B,), integers, 1 <= len <= T, else ValueError.  A CUDA tensor is
+    trusted (only its shape is checked): the kernels clamp its values to [0, T], and a zero-length utterance scores as
+    zero features."""
+    if lengths is None:
+        return None
+    if isinstance(lengths, torch.Tensor) and lengths.is_cuda:
+        if tuple(lengths.shape) != (Bsz,):
+            raise ValueError(f"lengths must have shape ({Bsz},), got {tuple(lengths.shape)}")
+        return lengths if lengths.dtype == torch.int32 and lengths.is_contiguous() else lengths.to(torch.int32).contiguous()
+    t = torch.as_tensor(lengths)
+    if tuple(t.shape) != (Bsz,) or t.is_floating_point() or t.is_complex() or t.dtype == torch.bool:
+        raise ValueError(f"lengths must be {Bsz} integer frame counts, got {tuple(t.shape)} {t.dtype}")
+    if Bsz and (int(t.min()) < 1 or int(t.max()) > T):
+        raise ValueError(f"lengths must lie in 1..{T} (the padded frame count), got {int(t.min())}..{int(t.max())}")
+    return t.to(torch.int32).to(device)
+
+
+def _forward_only(seqlens, *ts) -> None:
+    if seqlens is not None and _wants_grad(*ts):
+        raise NotImplementedError("lengths are supported for scoring only: run under torch.no_grad() / inference_mode()")
+
+
 def _f32c(t: Optional[torch.Tensor]) -> Optional[torch.Tensor]:
     return None if t is None else t.detach().to(torch.float32).contiguous()
 
@@ -148,8 +173,9 @@ def rows2d(t: torch.Tensor) -> torch.Tensor:
 # ----------------------------------------------------------------------------------------
 # raw kernels (no autograd)
 # ----------------------------------------------------------------------------------------
-def conv_fwd_raw(x, weight, bias, out, silu: bool):
-    """x (B, L, D) with unit channel stride; weight (D, K) fp32; out (B, ndir, L, D) view."""
+def conv_fwd_raw(x, weight, bias, out, silu: bool, seqlens: Optional[torch.Tensor] = None):
+    """x (B, L, D) with unit channel stride; weight (D, K) fp32; out (B, ndir, L, D) view.  seqlens: (B,) int32 device
+    frame counts (seqlens_tensor) or None; with them the padded frames of out are written as zeros."""
     lib = _lib.load()
     Bsz, L, D = x.shape
     ndir = out.shape[1]
@@ -157,10 +183,10 @@ def conv_fwd_raw(x, weight, bias, out, silu: bool):
     if x.stride(2) != 1 and D > 1:
         raise ValueError("x must have unit channel stride")
     with _timed("conv_fwd"):
-        rc = lib.bimamba_causal_conv1d_fwd(
-            _ptr(x), _ptr(weight), _ptr(bias), _ptr(out), Bsz, ndir, D, L, weight.shape[1],
+        rc = lib.bimamba_causal_conv1d_fwd_varlen(
+            _ptr(x), _ptr(weight), _ptr(bias), _ptr(out), _ptr(seqlens), Bsz, ndir, D, L, weight.shape[1],
             x.stride(0), x.stride(1), obs, ods, ots, _dt(x), _lib.FLAG_SILU if silu else 0, _stream())
-        _lib.check(rc, "bimamba_causal_conv1d_fwd")
+        _lib.check(rc, "bimamba_causal_conv1d_fwd_varlen")
 
 
 def conv_bwd_raw(x, weight, bias, dout, dx, silu: bool, dz_in=None, dz_out=None, defer: Optional[list] = None):
@@ -228,10 +254,15 @@ def _fill_desc(u, z, delta, bc, dtr, Wdt, A, D, delta_bias, softplus, dtr_padded
 
 
 def scan_fwd_raw(u, z, delta, bc, dtr, Wdt, A, D, delta_bias, softplus: bool, want_ckpt: bool,
-                 dtr_padded: bool = False):
+                 dtr_padded: bool = False, seqlens: Optional[torch.Tensor] = None):
     """All activations are (B, ndir, L, C) views with unit channel stride (z may be expanded over
-    dir).  Returns (out, ckpt, ypre): out / ypre are (B, ndir, L, dim) views of (B, L, ndir, dim)."""
+    dir).  Returns (out, ckpt, ypre): out / ypre are (B, ndir, L, dim) views of (B, L, ndir, dim).
+    seqlens: (B,) int32 device frame counts (seqlens_tensor) or None.  With them each utterance walks its own frames
+    (direction 1 from its last valid one), padded frames of out are zeros, and the serial walk is used: the time-split
+    forward has no variable-length form.  Forward only (want_ckpt must be False)."""
     lib = _lib.load()
+    if seqlens is not None and want_ckpt:
+        raise NotImplementedError("variable-length scan is forward-only (no checkpoints for a backward)")
     Bsz, ndir, L, dim = u.shape
     G, ngroups, nchunks = _lib.scan_plan(L, dim, Bsz * ndir, False)
     out = per_dir(Bsz, L, ndir, dim, u.device, u.dtype)
@@ -243,7 +274,7 @@ def scan_fwd_raw(u, z, delta, bc, dtr, Wdt, A, D, delta_bias, softplus: bool, wa
     d = _fill_desc(u, z, delta, bc, dtr, Wdt, A, D, delta_bias, softplus, dtr_padded, G)
     d.out, d.ypre, d.ckpt = _ptr(out), _ptr(ypre), _ptr(ckpt)
     d.out_bs, d.out_ds, d.out_ts = _s3(out)
-    nseg, seg_len = _lib.scan_split_plan(Bsz, ndir, L, dim, _dt(u))
+    nseg, seg_len = _lib.scan_split_plan(Bsz, ndir, L, dim, _dt(u)) if seqlens is None else (1, L)
     if nseg > 1:
         # long sequence, few channel lanes: time-parallel scan (carry pass + output pass, two launches)
         nbytes = lib.bimamba_scan_fwd_split_workspace_bytes(Bsz, ndir, dim, nseg)
@@ -254,7 +285,8 @@ def scan_fwd_raw(u, z, delta, bc, dtr, Wdt, A, D, delta_bias, softplus: bool, wa
         _lib.launch_count += 1   # two kernels per call
         return out, ckpt, ypre
     with _timed("scan_fwd"):
-        _lib.check(lib.bimamba_selective_scan_fwd(C.byref(d), _stream()), "bimamba_selective_scan_fwd")
+        _lib.check(lib.bimamba_selective_scan_fwd_varlen(C.byref(d), _ptr(seqlens), _stream()),
+                   "bimamba_selective_scan_fwd_varlen")
     return out, ckpt, ypre
 
 
@@ -757,10 +789,12 @@ class LayerNormFn(torch.autograd.Function):
         return dx.view(shape), dgb[0].to(wdt), dgb[1].to(bdt), None, None, None, None
 
 
-def head_fwd(x, norm_w, norm_b, att_w, att_b, cls_w, cls_b, eps=1e-5):
+def head_fwd(x, norm_w, norm_b, att_w, att_b, cls_w, cls_b, eps=1e-5, lengths=None):
     """Scoring head in one launch (no autograd): LayerNorm -> attention pooling over time -> classifier
-    (src/models/DualStreamSEMamba.py:759-767, eval mode).  x (B, T, C) -> features (B, C) fp32, logits (B, n) fp32."""
+    (src/models/DualStreamSEMamba.py:759-767, eval mode).  x (B, T, C) -> features (B, C) fp32, logits (B, n) fp32.
+    lengths (B,) (seqlens_tensor): pool utterance b over its first lengths[b] frames only."""
     lib = _lib.load()
+    seqlens = seqlens_tensor(lengths, x.shape[0], x.shape[1], x.device)
     _require_cuda(x)
     if x.dtype not in _DT:
         x = x.float()
@@ -774,8 +808,9 @@ def head_fwd(x, norm_w, norm_b, att_w, att_b, cls_w, cls_b, eps=1e-5):
     feats = torch.empty((Bsz, C_), device=x.device, dtype=torch.float32)
     logits = torch.empty((Bsz, ncls), device=x.device, dtype=torch.float32)
     with _timed("head_fwd"):
-        _lib.check(lib.bimamba_head_fwd(_ptr(x), _ptr(gw), _ptr(gb), _ptr(aw), _ptr(ab), _ptr(cw), _ptr(cb), _ptr(feats),
-                                        _ptr(logits), Bsz, T, C_, ncls, float(eps), _dt(x), _stream()), "bimamba_head_fwd")
+        _lib.check(lib.bimamba_head_fwd_varlen(_ptr(x), _ptr(gw), _ptr(gb), _ptr(aw), _ptr(ab), _ptr(cw), _ptr(cb),
+                                               _ptr(feats), _ptr(logits), _ptr(seqlens), Bsz, T, C_, ncls, float(eps),
+                                               _dt(x), _stream()), "bimamba_head_fwd_varlen")
     return feats, logits
 
 
@@ -936,7 +971,8 @@ class BiMambaInnerFn(torch.autograd.Function):
     """
 
     @staticmethod
-    def forward(ctx, x, W_in, conv_w, conv_b, W_x, W_dt, b_dt, A_log, Dp, W_out, bidirectional, cdtype, needs_bwd=True):
+    def forward(ctx, x, W_in, conv_w, conv_b, W_x, W_dt, b_dt, A_log, Dp, W_out, bidirectional, cdtype, needs_bwd=True,
+                seqlens=None):
         _require_cuda(x, W_in, conv_w, conv_b, W_x, W_dt, b_dt, A_log, Dp, W_out)
         with torch.autocast("cuda", enabled=False):
             Bsz, L, dm = x.shape
@@ -962,12 +998,12 @@ class BiMambaInnerFn(torch.autograd.Function):
             xz3 = xz.view(Bsz, L, 2 * D)
             xs, z = xz3[:, :, :D], xz3[:, :, D:]                              # :49 (views)
             xc = per_dir(Bsz, L, ndir, D, dev, cdtype)
-            conv_fwd_raw(xs, cw32, cb32, xc, True)                            # :52-55, both directions
+            conv_fwd_raw(xs, cw32, cb32, xc, True, seqlens)                   # :52-55, both directions
             xdbl = gemm_nt(rows2d(xc), Wxp)                                   # (M*ndir, 48)   :73
             xd4 = xdbl.view(Bsz, L, ndir, XW).permute(0, 2, 1, 3)
             y, ckpt, ypre = scan_fwd_raw(xc, z.unsqueeze(1).expand(Bsz, ndir, L, D), None, xd4[..., :2 * N],
                                          xd4[..., 2 * N:], Wd32, A32, D32, bdt32, True, needs_bwd,
-                                         dtr_padded=True)                     # :80-120, :61
+                                         dtr_padded=True, seqlens=seqlens)    # :80-120, :61
             out = gemm_nt(rows2d(y).view(M, ndir * D), Wo2).view(Bsz, L, dm)  # :62 + DualStreamSEMamba.py:481
             if needs_bwd:
                 ctx.save_for_backward(x2, xz, xc, xdbl, y, WiT, WxpT, WoT, WdT, Wd32, cw32, cb32, A32, D32, bdt32,
@@ -1044,7 +1080,7 @@ class BiMambaInnerFn(torch.autograd.Function):
                     "bimamba_finalize_param_grads")
         return (dx.to(xdt), dW_in.to(pdt[0]), dcw.to(pdt[1]), dcb.to(pdt[2]),
                 dW_x.to(pdt[3]), dW_dt.to(pdt[4]), dbdt.to(pdt[5]), dA_log.to(pdt[6]), dD.to(pdt[7]),
-                dW_out.to(pdt[8]), None, None, None)
+                dW_out.to(pdt[8]), None, None, None, None)
 
 
 # Eager mode (no CUDA-graph capture): the block runs through the one-call native entry points - the same kernels in the
@@ -1080,14 +1116,15 @@ class BiMambaNativeFn(torch.autograd.Function):
     """BiMambaInnerFn through bimamba_block_fwd / bimamba_block_bwd (csrc/block.cu): eager-mode fast path."""
 
     @staticmethod
-    def forward(ctx, x, W_in, conv_w, conv_b, W_x, W_dt, b_dt, A_log, Dp, W_out, bidirectional, cdtype, needs_bwd=True):
+    def forward(ctx, x, W_in, conv_w, conv_b, W_x, W_dt, b_dt, A_log, Dp, W_out, bidirectional, cdtype, needs_bwd=True,
+                seqlens=None):
         with torch.autocast("cuda", enabled=False):
             if A_log.shape[1] != D_STATE:
                 raise NotImplementedError("d_state must be 16 (the Phase-6 configuration)")
             if W_dt.shape[1] > MAX_DT_RANK:
                 raise NotImplementedError("dt_rank must be <= 16")
             nb = NativeBlock(x.detach().to(cdtype), W_in, conv_w, conv_b, W_x, W_dt, b_dt, A_log, Dp, W_out,
-                             bidirectional=bidirectional, save_for_backward=needs_bwd)
+                             bidirectional=bidirectional, save_for_backward=needs_bwd, seqlens=seqlens)
             out, nb.out = nb.out, None          # the output must not be reachable from ctx (reference cycle)
             if needs_bwd:
                 ctx.nb = nb
@@ -1099,19 +1136,24 @@ class BiMambaNativeFn(torch.autograd.Function):
         xdt, pdt = ctx.meta
         with torch.autocast("cuda", enabled=False):
             grads = ctx.nb.backward(dout)
-        return (grads[0].to(xdt), *[g.to(d) for g, d in zip(grads[1:], pdt)], None, None, None)
+        return (grads[0].to(xdt), *[g.to(d) for g, d in zip(grads[1:], pdt)], None, None, None, None)
 
 
 def bimamba_inner_fn(x, W_in, conv_w, conv_b, W_x, W_dt, b_dt, A_log, Dp, W_out, bidirectional=True,
-                     compute_dtype=None):
+                     compute_dtype=None, lengths=None):
     """x (B, L, d_model) -> (B, L, d_model).  compute_dtype: activation dtype of the kernels and
-    GEMMs (default: the autocast dtype when autocast is on, else x.dtype); scan state is fp32."""
+    GEMMs (default: the autocast dtype when autocast is on, else x.dtype); scan state is fp32.
+    lengths (B,): utterance b is frames 0 .. lengths[b]-1 of the right-padded x (seqlens_tensor); each valid output frame
+    equals that of the utterance run alone at its own length, output frames at padded positions are unspecified.
+    Scoring only: with lengths and autograd recording this raises NotImplementedError."""
     if compute_dtype is None:
         compute_dtype = torch.get_autocast_dtype("cuda") if torch.is_autocast_enabled("cuda") else x.dtype
+    seqlens = seqlens_tensor(lengths, x.shape[0], x.shape[1], x.device)
     _require_cuda(x, W_in, conv_w, conv_b, W_x, W_dt, b_dt, A_log, Dp, W_out)
+    ps = (x, W_in, conv_w, conv_b, W_x, W_dt, b_dt, A_log, Dp, W_out)
+    _forward_only(seqlens, *ps)
     fn = BiMambaNativeFn if _native_block_ok(x, W_in, compute_dtype) else BiMambaInnerFn
-    return fn.apply(x, W_in, conv_w, conv_b, W_x, W_dt, b_dt, A_log, Dp, W_out, bool(bidirectional),
-                    compute_dtype, _wants_grad(x, W_in, conv_w, conv_b, W_x, W_dt, b_dt, A_log, Dp, W_out))
+    return fn.apply(*ps, bool(bidirectional), compute_dtype, _wants_grad(*ps), seqlens)
 
 
 # ----------------------------------------------------------------------------------------
@@ -1123,7 +1165,7 @@ class NativeBlock:
     """State of one forward call of the native block: descriptor, saved-activation workspace, packed weights."""
 
     def __init__(self, x, W_in, conv_w, conv_b, W_x, W_dt, b_dt, A_log, Dp, W_out, bidirectional=True,
-                 save_for_backward=True):
+                 save_for_backward=True, seqlens=None):
         _require_cuda(x, W_in, conv_w, conv_b, W_x, W_dt, b_dt, A_log, Dp, W_out)
         if x.dtype not in (torch.bfloat16, torch.float16):
             raise TypeError("the native block entry points take bf16 / fp16 activations")
@@ -1153,7 +1195,7 @@ class NativeBlock:
         d.batch, d.seqlen, d.d_model, d.d_inner, d.dt_rank, d.d_conv, d.ndir = Bsz, L, dm, D, R, K, ndir
         d.io_dtype, d.save_for_backward = _dt(x), int(save_for_backward)
         self.desc = d
-        _lib.check(lib.bimamba_block_fwd(C.byref(d), _stream()), "bimamba_block_fwd")
+        _lib.check(lib.bimamba_block_fwd_varlen(C.byref(d), _ptr(seqlens), _stream()), "bimamba_block_fwd_varlen")
         _lib.launch_count += 4           # the call enqueues 5 kernels (3 GEMMs, conv, scan)
 
     def backward(self, dout):
@@ -1189,7 +1231,7 @@ class NativeLayer:
     """One forward call of the native encoder layer: descriptor, saved-activation workspace, packed Mamba weights."""
 
     def __init__(self, x, norm1_w, norm1_b, eps1, norm2_w, norm2_b, eps2, W1, b1, W2, b2, W_in, conv_w, conv_b, W_x, W_dt,
-                 b_dt, A_log, Dp, W_out, cdtype, save_for_backward=True):
+                 b_dt, A_log, Dp, W_out, cdtype, save_for_backward=True, seqlens=None):
         _require_cuda(x, norm1_w, W1, W_in)
         lib = _lib.load()
         Bsz, L, dm = x.shape
@@ -1220,7 +1262,7 @@ class NativeLayer:
         d.eps1, d.eps2, d.d_ff, d.x_dtype = float(eps1), float(eps2), dff, _dt(self.x)
         self.desc = d
         self._keep_fwd = (cw32,)
-        _lib.check(lib.bimamba_layer_fwd(C.byref(d), _stream()), "bimamba_layer_fwd")
+        _lib.check(lib.bimamba_layer_fwd_varlen(C.byref(d), _ptr(seqlens), _stream()), "bimamba_layer_fwd_varlen")
         _lib.launch_count += 11          # 12 kernels: 2 LayerNorm, 5 of the block, 2 weight casts, 2 GEMMs, GELU
 
     def backward(self, dout):
@@ -1256,14 +1298,14 @@ class EncoderLayerNativeFn(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, x, n1w, n1b, n2w, n2b, W1, b1, W2, b2, W_in, conv_w, conv_b, W_x, W_dt, b_dt, A_log, Dp, W_out,
-                eps1, eps2, cdtype, needs_bwd=True):
+                eps1, eps2, cdtype, needs_bwd=True, seqlens=None):
         with torch.autocast("cuda", enabled=False):
             if A_log.shape[1] != D_STATE:
                 raise NotImplementedError("d_state must be 16 (the Phase-6 configuration)")
             if W_dt.shape[1] > MAX_DT_RANK:
                 raise NotImplementedError("dt_rank must be <= 16")
             nl = NativeLayer(x, n1w, n1b, eps1, n2w, n2b, eps2, W1, b1, W2, b2, W_in, conv_w, conv_b, W_x, W_dt, b_dt,
-                             A_log, Dp, W_out, cdtype, save_for_backward=needs_bwd)
+                             A_log, Dp, W_out, cdtype, save_for_backward=needs_bwd, seqlens=seqlens)
             out, nl.out = nl.out, None          # the output must not be reachable from ctx (reference cycle)
             if needs_bwd:
                 ctx.nl = nl
@@ -1277,7 +1319,7 @@ class EncoderLayerNativeFn(torch.autograd.Function):
             r = ctx.nl.backward(dout)
         dx, dn1, dn2 = r[0], r[1], r[2]
         grads = [dn1[0], dn1[1], dn2[0], dn2[1], *r[3:]]
-        return (dx.view(dout.shape), *[g.to(d) for g, d in zip(grads, ctx.pdt)], None, None, None, None)
+        return (dx.view(dout.shape), *[g.to(d) for g, d in zip(grads, ctx.pdt)], None, None, None, None, None)
 
 
 def native_layer_ok(x, layer) -> bool:
@@ -1299,10 +1341,12 @@ def native_layer_ok(x, layer) -> bool:
             and m.dt_rank <= MAX_DT_RANK and not torch.cuda.is_current_stream_capturing())
 
 
-def encoder_layer_native(x, layer):
+def encoder_layer_native(x, layer, seqlens=None):
+    """seqlens: (B,) int32 device frame counts (seqlens_tensor) or None; scoring only."""
     cd = torch.get_autocast_dtype("cuda") if torch.is_autocast_enabled("cuda") else x.dtype
     m, ff = layer.mamba, layer.feed_forward
     ps = (layer.norm1.weight, layer.norm1.bias, layer.norm2.weight, layer.norm2.bias, ff[0].weight, ff[0].bias,
           ff[2].weight, ff[2].bias, m.in_proj.weight, m.conv1d.weight, m.conv1d.bias, m.x_proj.weight, m.dt_proj.weight,
           m.dt_proj.bias, m.A_log, m.D, m.out_proj.weight)
-    return EncoderLayerNativeFn.apply(x, *ps, layer.norm1.eps, layer.norm2.eps, cd, _wants_grad(x, *ps))
+    _forward_only(seqlens, x, *ps)
+    return EncoderLayerNativeFn.apply(x, *ps, layer.norm1.eps, layer.norm2.eps, cd, _wants_grad(x, *ps), seqlens)
