@@ -34,9 +34,11 @@ adamw_kernel(const bimamba_adamw_tensor* __restrict__ tab, const int2* __restric
   const int2 bm = blocks[blockIdx.x];
   const bimamba_adamw_tensor t = tab[bm.x];
   const float lr = hyper[0], b1 = hyper[1], b2 = hyper[2], eps = hyper[3], wd = hyper[4];
-  const float step = state[0];
-  const float inv_bc1 = 1.f / (1.f - powf(b1, step));
-  const float inv_sqrt_bc2 = rsqrtf(1.f - powf(b2, step));
+  // bias corrections 1 - beta^t in double: in fp32, 1 - powf(0.999f, t) keeps only about 1e-4 of its value at the first
+  // steps (the rounding of beta^t near 1 against a difference of t * 1e-3), a relative error of ~1e-5 in every update
+  const double step = state[0];
+  const float inv_bc1 = (float)(1.0 / (1.0 - pow((double)b1, step)));
+  const float inv_sqrt_bc2 = (float)(1.0 / sqrt(1.0 - pow((double)b2, step)));
   const float decay = 1.f - lr * wd;
   const int64_t base = (int64_t)bm.y * kAdamChunk;
   const int64_t end = min(t.n, base + kAdamChunk);
