@@ -30,6 +30,8 @@
  *
  *   bimamba_*_fwd_varlen              <- scoring of right-padded batches of utterances of different lengths
  *                                       (per-utterance frame counts; see "Variable-length scoring" below)
+ *   bimamba_*_varlen_train, *_bwd_varlen, bimamba_mask_frames
+ *                                    <- training on such batches (see "Variable-length training" below)
  *
  * Ownership: the library never allocates or frees device memory.  All tensors and
  * workspaces are caller-allocated; pointers are borrowed for the duration of the
@@ -155,8 +157,28 @@ int bimamba_selective_scan_bwd(const bimamba_scan_desc* d, bimamba_stream_t stre
  * by the conv, the scan or the head, so the padding may hold anything (NaN included).  Outputs a call owns per frame
  * (conv out, scan out / ypre) are written as zeros at padded frames; a zero-length utterance yields zeros.  A NULL
  * seqlens is the fixed-length call: bimamba_X(...) is bimamba_X_varlen(..., NULL, ...).  Forward only: the scan rejects
- * checkpoints (d->ckpt != NULL) and the block / layer reject save_for_backward != 0 with a negative code. */
+ * checkpoints (d->ckpt != NULL) and the block / layer reject save_for_backward != 0 with a negative code; the
+ * _varlen_train entries below are the training forms. */
 int bimamba_selective_scan_fwd_varlen(const bimamba_scan_desc* d, const int32_t* seqlens, bimamba_stream_t stream);
+
+/* ---- Variable-length training.  The training forward and the backward of each op walk the same per-utterance frames
+ * as the scoring calls above (seqlens: device int32, clamped to [0, seqlen]; NULL = the fixed-length call, so
+ * bimamba_X_bwd(...) is bimamba_X_bwd_varlen(..., NULL, ...)).  Each utterance gets the gradients it would get alone at
+ * its own length; parameter-gradient partials sum over utterances as a batch does.  Layouts and workspace sizes are
+ * those of the padded seqlen (checkpoints: ceil(seqlen / 8) per channel, chunk c = scan steps 8c .. 8c+7 of the
+ * utterance).  Gradients a call owns per frame (scan du / ddelta / dz and its [dB | dC] partial rows, conv dx and the
+ * folded dz, head dx) are written as zeros at padded frames; dout there is never read by the scan or the conv.
+ *
+ * The scan forward that also writes checkpoints and ypre (the refusal of bimamba_selective_scan_fwd_varlen lifted): */
+int bimamba_selective_scan_fwd_varlen_train(const bimamba_scan_desc* d, const int32_t* seqlens, bimamba_stream_t stream);
+int bimamba_selective_scan_bwd_varlen(const bimamba_scan_desc* d, const int32_t* seqlens, bimamba_stream_t stream);
+
+/* out (batch, seqlen, channels) = x where t < seqlens[b], zero elsewhere - by selection: padded frames are never read, so
+ * NaN padding cannot pass.  x and out contiguous in `dtype`; out may be x (in place).  One launch.  With the block and
+ * layer entries a host gets the masked training contract by masking x before the forward and dout before the backward
+ * (and, for the layer, the output after the forward: its feed-forward and residual make padded output rows non-zero). */
+int bimamba_mask_frames(const void* x, void* out, const int32_t* seqlens, int batch, int seqlen, int channels, int dtype,
+                        bimamba_stream_t stream);
 
 /* Time-parallel forward scan for long sequences at small batches (the scan as an associative operator on pairs,
  * (a2, b2) o (a1, b1) = (a2 a1, a2 b1 + b2); mamba_block.py:92-117 is the serial loop).  Scan time is cut into nseg
@@ -199,6 +221,13 @@ int bimamba_causal_conv1d_bwd(const void* x, const float* weight, const float* b
                               int batch, int ndir, int dim, int seqlen, int width,
                               int64_t x_bs, int64_t x_ts, int64_t dout_bs, int64_t dout_ds, int64_t dout_ts,
                               int64_t dx_bs, int64_t dx_ts, int dtype, int flags, bimamba_stream_t stream);
+/* Backward of bimamba_causal_conv1d_fwd_varlen: frames t >= seqlens[b] of x and dout are never read; dx and dz_out are
+ * zero there. */
+int bimamba_causal_conv1d_bwd_varlen(const void* x, const float* weight, const float* bias, const void* dout,
+                                     void* dx, const void* dz_in, void* dz_out, float* dwb_part, const int32_t* seqlens,
+                                     int batch, int ndir, int dim, int seqlen, int width,
+                                     int64_t x_bs, int64_t x_ts, int64_t dout_bs, int64_t dout_ds, int64_t dout_ts,
+                                     int64_t dx_bs, int64_t dx_ts, int dtype, int flags, bimamba_stream_t stream);
 
 /* For every g < groups:  out[g*out_gs + j] (+)= sum_{i < rows} part[g*part_gs + i*row_stride + j],
  * j < cols, summed in fixed order (deterministic).  out element type out_dtype;
@@ -239,6 +268,12 @@ int bimamba_head_fwd_varlen(const void* x, const float* gamma, const float* beta
 int bimamba_head_pool_bwd(const void* x, const float* gamma, const float* beta, const float* w_att, const float* b_att,
                           const float* dfeatures, void* dx, float* part, int batch, int seqlen, int channels, float eps,
                           int dtype, bimamba_stream_t stream);
+/* Backward of bimamba_head_fwd_varlen (nclasses = 0): both passes over t < seqlens[b]; dx is zero at padded frames and a
+ * zero-length utterance gets zero dx and a zero partial row. */
+int bimamba_head_pool_bwd_varlen(const void* x, const float* gamma, const float* beta, const float* w_att,
+                                 const float* b_att, const float* dfeatures, void* dx, float* part,
+                                 const int32_t* seqlens, int batch, int seqlen, int channels, float eps, int dtype,
+                                 bimamba_stream_t stream);
 
 /* AdamW (torch.optim.AdamW semantics: decoupled weight decay, no amsgrad - the optimizer of src/main.py:453) over a
  * list of fp32 tensors in one launch.  `table` (device): one entry per tensor; `block_map` (device): nblocks pairs
@@ -410,6 +445,14 @@ int bimamba_block_fwd(const bimamba_block_desc* d, bimamba_stream_t stream);
 int bimamba_block_fwd_varlen(const bimamba_block_desc* d, const int32_t* seqlens, bimamba_stream_t stream);
 /* `d` is the descriptor the forward ran with (same workspace, save_for_backward != 0). */
 int bimamba_block_bwd(const bimamba_block_desc* d, const bimamba_block_grads* g, bimamba_stream_t stream);
+/* Variable-length training (see "Variable-length training" above): the forward accepts save_for_backward, and the
+ * backward takes the seqlens the forward ran with.  These calls do not mask: padded input rows never reach a valid
+ * output or a gradient through the conv and the scan, but the products run over every row, so a host masks x with
+ * bimamba_mask_frames before the forward (NaN padding would otherwise reach dW_in) and may mask dout before the backward.
+ * Output rows at padded frames are zero (the scan writes zeros there and out_proj has no bias). */
+int bimamba_block_fwd_varlen_train(const bimamba_block_desc* d, const int32_t* seqlens, bimamba_stream_t stream);
+int bimamba_block_bwd_varlen(const bimamba_block_desc* d, const bimamba_block_grads* g, const int32_t* seqlens,
+                             bimamba_stream_t stream);
 
 /* ---- The whole encoder layer in one call each way: PN_BiMambas_Encoder.forward (DualStreamSEMamba.py:467-486)
  *   out = FFN(LN2(M(LN1 x) + flip(M(flip(LN1 x))))) + x,   FFN = Linear(d_model, d_ff) -> GELU (erf) -> Linear(d_ff, d_model)
@@ -461,6 +504,13 @@ int bimamba_layer_fwd(const bimamba_layer_desc* d, bimamba_stream_t stream);
  * rows at padded frames are unspecified. */
 int bimamba_layer_fwd_varlen(const bimamba_layer_desc* d, const int32_t* seqlens, bimamba_stream_t stream);
 int bimamba_layer_bwd(const bimamba_layer_desc* d, const bimamba_layer_grads* g, bimamba_stream_t stream);
+/* Variable-length training of the layer.  No masking inside: the masked contract (padded output frames exactly zero,
+ * zero gradient at padded input frames, nothing from the padding in any parameter gradient) is
+ *   bimamba_mask_frames(x) -> bimamba_layer_fwd_varlen_train -> bimamba_mask_frames(out)
+ *   bimamba_mask_frames(dout) -> bimamba_layer_bwd_varlen -> (dx is then zero at padded frames). */
+int bimamba_layer_fwd_varlen_train(const bimamba_layer_desc* d, const int32_t* seqlens, bimamba_stream_t stream);
+int bimamba_layer_bwd_varlen(const bimamba_layer_desc* d, const bimamba_layer_grads* g, const int32_t* seqlens,
+                             bimamba_stream_t stream);
 
 #ifdef __cplusplus
 }

@@ -32,6 +32,9 @@ EXPORTS = (
     "bimamba_layer_fwd_workspace_bytes", "bimamba_layer_bwd_workspace_bytes", "bimamba_layer_fwd", "bimamba_layer_bwd",
     "bimamba_causal_conv1d_fwd_varlen", "bimamba_selective_scan_fwd_varlen", "bimamba_head_fwd_varlen",
     "bimamba_block_fwd_varlen", "bimamba_layer_fwd_varlen",
+    "bimamba_selective_scan_fwd_varlen_train", "bimamba_selective_scan_bwd_varlen", "bimamba_causal_conv1d_bwd_varlen",
+    "bimamba_head_pool_bwd_varlen", "bimamba_block_fwd_varlen_train", "bimamba_block_bwd_varlen",
+    "bimamba_layer_fwd_varlen_train", "bimamba_layer_bwd_varlen", "bimamba_mask_frames",
 )
 
 
@@ -226,6 +229,25 @@ def load() -> C.CDLL:
         lib.bimamba_layer_fwd_varlen.argtypes = [C.POINTER(LayerDesc), vp, vp]
         lib.bimamba_layer_bwd.restype = i32
         lib.bimamba_layer_bwd.argtypes = [C.POINTER(LayerDesc), C.POINTER(LayerGrads), vp]
+        for name in ("bimamba_selective_scan_fwd_varlen_train", "bimamba_selective_scan_bwd_varlen"):
+            fn = getattr(lib, name)
+            fn.restype = i32
+            fn.argtypes = [C.POINTER(ScanDesc), vp, vp]
+        lib.bimamba_causal_conv1d_bwd_varlen.restype = i32
+        lib.bimamba_causal_conv1d_bwd_varlen.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, vp, i32, i32, i32, i32, i32,
+                                                         i64, i64, i64, i64, i64, i64, i64, i32, i32, vp]
+        lib.bimamba_head_pool_bwd_varlen.restype = i32
+        lib.bimamba_head_pool_bwd_varlen.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, vp, i32, i32, i32, C.c_float, i32, vp]
+        lib.bimamba_block_fwd_varlen_train.restype = i32
+        lib.bimamba_block_fwd_varlen_train.argtypes = [C.POINTER(BlockDesc), vp, vp]
+        lib.bimamba_block_bwd_varlen.restype = i32
+        lib.bimamba_block_bwd_varlen.argtypes = [C.POINTER(BlockDesc), C.POINTER(BlockGrads), vp, vp]
+        lib.bimamba_layer_fwd_varlen_train.restype = i32
+        lib.bimamba_layer_fwd_varlen_train.argtypes = [C.POINTER(LayerDesc), vp, vp]
+        lib.bimamba_layer_bwd_varlen.restype = i32
+        lib.bimamba_layer_bwd_varlen.argtypes = [C.POINTER(LayerDesc), C.POINTER(LayerGrads), vp, vp]
+        lib.bimamba_mask_frames.restype = i32
+        lib.bimamba_mask_frames.argtypes = [vp, vp, vp, i32, i32, i32, i32, vp]
         got = lib.bimamba_abi_version()
         if got != ABI_VERSION:
             raise RuntimeError(f"libbimamba ABI {got} != expected {ABI_VERSION}; rebuild the library")

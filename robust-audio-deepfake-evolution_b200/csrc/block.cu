@@ -143,14 +143,20 @@ extern "C" int bimamba_block_fwd(const bimamba_block_desc* d, bimamba_stream_t s
   return bimamba_block_fwd_varlen(d, nullptr, stream);
 }
 
-// seqlens != NULL: scoring of right-padded utterances of different lengths.  The products run on every row (a row of a
-// product depends on that row only); the conv and the scan walk each utterance's own frames and write zeros to the
-// padded ones, so valid outputs do not depend on what the padding holds.
+// seqlens != NULL: right-padded utterances of different lengths.  The products run on every row (a row of a product
+// depends on that row only); the conv and the scan walk each utterance's own frames and write zeros to the padded ones,
+// so valid outputs do not depend on what the padding holds.
 extern "C" int bimamba_block_fwd_varlen(const bimamba_block_desc* d, const int32_t* seqlens, bimamba_stream_t stream) {
   if (d && seqlens && d->save_for_backward) {
     set_err("block_fwd_varlen: variable-length batches are forward-only (save_for_backward must be 0)");
     return -9;
   }
+  return bimamba_block_fwd_varlen_train(d, seqlens, stream);
+}
+
+// The training forward: with save_for_backward the scan also writes its checkpoints (ceil(seqlen / 8) per channel, the
+// padded layout) and the ungated y for bimamba_block_bwd_varlen.
+extern "C" int bimamba_block_fwd_varlen_train(const bimamba_block_desc* d, const int32_t* seqlens, bimamba_stream_t stream) {
   int rc = check_block(d);
   if (rc) return rc;
   if (d->batch == 0 || d->seqlen == 0) return 0;
@@ -181,13 +187,20 @@ extern "C" int bimamba_block_fwd_varlen(const bimamba_block_desc* d, const int32
   int G = 0, ng = 0;
   bimamba_scan_plan((int)L, D, (int)(B * nd), 0, &G, &ng);
   s.group_channels = G;
-  rc = bimamba_selective_scan_fwd_varlen(&s, seqlens, stream);
+  rc = bimamba_selective_scan_fwd_varlen_train(&s, seqlens, stream);
   if (rc) return rc;
   // out_proj of the sum of the directions as one product over [y_fwd | y_rev] (:62, DualStreamSEMamba.py:481)
   return bimamba_gemm_nt(y, (int64_t)nd * D, d->Wo2, (int64_t)nd * D, d->out, dm, nullptr, nullptr, M, dm, nd * D, dt, dt, stream);
 }
 
 extern "C" int bimamba_block_bwd(const bimamba_block_desc* d, const bimamba_block_grads* g, bimamba_stream_t stream) {
+  return bimamba_block_bwd_varlen(d, g, nullptr, stream);
+}
+
+// seqlens != NULL: the backward of bimamba_block_fwd_varlen_train (same seqlens).  The scan and the conv walk each
+// utterance's own frames and write zero gradients at padded frames, so every product over the rows sees zeros there.
+extern "C" int bimamba_block_bwd_varlen(const bimamba_block_desc* d, const bimamba_block_grads* g, const int32_t* seqlens,
+                                        bimamba_stream_t stream) {
   int rc = check_block(d);
   if (rc) return rc;
   if (!g) { set_err("block_bwd: null gradient descriptor"); return -1; }
@@ -244,7 +257,7 @@ extern "C" int bimamba_block_bwd(const bimamba_block_desc* d, const bimamba_bloc
   s.du = du; s.ddelta = ddelta; s.dz = dz;
   s.dbc_part = dbc_part; s.dA_part = dA_part; s.dD_part = dD_part; s.dbias_part = db_part;
   s.group_channels = 32;
-  BIMAMBA_TRY(bimamba_selective_scan_bwd(&s, stream));
+  BIMAMBA_TRY(bimamba_selective_scan_bwd_varlen(&s, seqlens, stream));
   // [dB | dC]: fixed-order sum over the channel groups, written next to where ddt_r goes (no concatenation)
   BIMAMBA_TRY(bimamba_reduce_rows32(dbc_part, dxdbl, B, w.ngroups, L * nd, kXW, dt, stream));
   BIMAMBA_TRY(bimamba_reduce_partials(dA_part, dA, 1, B * nd, (int64_t)D * kN, 0, (int64_t)D * kN, 0, BIMAMBA_F32, 0, stream));
@@ -258,9 +271,10 @@ extern "C" int bimamba_block_bwd(const bimamba_block_desc* d, const bimamba_bloc
   // x_proj data gradient + the scan's du
   BIMAMBA_TRY(bimamba_gemm_nt(dxdbl, kXW, g->WxpT, kXW, dxc, D, nullptr, du, M * nd, D, kXW, dt, dt, stream));
   // conv backward: dx into the x half and dz_fwd + dz_rev into the z half of one [dx | dz] matrix
-  BIMAMBA_TRY(bimamba_causal_conv1d_bwd(xz, d->conv_w, d->conv_b, dxc, dxz, dz, static_cast<unsigned char*>(dxz) + (size_t)D * es,
-                                        conv_part, (int)B, nd, D, (int)L, K, L * 2 * D, 2 * D, L * nd * D, D, (int64_t)nd * D,
-                                        L * 2 * D, 2 * D, dt, BIMAMBA_FLAG_SILU, stream));
+  BIMAMBA_TRY(bimamba_causal_conv1d_bwd_varlen(xz, d->conv_w, d->conv_b, dxc, dxz, dz,
+                                               static_cast<unsigned char*>(dxz) + (size_t)D * es, conv_part, seqlens, (int)B, nd,
+                                               D, (int)L, K, L * 2 * D, 2 * D, L * nd * D, D, (int64_t)nd * D, L * 2 * D, 2 * D,
+                                               dt, BIMAMBA_FLAG_SILU, stream));
   BIMAMBA_TRY(bimamba_reduce_partials(conv_part, dwb, 1, w.conv_slices, (int64_t)D * (K + 1), 0, (int64_t)D * (K + 1), 0,
                                       BIMAMBA_F32, 0, stream));
   // in_proj
@@ -383,6 +397,10 @@ extern "C" int bimamba_layer_fwd_varlen(const bimamba_layer_desc* d, const int32
     set_err("layer_fwd_varlen: variable-length batches are forward-only (save_for_backward must be 0)");
     return -9;
   }
+  return bimamba_layer_fwd_varlen_train(d, seqlens, stream);
+}
+
+extern "C" int bimamba_layer_fwd_varlen_train(const bimamba_layer_desc* d, const int32_t* seqlens, bimamba_stream_t stream) {
   int rc = check_layer(d);
   if (rc) return rc;
   bimamba_block_desc k = d->block;
@@ -406,7 +424,7 @@ extern "C" int bimamba_layer_fwd_varlen(const bimamba_layer_desc* d, const int32
   k.out = mo;
   k.workspace = ws + c.block;
   k.workspace_bytes = d->workspace_bytes - c.block;
-  BIMAMBA_TRY(bimamba_block_fwd_varlen(&k, seqlens, stream));
+  BIMAMBA_TRY(bimamba_block_fwd_varlen_train(&k, seqlens, stream));
   // norm2 (:482)
   BIMAMBA_TRY(bimamba_layernorm_fwd(mo, d->norm2_w, d->norm2_b, mn, mean2, rstd2, M, dm, d->eps2, cd, cd, stream));
   // feed-forward + residual (:483-485): weights cast (and transposed for the backward), two products with the bias and
@@ -421,6 +439,13 @@ extern "C" int bimamba_layer_fwd_varlen(const bimamba_layer_desc* d, const int32
 }
 
 extern "C" int bimamba_layer_bwd(const bimamba_layer_desc* d, const bimamba_layer_grads* g, bimamba_stream_t stream) {
+  return bimamba_layer_bwd_varlen(d, g, nullptr, stream);
+}
+
+// seqlens != NULL: the backward of bimamba_layer_fwd_varlen_train; the block's backward walks each utterance's frames.
+// The norms and the feed-forward are per row: for the masked contract dout must be zero at padded frames.
+extern "C" int bimamba_layer_bwd_varlen(const bimamba_layer_desc* d, const bimamba_layer_grads* g, const int32_t* seqlens,
+                                        bimamba_stream_t stream) {
   int rc = check_layer(d);
   if (rc) return rc;
   if (!g) { set_err("layer_bwd: null gradient descriptor"); return -1; }
@@ -476,7 +501,7 @@ extern "C" int bimamba_layer_bwd(const bimamba_layer_desc* d, const bimamba_laye
   kg.dx = dxn;
   kg.workspace = bs + w.block;
   kg.workspace_bytes = g->workspace_bytes - w.block;
-  BIMAMBA_TRY(bimamba_block_bwd(&k, &kg, stream));
+  BIMAMBA_TRY(bimamba_block_bwd_varlen(&k, &kg, seqlens, stream));
   // norm1 backward + the residual branch's gradient
   BIMAMBA_TRY(bimamba_layernorm_bwd(d->x, dxn, d->norm1_w, mean1, rstd1, g->dout, g->dx, ln_part, M, dm, xd, cd, stream));
   BIMAMBA_TRY(bimamba_reduce_partials(ln_part, g->dnorm1, 1, w.ln_blocks, 2 * dm, 0, 2 * dm, 0, BIMAMBA_F32, 0, stream));

@@ -138,15 +138,19 @@ conv_fwd_kernel(const T* __restrict__ x, const float* __restrict__ w, const floa
 //   dw[k]   += sum_t g_0[t] x[t-H+k] + g_1[t] x[t+H-k];   dbias += sum_t g_0[t] + g_1[t]
 // from shared memory.  dw / dbias leave as one partial row per CTA (fixed-order reduction afterwards); the sum
 // of the two directions' gate gradients dz is folded into the same pass (global -> global, coalesced).
+// kVar (both backward kernels): the mirror of the masked forward.  Frames t >= len_b = clamp(seqlens[b], 0, L) of x and
+// dout are never loaded (they read as zero), so the padded outputs contribute nothing and the reverse direction's taps
+// past len_b add nothing to dw or dbias; dx and the folded dz are written as zeros at padded frames.
 constexpr int kBwdT = 16;
 constexpr int kBwdC = 64;
 
-template <typename T, int K>
+template <typename T, int K, bool kVar>
 __global__ void __launch_bounds__(kConvThreads)
 conv_bwd_tile_kernel(const T* __restrict__ x, const float* __restrict__ w, const float* __restrict__ bias,
                      const T* __restrict__ dout, T* __restrict__ dx, const T* __restrict__ dz_in, T* __restrict__ dz_out,
                      float* __restrict__ part, int batch, int ndir, int dim, int L, int64_t x_bs, int64_t x_ts,
-                     int64_t g_bs, int64_t g_ds, int64_t g_ts, int64_t dx_bs, int64_t dx_ts, int silu, int vec) {
+                     int64_t g_bs, int64_t g_ds, int64_t g_ts, int64_t dx_bs, int64_t dx_ts, int silu, int vec,
+                     const int32_t* __restrict__ seqlens) {
   pdl_prologue();
   constexpr int H = K - 1;
   constexpr int XR = kBwdT + 4 * H, GR = kBwdT + 2 * H;   // rows of the x and g tiles
@@ -163,6 +167,7 @@ conv_bwd_tile_kernel(const T* __restrict__ x, const float* __restrict__ w, const
   const int c0 = ct * kBwdC, t0 = tt * kBwdT;
   const T* xb = x + (int64_t)b * x_bs;
   const T* gb = dout + (int64_t)b * g_bs;
+  const int Lv = kVar ? min(max(__ldg(seqlens + b), 0), L) : L;   // frames that exist
 
   // ---- stage: x rows [t0-2H, t0+T+2H), g rows [t0-H, t0+T+H) of both directions (zero outside [0, L) x [0, dim))
   if (vec) {
@@ -170,14 +175,14 @@ conv_bwd_tile_kernel(const T* __restrict__ x, const float* __restrict__ w, const
     for (int e = tid; e < XR * VPR; e += kConvThreads) {
       const int r = e / VPR, v = e - r * VPR;
       const int t = t0 - 2 * H + r, c = c0 + v * kV;
-      const bool ok = t >= 0 && t < L && c < dim;
+      const bool ok = t >= 0 && t < Lv && c < dim;
       cp_async16(s_xraw + r * kBwdC + v * kV, ok ? xb + (int64_t)t * x_ts + c : xb, ok);
     }
     for (int e = tid; e < 2 * GR * VPR; e += kConvThreads) {
       const int dsel = e / (GR * VPR), rr = e - dsel * GR * VPR;
       const int r = rr / VPR, v = rr - r * VPR;
       const int t = t0 - H + r, c = c0 + v * kV;
-      const bool ok = t >= 0 && t < L && c < dim && dsel < ndir;
+      const bool ok = t >= 0 && t < Lv && c < dim && dsel < ndir;
       cp_async16(s_graw + (dsel * GR + r) * kBwdC + v * kV, ok ? gb + (int64_t)dsel * g_ds + (int64_t)t * g_ts + c : gb, ok);
     }
     cp_async_commit();
@@ -186,13 +191,13 @@ conv_bwd_tile_kernel(const T* __restrict__ x, const float* __restrict__ w, const
     for (int e = tid; e < XR * kBwdC; e += kConvThreads) {
       const int r = e / kBwdC, cc = e - r * kBwdC;
       const int t = t0 - 2 * H + r, c = c0 + cc;
-      s_xraw[e] = (t >= 0 && t < L && c < dim) ? xb[(int64_t)t * x_ts + c] : from_f<T>(0.f);
+      s_xraw[e] = (t >= 0 && t < Lv && c < dim) ? xb[(int64_t)t * x_ts + c] : from_f<T>(0.f);
     }
     for (int e = tid; e < 2 * GR * kBwdC; e += kConvThreads) {
       const int dsel = e / (GR * kBwdC), rr = e - dsel * GR * kBwdC;
       const int r = rr / kBwdC, cc = rr - r * kBwdC;
       const int t = t0 - H + r, c = c0 + cc;
-      s_graw[e] = (t >= 0 && t < L && c < dim && dsel < ndir) ? gb[(int64_t)dsel * g_ds + (int64_t)t * g_ts + c] : from_f<T>(0.f);
+      s_graw[e] = (t >= 0 && t < Lv && c < dim && dsel < ndir) ? gb[(int64_t)dsel * g_ds + (int64_t)t * g_ts + c] : from_f<T>(0.f);
     }
   }
   __syncthreads();
@@ -247,11 +252,15 @@ conv_bwd_tile_kernel(const T* __restrict__ x, const float* __restrict__ w, const
       for (int k = 0; k < K; ++k)
         dwl[k] += g0 * s_x[(i + 2 * H - H + k) * kBwdC + cc] + g1 * s_x[(i + 2 * H + H - k) * kBwdC + cc];
       if (c < dim) {
-        dxb[(int64_t)tau * dx_ts + c] = from_f<T>(acc);
+        const bool pad = kVar && tau >= Lv;
+        dxb[(int64_t)tau * dx_ts + c] = from_f<T>(pad ? 0.f : acc);
         if (dz_in) {
-          const T* zi = dz_in + (int64_t)b * g_bs + (int64_t)tau * g_ts + c;
-          float zz = to_f(zi[0]);
-          if (ndir > 1) zz += to_f(zi[g_ds]);
+          float zz = 0.f;
+          if (!pad) {
+            const T* zi = dz_in + (int64_t)b * g_bs + (int64_t)tau * g_ts + c;
+            zz = to_f(zi[0]);
+            if (ndir > 1) zz += to_f(zi[g_ds]);
+          }
           dz_out[(int64_t)b * dx_bs + (int64_t)tau * dx_ts + c] = from_f<T>(zz);
         }
       }
@@ -337,12 +346,13 @@ colsum_kernel(const T* __restrict__ x, float* __restrict__ part, int64_t rows, i
 // taps of pre_fwd[tau+3] and of pre_rev[tau].  Everything is read straight from global memory in 8/16-byte row
 // vectors (consecutive threads = consecutive channels), nothing goes through shared memory: ~65 instructions per
 // (step, channel) against ~230 for the tile kernel above, which stays as the fallback for ragged shapes.
-template <typename T>
+template <typename T, bool kVar>
 __global__ void __launch_bounds__(kConvThreads)
 conv_bwd_seg_kernel(const T* __restrict__ x, const float* __restrict__ w, const float* __restrict__ bias,
                     const T* __restrict__ dout, T* __restrict__ dx, const T* __restrict__ dz_in, T* __restrict__ dz_out,
                     float* __restrict__ part, int batch, int ndir, int dim, int L, int64_t x_bs, int64_t x_ts,
-                    int64_t g_bs, int64_t g_ds, int64_t g_ts, int64_t dx_bs, int64_t dx_ts, int silu) {
+                    int64_t g_bs, int64_t g_ds, int64_t g_ts, int64_t dx_bs, int64_t dx_ts, int silu,
+                    const int32_t* __restrict__ seqlens) {
   pdl_prologue();
   constexpr int K = 4, H = 3, V = 4;
   const int nvec = dim / V;
@@ -354,6 +364,7 @@ conv_bwd_seg_kernel(const T* __restrict__ x, const float* __restrict__ w, const 
   const int seg = (int)((gid / nvec) % nseg);
   const int b = (int)(gid / ((int64_t)nvec * nseg));
   const int c = cv * V, t0 = seg * kBwdT, t1 = min(L, t0 + kBwdT);
+  const int Lv = kVar ? min(max(__ldg(seqlens + b), 0), L) : L;   // frames that exist
   const T* xb = x + (int64_t)b * x_bs + c;
   const T* g0b = dout + (int64_t)b * g_bs + c;
   const T* g1b = ndir > 1 ? g0b + g_ds : nullptr;
@@ -383,7 +394,7 @@ conv_bwd_seg_kernel(const T* __restrict__ x, const float* __restrict__ w, const 
       gr[j][v] = 0.f;
     }
   auto ldx = [&](int t, float (&o)[V]) {
-    if (t >= 0 && t < L) load_row<T, V>(xb + (int64_t)t * x_ts, o);
+    if (t >= 0 && t < Lv) load_row<T, V>(xb + (int64_t)t * x_ts, o);
     else {
 #pragma unroll
       for (int v = 0; v < V; ++v) o[v] = 0.f;
@@ -408,8 +419,8 @@ conv_bwd_seg_kernel(const T* __restrict__ x, const float* __restrict__ w, const 
     ldx(tau + H, xw[K - 1]);
     const int tf = tau + H;                    // time of the forward-direction value made in this iteration
     float d0[V], d1[V];
-    const bool f_in = tf < L;                  // tf >= t0 - 0 >= 0 always
-    const bool r_in = tau >= 0;                // tau < t1 <= L always
+    const bool f_in = tf < Lv;                 // tf >= t0 - 0 >= 0 always
+    const bool r_in = tau >= 0 && (!kVar || tau < Lv);   // tau < t1 <= L always
     if (f_in) load_row<T, V>(g0b + (int64_t)tf * g_ts, d0);
     if (r_in && g1b) load_row<T, V>(g1b + (int64_t)tau * g_ts, d1);
 #pragma unroll
@@ -444,16 +455,21 @@ conv_bwd_seg_kernel(const T* __restrict__ x, const float* __restrict__ w, const 
           acc = fmaf(wk[v][k], gf[K - 1 - k][v], acc);   // g_fwd[tau+3-k]
           acc = fmaf(wk[v][k], gr[k][v], acc);           // g_rev[tau-3+k]
         }
-        o[v] = acc;
+        o[v] = (kVar && tau >= Lv) ? 0.f : acc;
       }
       store_row<T, V>(dxb + (int64_t)tau * dx_ts, o);
       if (z0b) {
         float za[V], zb[V];
-        load_row<T, V>(z0b + (int64_t)tau * g_ts, za);
-        if (ndir > 1) {
-          load_row<T, V>(z0b + g_ds + (int64_t)tau * g_ts, zb);
+        if (kVar && tau >= Lv) {
 #pragma unroll
-          for (int v = 0; v < V; ++v) za[v] += zb[v];
+          for (int v = 0; v < V; ++v) za[v] = 0.f;
+        } else {
+          load_row<T, V>(z0b + (int64_t)tau * g_ts, za);
+          if (ndir > 1) {
+            load_row<T, V>(z0b + g_ds + (int64_t)tau * g_ts, zb);
+#pragma unroll
+            for (int v = 0; v < V; ++v) za[v] += zb[v];
+          }
         }
         store_row<T, V>(zob + (int64_t)tau * dx_ts, za);
       }
@@ -486,11 +502,11 @@ static void launch_conv_fwd(const void* x, const float* w, const float* bias, vo
   }
 }
 
-template <typename T>
+template <typename T, bool kVar>
 static void launch_conv_bwd(const void* x, const float* w, const float* bias, const void* dout, void* dx,
                             const void* dz_in, void* dz_out, float* part, int batch, int ndir, int dim, int L, int width,
                             int64_t x_bs, int64_t x_ts, int64_t g_bs, int64_t g_ds, int64_t g_ts, int64_t dx_bs,
-                            int64_t dx_ts, int silu, int vec, cudaStream_t st) {
+                            int64_t dx_ts, int silu, int vec, const int32_t* seqlens, cudaStream_t st) {
   const int nct = (dim + kBwdC - 1) / kBwdC, ntt = conv_bwd_time_tiles(L);
   const unsigned blocks = (unsigned)((int64_t)batch * ntt * nct);
   const T* xp = reinterpret_cast<const T*>(x);
@@ -499,9 +515,9 @@ static void launch_conv_bwd(const void* x, const float* w, const float* bias, co
   T* dxp = reinterpret_cast<T*>(dx);
   T* zo = reinterpret_cast<T*>(dz_out);
   switch (width) {
-    case 2: launch_k(conv_bwd_tile_kernel<T, 2>, blocks, kConvThreads, 0, st, xp, w, bias, gp, dxp, zi, zo, part, batch, ndir, dim, L, x_bs, x_ts, g_bs, g_ds, g_ts, dx_bs, dx_ts, silu, vec); break;
-    case 3: launch_k(conv_bwd_tile_kernel<T, 3>, blocks, kConvThreads, 0, st, xp, w, bias, gp, dxp, zi, zo, part, batch, ndir, dim, L, x_bs, x_ts, g_bs, g_ds, g_ts, dx_bs, dx_ts, silu, vec); break;
-    default: launch_k(conv_bwd_tile_kernel<T, 4>, blocks, kConvThreads, 0, st, xp, w, bias, gp, dxp, zi, zo, part, batch, ndir, dim, L, x_bs, x_ts, g_bs, g_ds, g_ts, dx_bs, dx_ts, silu, vec); break;
+    case 2: launch_k(conv_bwd_tile_kernel<T, 2, kVar>, blocks, kConvThreads, 0, st, xp, w, bias, gp, dxp, zi, zo, part, batch, ndir, dim, L, x_bs, x_ts, g_bs, g_ds, g_ts, dx_bs, dx_ts, silu, vec, seqlens); break;
+    case 3: launch_k(conv_bwd_tile_kernel<T, 3, kVar>, blocks, kConvThreads, 0, st, xp, w, bias, gp, dxp, zi, zo, part, batch, ndir, dim, L, x_bs, x_ts, g_bs, g_ds, g_ts, dx_bs, dx_ts, silu, vec, seqlens); break;
+    default: launch_k(conv_bwd_tile_kernel<T, 4, kVar>, blocks, kConvThreads, 0, st, xp, w, bias, gp, dxp, zi, zo, part, batch, ndir, dim, L, x_bs, x_ts, g_bs, g_ds, g_ts, dx_bs, dx_ts, silu, vec, seqlens); break;
   }
 }
 
@@ -562,6 +578,17 @@ extern "C" int bimamba_causal_conv1d_bwd(const void* x, const float* weight, con
                                          int seqlen, int width, int64_t x_bs, int64_t x_ts, int64_t dout_bs,
                                          int64_t dout_ds, int64_t dout_ts, int64_t dx_bs, int64_t dx_ts, int dtype,
                                          int flags, bimamba_stream_t stream) {
+  return bimamba_causal_conv1d_bwd_varlen(x, weight, bias, dout, dx, dz_in, dz_out, dwb_part, nullptr, batch, ndir, dim,
+                                          seqlen, width, x_bs, x_ts, dout_bs, dout_ds, dout_ts, dx_bs, dx_ts, dtype, flags,
+                                          stream);
+}
+
+extern "C" int bimamba_causal_conv1d_bwd_varlen(const void* x, const float* weight, const float* bias, const void* dout,
+                                                void* dx, const void* dz_in, void* dz_out, float* dwb_part,
+                                                const int32_t* seqlens, int batch, int ndir, int dim, int seqlen, int width,
+                                                int64_t x_bs, int64_t x_ts, int64_t dout_bs, int64_t dout_ds,
+                                                int64_t dout_ts, int64_t dx_bs, int64_t dx_ts, int dtype, int flags,
+                                                bimamba_stream_t stream) {
   if (batch == 0 || seqlen == 0) return 0;
   if (!x || !weight || !dout || !dx || !dwb_part) { set_err("conv bwd: null operand"); return -1; }
   if ((dz_in == nullptr) != (dz_out == nullptr)) { set_err("conv bwd: dz_in and dz_out go together"); return -1; }
@@ -579,19 +606,23 @@ extern "C" int bimamba_causal_conv1d_bwd(const void* x, const float* weight, con
   if (seg4) {
     const int64_t total = (int64_t)batch * conv_bwd_time_tiles(seqlen) * (dim / 4);
     const unsigned blocks = (unsigned)((total + kConvThreads - 1) / kConvThreads);
-#define CONV_SEG(T) launch_k(conv_bwd_seg_kernel<T>, blocks, kConvThreads, 0, st, reinterpret_cast<const T*>(x), weight, bias, reinterpret_cast<const T*>(dout), reinterpret_cast<T*>(dx), reinterpret_cast<const T*>(dz_in), reinterpret_cast<T*>(dz_out), dwb_part, batch, ndir, dim, seqlen, x_bs, x_ts, dout_bs, dout_ds, dout_ts, dx_bs, dx_ts, silu)
-    if (dtype == BIMAMBA_F32) CONV_SEG(float);
-    else if (dtype == BIMAMBA_BF16) CONV_SEG(__nv_bfloat16);
-    else CONV_SEG(__half);
+#define CONV_SEG(T, VAR) launch_k(conv_bwd_seg_kernel<T, VAR>, blocks, kConvThreads, 0, st, reinterpret_cast<const T*>(x), weight, bias, reinterpret_cast<const T*>(dout), reinterpret_cast<T*>(dx), reinterpret_cast<const T*>(dz_in), reinterpret_cast<T*>(dz_out), dwb_part, batch, ndir, dim, seqlen, x_bs, x_ts, dout_bs, dout_ds, dout_ts, dx_bs, dx_ts, silu, seqlens)
+#define CONV_SEG2(T) do { if (seqlens) CONV_SEG(T, true); else CONV_SEG(T, false); } while (0)
+    if (dtype == BIMAMBA_F32) CONV_SEG2(float);
+    else if (dtype == BIMAMBA_BF16) CONV_SEG2(__nv_bfloat16);
+    else CONV_SEG2(__half);
+#undef CONV_SEG2
 #undef CONV_SEG
     cudaError_t e2 = cudaGetLastError();
     if (e2 != cudaSuccess) { set_err(cudaGetErrorString(e2)); return (int)e2; }
     return 0;
   }
-#define CONV_BWD(T) launch_conv_bwd<T>(x, weight, bias, dout, dx, dz_in, dz_out, dwb_part, batch, ndir, dim, seqlen, width, x_bs, x_ts, dout_bs, dout_ds, dout_ts, dx_bs, dx_ts, silu, vec, st)
-  if (dtype == BIMAMBA_F32) CONV_BWD(float);
-  else if (dtype == BIMAMBA_BF16) CONV_BWD(__nv_bfloat16);
-  else CONV_BWD(__half);
+#define CONV_BWD(T, VAR) launch_conv_bwd<T, VAR>(x, weight, bias, dout, dx, dz_in, dz_out, dwb_part, batch, ndir, dim, seqlen, width, x_bs, x_ts, dout_bs, dout_ds, dout_ts, dx_bs, dx_ts, silu, vec, seqlens, st)
+#define CONV_BWD2(T) do { if (seqlens) CONV_BWD(T, true); else CONV_BWD(T, false); } while (0)
+  if (dtype == BIMAMBA_F32) CONV_BWD2(float);
+  else if (dtype == BIMAMBA_BF16) CONV_BWD2(__nv_bfloat16);
+  else CONV_BWD2(__half);
+#undef CONV_BWD2
 #undef CONV_BWD
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) { set_err(cudaGetErrorString(e)); return (int)e; }

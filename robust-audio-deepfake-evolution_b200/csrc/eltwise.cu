@@ -204,6 +204,29 @@ __global__ void __launch_bounds__(256) finalize_kernel(const FinalizeArgs a) {
   }
 }
 
+
+// out[b, t, :] = t < len_b ? x[b, t, :] : 0 with len_b = clamp(seqlens[b], 0, T): the frame mask of variable-length
+// training.  Selection, not a product: a padded frame is never loaded, so NaN or huge padding cannot pass.  kVec: rows
+// of 16-byte vectors (channels a multiple of the vector width, aligned bases); out may alias x.
+template <typename T, bool kVec>
+__global__ void __launch_bounds__(256) mask_frames_kernel(const T* x, T* out, const int32_t* __restrict__ seqlens, int T_,
+                                                          int64_t C, int64_t n) {
+  pdl_prologue();
+  constexpr int kV = kVec ? 16 / sizeof(T) : 1;
+  const int64_t nv = n / kV, cv = C / kV;
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < nv; i += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t row = i / cv;
+    const int b = (int)(row / T_), t = (int)(row - (int64_t)b * T_);
+    const bool keep = t < min(max(__ldg(seqlens + b), 0), T_);
+    if constexpr (kVec) {
+      const uint4 v = keep ? *(reinterpret_cast<const uint4*>(x) + i) : make_uint4(0u, 0u, 0u, 0u);
+      *(reinterpret_cast<uint4*>(out) + i) = v;
+    } else {
+      out[i] = keep ? x[i] : from_f<T>(0.f);
+    }
+  }
+}
+
 }  // namespace bimamba
 
 using namespace bimamba;
@@ -351,6 +374,22 @@ extern "C" int bimamba_scale_by(const void* x, const float* g, void* dx, int64_t
   if (!x || !g || !dx || n < 0 || dtype < 0 || dtype > 2) { set_err("scale_by: bad arguments"); return -1; }
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   EW_DISPATCH1(dtype, (launch_k(scale_by_kernel<T>, ew_blocks(n, 1024), 256, 0, st, (const T*)x, g, (T*)dx, n, scale)));
+  cudaError_t e = cudaGetLastError();
+  if (e != cudaSuccess) { set_err(cudaGetErrorString(e)); return (int)e; }
+  return 0;
+}
+
+extern "C" int bimamba_mask_frames(const void* x, void* out, const int32_t* seqlens, int batch, int seqlen, int channels,
+                                   int dtype, bimamba_stream_t stream) {
+  if (batch == 0 || seqlen == 0 || channels == 0) return 0;
+  if (!x || !out || !seqlens) { set_err("mask_frames: null operand"); return -1; }
+  if (batch < 0 || seqlen < 0 || channels < 0 || dtype < 0 || dtype > 2) { set_err("mask_frames: bad sizes"); return -3; }
+  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+  const int64_t n = (int64_t)batch * seqlen * channels;
+  const int kV = dtype == BIMAMBA_F32 ? 4 : 8;
+  const bool vec = channels % kV == 0 && aligned16(x) && aligned16(out);
+  if (vec) EW_DISPATCH1(dtype, (launch_k(mask_frames_kernel<T, true>, ew_blocks(n / kV, 256), 256, 0, st, (const T*)x, (T*)out, seqlens, seqlen, (int64_t)channels, n)));
+  else EW_DISPATCH1(dtype, (launch_k(mask_frames_kernel<T, false>, ew_blocks(n, 256), 256, 0, st, (const T*)x, (T*)out, seqlens, seqlen, (int64_t)channels, n)));
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) { set_err(cudaGetErrorString(e)); return (int)e; }
   return 0;

@@ -122,11 +122,14 @@ head_fwd_kernel(const T* __restrict__ x, const float* __restrict__ gamma, const 
 // forms   ds_t = a_t (df . y_t - df . f),   dy_t = a_t df + ds_t w,   dx_t = LayerNorm backward of dy_t,
 // accumulating dgamma, dbeta, dw_att (and db_att = sum_t ds_t, which is 0 up to rounding) per warp; the eight warps are
 // merged in fixed order into this utterance's partial row; bimamba_reduce_partials sums over the batch.
-template <typename T, int NPL>
+// kVar: both passes run over t < clamp(seqlens[b], 0, L), the frames the variable-length forward pooled; dx is written as
+// zeros at padded frames, and a zero-length utterance gets zero dx and a zero partial row.
+template <typename T, int NPL, bool kVar>
 __global__ void __launch_bounds__(kHeadThreads)
 head_bwd_kernel(const T* __restrict__ x, const float* __restrict__ gamma, const float* __restrict__ beta,
                 const float* __restrict__ w_att, const float* __restrict__ b_att, const float* __restrict__ dfeat,
-                T* __restrict__ dx, float* __restrict__ part /* (batch, 4, C) */, int L, int C, float eps) {
+                T* __restrict__ dx, float* __restrict__ part /* (batch, 4, C) */, int L, int C, float eps,
+                const int32_t* __restrict__ seqlens) {
   pdl_prologue();
   __shared__ float s_m[kHeadWarps], s_l[kHeadWarps];
   __shared__ float s_acc[kHeadWarps][32 * NPL];
@@ -146,6 +149,17 @@ head_bwd_kernel(const T* __restrict__ x, const float* __restrict__ gamma, const 
     acc[i] = 0.f;
   }
   const float ba = b_att ? __ldg(b_att) : 0.f;
+  const int Lb = kVar ? min(max(__ldg(seqlens + b), 0), L) : L;
+  if (kVar) {
+    for (int t = Lb + warp; t < L; t += kHeadWarps) {
+      T* dr = dxb + (int64_t)t * C;
+#pragma unroll
+      for (int i = 0; i < NPL; ++i) {
+        const int c = lane + 32 * i;
+        if (c < C) dr[c] = from_f<T>(0.f);
+      }
+    }
+  }
   // normalised frame in registers; returns the attention logit
   auto frame = [&](int t, float (&v)[NPL], float (&xh)[NPL], float& rs) -> float {
     const T* xr = xb + (int64_t)t * C;
@@ -177,7 +191,7 @@ head_bwd_kernel(const T* __restrict__ x, const float* __restrict__ gamma, const 
   };
   // ---- pass 1: M, denominator, f
   float m = -INFINITY, l = 0.f;
-  for (int t = warp; t < L; t += kHeadWarps) {
+  for (int t = warp; t < Lb; t += kHeadWarps) {
     float v[NPL], xh[NPL], rs;
     const float sc = frame(t, v, xh, rs);
     const float mn = fmaxf(m, sc);
@@ -218,7 +232,7 @@ head_bwd_kernel(const T* __restrict__ x, const float* __restrict__ gamma, const 
   float dga[NPL], dbe[NPL], dwa[NPL], dba = 0.f;
 #pragma unroll
   for (int i = 0; i < NPL; ++i) dga[i] = dbe[i] = dwa[i] = 0.f;
-  for (int t = warp; t < L; t += kHeadWarps) {
+  for (int t = warp; t < Lb; t += kHeadWarps) {
     float v[NPL], xh[NPL], rs;
     const float sc = frame(t, v, xh, rs);
     const float a = ex2_approx((sc - M) * kLog2e) * rden;
@@ -321,24 +335,35 @@ extern "C" int bimamba_head_fwd_varlen(const void* x, const float* gamma, const 
 extern "C" int bimamba_head_pool_bwd(const void* x, const float* gamma, const float* beta, const float* w_att,
                                      const float* b_att, const float* dfeatures, void* dx, float* part, int batch,
                                      int seqlen, int channels, float eps, int dtype, bimamba_stream_t stream) {
+  return bimamba_head_pool_bwd_varlen(x, gamma, beta, w_att, b_att, dfeatures, dx, part, nullptr, batch, seqlen, channels,
+                                      eps, dtype, stream);
+}
+
+extern "C" int bimamba_head_pool_bwd_varlen(const void* x, const float* gamma, const float* beta, const float* w_att,
+                                            const float* b_att, const float* dfeatures, void* dx, float* part,
+                                            const int32_t* seqlens, int batch, int seqlen, int channels, float eps,
+                                            int dtype, bimamba_stream_t stream) {
   if (batch == 0) return 0;
   if (!x || !gamma || !beta || !w_att || !dfeatures || !dx || !part) { set_err("head_pool_bwd: null operand"); return -1; }
   if (batch < 0 || seqlen < 1 || channels < 1 || channels > 256) { set_err("head_pool_bwd: seqlen >= 1, channels 1..256"); return -3; }
   if (dtype < 0 || dtype > 2) { set_err("head_pool_bwd: bad dtype"); return -6; }
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+#define HEAD_BWD1(T, NPL, VAR) launch_k(head_bwd_kernel<T, NPL, VAR>, batch, kHeadThreads, 0, st, (const T*)x, gamma, beta, w_att, b_att, dfeatures, (T*)dx, part, seqlen, channels, eps, seqlens)
 #define HEAD_BWD(T)                                                                                                         \
   do {                                                                                                                      \
-    if (channels <= 160)                                                                                                    \
-      launch_k(head_bwd_kernel<T, 5>, batch, kHeadThreads, 0, st, (const T*)x, gamma, beta, w_att, b_att, dfeatures, (T*)dx, part, \
-                                                            seqlen, channels, eps);                                         \
-    else                                                                                                                    \
-      launch_k(head_bwd_kernel<T, 8>, batch, kHeadThreads, 0, st, (const T*)x, gamma, beta, w_att, b_att, dfeatures, (T*)dx, part, \
-                                                            seqlen, channels, eps);                                         \
+    if (channels <= 160) {                                                                                                  \
+      if (seqlens) HEAD_BWD1(T, 5, true);                                                                                   \
+      else HEAD_BWD1(T, 5, false);                                                                                          \
+    } else {                                                                                                                \
+      if (seqlens) HEAD_BWD1(T, 8, true);                                                                                   \
+      else HEAD_BWD1(T, 8, false);                                                                                          \
+    }                                                                                                                       \
   } while (0)
   if (dtype == BIMAMBA_F32) HEAD_BWD(float);
   else if (dtype == BIMAMBA_BF16) HEAD_BWD(__nv_bfloat16);
   else HEAD_BWD(__half);
 #undef HEAD_BWD
+#undef HEAD_BWD1
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) { set_err(cudaGetErrorString(e)); return (int)e; }
   return 0;

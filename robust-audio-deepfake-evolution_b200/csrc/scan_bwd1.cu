@@ -34,6 +34,11 @@
 //     per-lane assignment of 16-byte cp.async into double buffers one chunk ahead (generic element-wise staging for
 //     tensors that are not 16-byte friendly).
 //   * all element math is branch-free (the softplus / gate / ypre flags select).
+//   * kVar: utterance b walks its own len_b = clamp(seqlens[b], 0, seqlen) steps from its own last chunk (direction 1
+//     from frame len_b - 1), the mirror of the variable-length forward.  Every layout keeps the padded seqlen: the
+//     checkpoint stride ceil(seqlen / 8) and the (B, ngroups, seqlen, ndir, 32) partial rows.  Padded frames of du,
+//     ddelta, dz and of the partial rows are written as zeros (the row sums and the weight-gradient products downstream
+//     run over every row); dout there is never read, and dA / dD / dbias see valid steps only.
 #include "common.cuh"
 
 namespace bimamba {
@@ -63,8 +68,8 @@ struct LaneSmem {
   static_assert(total <= 28160 || (kMode == 2 && sizeof(T) == 4), "8 CTAs per SM");
 };
 
-template <typename T, int kMode>
-__global__ void __launch_bounds__(32, 1) scan_bwd_lane_kernel(const bimamba_scan_desc p) {
+template <typename T, int kMode, bool kVar>
+__global__ void __launch_bounds__(32, 1) scan_bwd_lane_kernel(const bimamba_scan_desc p, const int32_t* __restrict__ seqlens) {
   pdl_prologue();
   extern __shared__ __align__(16) unsigned char smem_raw[];
   using SM = LaneSmem<T, kMode>;
@@ -78,7 +83,8 @@ __global__ void __launch_bounds__(32, 1) scan_bwd_lane_kernel(const bimamba_scan
   const int b = blockIdx.z, dir = blockIdx.y, g = blockIdx.x, d0 = g * G, d = d0 + lane;
   const int ngroups = gridDim.x;
   const bool ok = d < p.dim;
-  const int L = p.seqlen, nsub = (L + kLT - 1) / kLT;
+  const int L = kVar ? min(max(__ldg(seqlens + b), 0), p.seqlen) : p.seqlen, nsub = (L + kLT - 1) / kLT;
+  const int nck = kVar ? (p.seqlen + kLT - 1) / kLT : nsub;   // checkpoint stride (padded length)
   const bool gated = p.z != nullptr, need_yp = gated && p.dz != nullptr;
   const bool softplus = (p.flags & BIMAMBA_FLAG_SOFTPLUS) != 0;
   const int R = expl ? 0 : p.dt_rank;
@@ -97,8 +103,19 @@ __global__ void __launch_bounds__(32, 1) scan_bwd_lane_kernel(const bimamba_scan
   T* gdz = need_yp ? reinterpret_cast<T*>(p.dz) + obase + d : nullptr;
   // partial layout (batch, ngroups, L, ndir, 32): reducing over ngroups leaves rows ordered (b, t, dir)
   const int pb_ts = p.ndir * 2 * kN;
-  float* partB = p.dbc_part + (((int64_t)b * ngroups + g) * L) * pb_ts + dir * 2 * kN;
-  const float* gck = p.ckpt ? p.ckpt + bd * nsub * (int64_t)p.dim * kN : nullptr;
+  float* partB = p.dbc_part + (((int64_t)b * ngroups + g) * (kVar ? p.seqlen : L)) * pb_ts + dir * 2 * kN;
+  const float* gck = p.ckpt ? p.ckpt + bd * nck * (int64_t)p.dim * kN : nullptr;
+  if (kVar) {   // padded frames: zero gradients and zero partial rows (one column per lane: 32 == 2 * kN)
+    for (int t = L; t < p.seqlen; ++t) {
+      const int64_t o = (int64_t)t * p.out_ts;
+      if (ok) {
+        gdu[o] = from_f<T>(0.f);
+        gdd[o] = from_f<T>(0.f);
+        if (gdz) gdz[o] = from_f<T>(0.f);
+      }
+      partB[(int64_t)t * pb_ts + lane] = 0.f;
+    }
+  }
 
   // ---- shared memory carve
   float4* s_ck = reinterpret_cast<float4*>(smem_raw);               // [2][4][NT]  checkpoint (state entering the chunk)
@@ -444,25 +461,26 @@ __global__ void __launch_bounds__(32, 1) scan_bwd_lane_kernel(const bimamba_scan
 
 // group_channels == 32 (checked by the caller): one warp per CTA, one lane per channel.
 template <typename T, int kMode>
-static void launch_lane2(const bimamba_scan_desc* d, cudaStream_t st) {
+static void launch_lane2(const bimamba_scan_desc* d, const int32_t* seqlens, cudaStream_t st) {
   constexpr size_t smem = LaneSmem<T, kMode>::total;
   dim3 grid((d->dim + 31) / 32, d->ndir, d->batch);
-  launch_k(scan_bwd_lane_kernel<T, kMode>, grid, 32, smem, st, *d);
+  if (seqlens) launch_k(scan_bwd_lane_kernel<T, kMode, true>, grid, 32, smem, st, *d, seqlens);
+  else launch_k(scan_bwd_lane_kernel<T, kMode, false>, grid, 32, smem, st, *d, seqlens);
 }
 
 template <typename T>
-static void launch_lane(const bimamba_scan_desc* d, cudaStream_t st) {
+static void launch_lane(const bimamba_scan_desc* d, const int32_t* seqlens, cudaStream_t st) {
   const int mode = d->delta ? 0 : (d->dt_rank <= 12 ? 1 : 2);
-  if (mode == 0) launch_lane2<T, 0>(d, st);
-  else if (mode == 1) launch_lane2<T, 1>(d, st);
-  else launch_lane2<T, 2>(d, st);
+  if (mode == 0) launch_lane2<T, 0>(d, seqlens, st);
+  else if (mode == 1) launch_lane2<T, 1>(d, seqlens, st);
+  else launch_lane2<T, 2>(d, seqlens, st);
 }
 
-void launch_bwd_lane(const bimamba_scan_desc* d, cudaStream_t st) {
+void launch_bwd_lane(const bimamba_scan_desc* d, const int32_t* seqlens, cudaStream_t st) {
   switch (d->io_dtype) {
-    case BIMAMBA_F32: launch_lane<float>(d, st); break;
-    case BIMAMBA_BF16: launch_lane<__nv_bfloat16>(d, st); break;
-    default: launch_lane<__half>(d, st); break;
+    case BIMAMBA_F32: launch_lane<float>(d, seqlens, st); break;
+    case BIMAMBA_BF16: launch_lane<__nv_bfloat16>(d, seqlens, st); break;
+    default: launch_lane<__half>(d, seqlens, st); break;
   }
 }
 
@@ -473,11 +491,15 @@ int check_desc(const bimamba_scan_desc* d, bool bwd);  // api.cu
 using namespace bimamba;
 
 extern "C" int bimamba_selective_scan_bwd(const bimamba_scan_desc* d, bimamba_stream_t stream) {
+  return bimamba_selective_scan_bwd_varlen(d, nullptr, stream);
+}
+
+extern "C" int bimamba_selective_scan_bwd_varlen(const bimamba_scan_desc* d, const int32_t* seqlens, bimamba_stream_t stream) {
   if (d && (d->batch == 0 || d->seqlen == 0)) return 0;
   int rc = check_desc(d, true);
   if (rc) return rc;
   if (d->group_channels != 32) { set_err("backward group_channels must be 32 (use bimamba_scan_plan)"); return -5; }
-  launch_bwd_lane(d, reinterpret_cast<cudaStream_t>(stream));
+  launch_bwd_lane(d, seqlens, reinterpret_cast<cudaStream_t>(stream));
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) { set_err(cudaGetErrorString(e)); return (int)e; }
   return 0;

@@ -33,7 +33,7 @@ namespace bimamba {
 constexpr int kFwdMaxThreads = 128;
 
 // kMode: 0 = delta given; 1 = fused dt projection with dt_rank <= 12; 2 = dt_rank <= 16.
-// kVar: per-utterance frame counts, as in scan_fwd_warp_kernel (scan_fwd1.cu).
+// kVar: per-utterance frame counts, as in scan_fwd_warp_kernel (scan_fwd1.cu), checkpoint layout included.
 template <typename T, int kMode, bool kGate, bool kVar>
 __global__ void __launch_bounds__(kFwdMaxThreads) scan_fwd_kernel(const bimamba_scan_desc p, const int32_t* __restrict__ seqlens) {
   pdl_prologue();
@@ -44,7 +44,7 @@ __global__ void __launch_bounds__(kFwdMaxThreads) scan_fwd_kernel(const bimamba_
   const int b = blockIdx.z, dir = blockIdx.y, d0 = blockIdx.x * G, d = d0 + tid;
   const bool ok = d < p.dim;
   const int L = kVar ? min(max(__ldg(seqlens + b), 0), p.seqlen) : p.seqlen;
-  const int nck = (L + kT - 1) / kT, nckpt = (L + BIMAMBA_CKPT - 1) / BIMAMBA_CKPT;
+  const int nck = (L + kT - 1) / kT, nckpt = ((kVar ? p.seqlen : L) + BIMAMBA_CKPT - 1) / BIMAMBA_CKPT;
   const bool softplus = (p.flags & BIMAMBA_FLAG_SOFTPLUS) != 0;
   const int R = expl ? 0 : p.dt_rank;
 
@@ -54,7 +54,7 @@ __global__ void __launch_bounds__(kFwdMaxThreads) scan_fwd_kernel(const bimamba_
   const T* gbc = reinterpret_cast<const T*>(p.bc) + (int64_t)b * p.bc_bs + (int64_t)dir * p.bc_ds;
   const T* gdtr = expl ? nullptr : reinterpret_cast<const T*>(p.dtr) + (int64_t)b * p.dtr_bs + (int64_t)dir * p.dtr_ds;
   const int64_t obase = (int64_t)b * p.out_bs + (int64_t)dir * p.out_ds;
-  if (kVar && ok) {   // padded frames (the variable-length entry takes no checkpoints)
+  if (kVar && ok) {   // padded frames
     for (int t = L; t < p.seqlen; ++t) {
       const int64_t o = obase + (int64_t)t * p.out_ts + d;
       reinterpret_cast<T*>(p.out)[o] = from_f<T>(0.f);
@@ -249,11 +249,8 @@ extern "C" int bimamba_selective_scan_fwd(const bimamba_scan_desc* d, bimamba_st
   return bimamba_selective_scan_fwd_varlen(d, nullptr, stream);
 }
 
-extern "C" int bimamba_selective_scan_fwd_varlen(const bimamba_scan_desc* d, const int32_t* seqlens, bimamba_stream_t stream) {
-  if (d && (d->batch == 0 || d->seqlen == 0)) return 0;  // empty: nothing to do (pointers may be null)
-  int rc = check_desc(d, false);
-  if (rc) return rc;
-  if (seqlens && d->ckpt) { set_err("scan fwd: checkpoints feed the backward, which has no variable-length form"); return -9; }
+// The kernels after the descriptor check; seqlens may come with checkpoints (the training forward).
+static int scan_fwd_run(const bimamba_scan_desc* d, const int32_t* seqlens, bimamba_stream_t stream) {
   const int G = d->group_channels;
   if (G < 32 || G > kFwdMaxThreads || (G & 31)) { set_err("forward group_channels must be 32, 64, 96 or 128 (use bimamba_scan_plan)"); return -5; }
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
@@ -279,4 +276,20 @@ extern "C" int bimamba_selective_scan_fwd_varlen(const bimamba_scan_desc* d, con
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) { set_err(cudaGetErrorString(e)); return (int)e; }
   return 0;
+}
+
+extern "C" int bimamba_selective_scan_fwd_varlen(const bimamba_scan_desc* d, const int32_t* seqlens, bimamba_stream_t stream) {
+  if (d && (d->batch == 0 || d->seqlen == 0)) return 0;  // empty: nothing to do (pointers may be null)
+  int rc = check_desc(d, false);
+  if (rc) return rc;
+  if (seqlens && d->ckpt) { set_err("scan fwd: checkpoints belong to the training forward (bimamba_selective_scan_fwd_varlen_train)"); return -9; }
+  return scan_fwd_run(d, seqlens, stream);
+}
+
+extern "C" int bimamba_selective_scan_fwd_varlen_train(const bimamba_scan_desc* d, const int32_t* seqlens,
+                                                       bimamba_stream_t stream) {
+  if (d && (d->batch == 0 || d->seqlen == 0)) return 0;
+  int rc = check_desc(d, false);
+  if (rc) return rc;
+  return scan_fwd_run(d, seqlens, stream);
 }

@@ -11,7 +11,8 @@ namespace bimamba {
 constexpr int kF1G = 32;
 
 // kVar: utterance b walks its own len_b = clamp(seqlens[b], 0, seqlen) steps (direction 1 starts at len_b - 1) and the
-// padded frames len_b .. seqlen-1 of out (and ypre) are written as zeros.
+// padded frames len_b .. seqlen-1 of out (and ypre) are written as zeros.  Checkpoint chunk c holds the state entering
+// scan steps 8c .. 8c+7 of the utterance; the checkpoint stride stays ceil(seqlen / 8) of the padded length.
 template <typename T, int kMode, bool kGate, bool kVar>
 __global__ void __launch_bounds__(kF1G) scan_fwd_warp_kernel(const bimamba_scan_desc p, const int32_t* __restrict__ seqlens) {
   pdl_prologue();
@@ -25,7 +26,7 @@ __global__ void __launch_bounds__(kF1G) scan_fwd_warp_kernel(const bimamba_scan_
   const int b = blockIdx.z, dir = blockIdx.y, d0 = blockIdx.x * G, d = d0 + tid;
   const bool ok = d < p.dim;
   const int L = kVar ? min(max(__ldg(seqlens + b), 0), p.seqlen) : p.seqlen;
-  const int nck = (L + kT - 1) / kT, nckpt = (L + BIMAMBA_CKPT - 1) / BIMAMBA_CKPT;
+  const int nck = (L + kT - 1) / kT, nckpt = ((kVar ? p.seqlen : L) + BIMAMBA_CKPT - 1) / BIMAMBA_CKPT;
   const bool softplus = (p.flags & BIMAMBA_FLAG_SOFTPLUS) != 0;
   const int R = expl ? 0 : p.dt_rank;
 
@@ -35,7 +36,7 @@ __global__ void __launch_bounds__(kF1G) scan_fwd_warp_kernel(const bimamba_scan_
   const T* gbc = reinterpret_cast<const T*>(p.bc) + (int64_t)b * p.bc_bs + (int64_t)dir * p.bc_ds;
   const T* gdtr = expl ? nullptr : reinterpret_cast<const T*>(p.dtr) + (int64_t)b * p.dtr_bs + (int64_t)dir * p.dtr_ds;
   const int64_t obase = (int64_t)b * p.out_bs + (int64_t)dir * p.out_ds;
-  if (kVar && ok) {   // padded frames (the variable-length entry takes no checkpoints)
+  if (kVar && ok) {   // padded frames
     for (int t = L; t < p.seqlen; ++t) {
       const int64_t o = obase + (int64_t)t * p.out_ts + d;
       reinterpret_cast<T*>(p.out)[o] = from_f<T>(0.f);

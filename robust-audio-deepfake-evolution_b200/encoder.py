@@ -7,8 +7,8 @@ import torch.nn as nn
 import torch.nn.functional as F
 
 from .mamba_simple import Mamba
-from .ops import (_forward_only, encoder_layer_native, feed_forward_fn, head_fwd, head_pool_fn, layer_norm_fn,
-                  native_layer_ok, seqlens_tensor)
+from .ops import (_check_mask_padding, _forward_only, _wants_grad, encoder_layer_native, feed_forward_fn, head_fwd,
+                  head_pool_fn, layer_norm_fn, mask_frames, native_layer_ok, seqlens_tensor)
 
 
 class PN_BiMambas_Encoder(nn.Module):
@@ -27,26 +27,37 @@ class PN_BiMambas_Encoder(nn.Module):
             nn.Linear(d_model * 4, d_model),
         )
 
-    def forward(self, x, lengths=None):
-        """x (B, T, d_model) -> (B, T, d_model).  lengths (B,) (list, CPU or CUDA tensor; scoring only): per-utterance
-        frame counts of a right-padded x; valid output frames equal the utterance's own, padded ones are unspecified."""
+    def forward(self, x, lengths=None, *, mask_padding=False):
+        """x (B, T, d_model) -> (B, T, d_model).  lengths (B,) (list, CPU or CUDA tensor): per-utterance frame counts of a
+        right-padded x; valid output frames equal the utterance's own, padded ones are unspecified.  Without
+        mask_padding that is scoring only.  mask_padding=True (training): the padded input frames are replaced by zeros
+        and the padded output frames are exactly zero, in the forward and (their gradients) in the backward, so the loss
+        and every gradient are those of each utterance run alone whatever the padding holds."""
+        _check_mask_padding(lengths, mask_padding)
         seqlens = None
         if lengths is not None:
             seqlens = seqlens_tensor(lengths, x.shape[0], x.shape[1], x.device)
-            _forward_only(seqlens, x, *self.parameters())
+            if not mask_padding:
+                _forward_only(seqlens, x, *self.parameters())
         if native_layer_ok(x, self):
             # eager mode: the whole layer in one native call each way (same kernels, same order, same bits; a captured
             # step keeps the sequenced Functions below, which overlap the weight-gradient products on a second stream)
-            return encoder_layer_native(x, self, seqlens)
+            return encoder_layer_native(x, self, seqlens, mask_padding)
+        if mask_padding:
+            x = mask_frames(x, seqlens)
         # :471-472; the residual branch leaves the LayerNorm Function as its second output, so its gradient is added to dx
         # inside the LayerNorm backward kernel (no separate autograd add)
         x_norm, residual = layer_norm_fn(x, self.norm1.weight, self.norm1.bias, self.norm1.eps, with_residual=True)
-        mamba_out = self.mamba.forward_bidirectional(x_norm, seqlens)                                # :473-481 in one fused pass
+        mamba_out = self.mamba.forward_bidirectional(x_norm, seqlens, mask_padding=mask_padding)    # :473-481 in one fused pass
         mamba_out = layer_norm_fn(mamba_out, self.norm2.weight, self.norm2.bias, self.norm2.eps)    # :482
         if isinstance(self.feed_forward[1], nn.GELU) and self.feed_forward[1].approximate == "none":
             l1, l2 = self.feed_forward[0], self.feed_forward[2]
-            return feed_forward_fn(mamba_out, l1.weight, l1.bias, l2.weight, l2.bias, residual=residual)   # :483-485
-        return self.feed_forward(mamba_out) + residual
+            out = feed_forward_fn(mamba_out, l1.weight, l1.bias, l2.weight, l2.bias, residual=residual)   # :483-485
+        else:
+            out = self.feed_forward(mamba_out) + residual
+        # the feed-forward and the norms make padded rows non-zero: without this mask a loss that touches them would
+        # reach the feed-forward's weight gradients
+        return mask_frames(out, seqlens) if mask_padding else out
 
 
 class BiMambaBackend(nn.Module):
@@ -62,28 +73,34 @@ class BiMambaBackend(nn.Module):
         self.dropout = nn.Dropout(0.1)
         self.classifier = nn.Linear(emb_size, 2)
 
-    def forward_features(self, f_fused, lengths=None):
-        """lengths (B,) (list, CPU or CUDA tensor; scoring only): per-utterance frame counts of the right-padded
-        f_fused.  Output frames at padded positions are unspecified."""
+    def forward_features(self, f_fused, lengths=None, *, mask_padding=False):
+        """lengths (B,) (list, CPU or CUDA tensor): per-utterance frame counts of the right-padded f_fused.  Output
+        frames at padded positions are unspecified; with mask_padding=True (training, see PN_BiMambas_Encoder.forward)
+        they are zero."""
+        _check_mask_padding(lengths, mask_padding)
         seqlens = seqlens_tensor(lengths, f_fused.shape[0], f_fused.shape[1], f_fused.device)
         for layer in self.backbone_layers:
-            f_fused = layer(f_fused, seqlens)
+            f_fused = layer(f_fused, seqlens, mask_padding=mask_padding)
         return f_fused
 
-    def forward(self, f_fused, lengths=None):
+    def forward(self, f_fused, lengths=None, *, mask_padding=False):
         """f_fused (B, T, emb) -> (features, logits).  lengths (B,): see forward_features; every utterance is scored
-        as if it ran alone at its own length (net(x, lengths) with x padded on the right)."""
+        as if it ran alone at its own length (net(x, lengths) with x padded on the right).  mask_padding=True trains on
+        such a batch: the loss and every gradient are those of each utterance run alone, summed over utterances."""
+        _check_mask_padding(lengths, mask_padding)
         seqlens = seqlens_tensor(lengths, f_fused.shape[0], f_fused.shape[1], f_fused.device)
-        return backend_head(self, self.forward_features(f_fused, seqlens), seqlens)
+        return backend_head(self, self.forward_features(f_fused, seqlens, mask_padding=mask_padding), seqlens,
+                            mask_padding=mask_padding)
 
 
-def backend_head(m, f_fused, lengths=None):
+def backend_head(m, f_fused, lengths=None, *, mask_padding=False):
     """norm_f -> attention pooling -> dropout -> classifier on a module that carries the reference's attribute names
     (`norm_f`, `attention_pool`, `dropout`, `classifier`; DualStreamSEMamba.py:759-767).  Returns (features, logits).
-    lengths (B,) (list, CPU or CUDA tensor; scoring only): norm, softmax and pooling over each utterance's first
-    lengths[b] frames only."""
+    lengths (B,) (list, CPU or CUDA tensor): norm, softmax and pooling over each utterance's first lengths[b] frames
+    only; scoring only unless mask_padding=True, which also takes the gradient over those frames (zero at the others)."""
+    _check_mask_padding(lengths, mask_padding)
     if lengths is not None:
-        return _backend_head_varlen(m, f_fused, lengths)
+        return _backend_head_varlen(m, f_fused, lengths, mask_padding)
     if not torch.is_grad_enabled() and not m.training and f_fused.shape[-1] <= 256:
         # scoring (src/main.py:958-995): norm_f, attention pooling and the classifier in one launch
         feats, logits = head_fwd(f_fused, m.norm_f.weight, m.norm_f.bias, m.attention_pool.weight,
@@ -101,10 +118,16 @@ def backend_head(m, f_fused, lengths=None):
     return features, m.classifier(features)                                         # :767
 
 
-def _backend_head_varlen(m, f_fused, lengths):
+def _backend_head_varlen(m, f_fused, lengths, mask_padding):
     seqlens = seqlens_tensor(lengths, f_fused.shape[0], f_fused.shape[1], f_fused.device)
-    _forward_only(seqlens, f_fused, *m.norm_f.parameters(), *m.attention_pool.parameters(), *m.classifier.parameters())
-    if f_fused.shape[-1] <= 256:
+    ps = (f_fused, *m.norm_f.parameters(), *m.attention_pool.parameters(), *m.classifier.parameters())
+    if not mask_padding:
+        _forward_only(seqlens, *ps)
+    if f_fused.shape[-1] <= 256 and _wants_grad(*ps):
+        # training: norm_f + attention pooling over the valid frames as one kernel forward and one backward
+        features = head_pool_fn(f_fused, m.norm_f.weight, m.norm_f.bias, m.attention_pool.weight, m.attention_pool.bias,
+                                m.norm_f.eps, seqlens).to(f_fused.dtype)
+    elif f_fused.shape[-1] <= 256:
         feats, logits = head_fwd(f_fused, m.norm_f.weight, m.norm_f.bias, m.attention_pool.weight,
                                  m.attention_pool.bias, m.classifier.weight, m.classifier.bias, m.norm_f.eps, seqlens)
         if not m.training:

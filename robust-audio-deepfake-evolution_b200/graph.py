@@ -43,6 +43,11 @@ class GraphedTrainStep:
     `run(x)` copies x (host-pinned or device) into the static input, replays, and returns the static
     loss tensor (read it with .item() to synchronise).
 
+    With `lengths` (an example (B,) vector of frame counts, see ops.seqlens_tensor) step_fn is called as
+    step_fn(x, lengths) with the lengths in a static int32 device buffer, and run(x, lengths) copies both: one captured
+    training step then serves every mix of utterance lengths padded to the example's shape (variable-length training,
+    e.g. net(x, lengths, mask_padding=True)).
+
     The `warmup` iterations before the capture run real optimizer steps on the example batch (lazy initialisation of
     handles, function attributes and optimizer state must happen outside the capture); with restore_after_warmup
     (default) the parameters and the optimizer state are put back afterwards, so building the runner - e.g. right
@@ -51,9 +56,14 @@ class GraphedTrainStep:
     def __init__(self, step_fn: Callable[[torch.Tensor], torch.Tensor], example: torch.Tensor,
                  zero_grad: Callable[[], None], optimizer: Optional[torch.optim.Optimizer] = None,
                  warmup: int = 3, post_backward: Optional[Callable[[], None]] = None,
-                 capture_error_mode: Optional[str] = None, restore_after_warmup: bool = True):
+                 capture_error_mode: Optional[str] = None, restore_after_warmup: bool = True, lengths=None):
         self.static_x = torch.empty_like(example, device="cuda")
         self.static_x.copy_(example)
+        self.static_lengths = None
+        args = (self.static_x,)
+        if lengths is not None:
+            self.static_lengths = seqlens_tensor(lengths, example.shape[0], example.shape[1], self.static_x.device).clone()
+            args = (self.static_x, self.static_lengths)
         self.optimizer = optimizer
         snap = _snapshot(optimizer) if (optimizer is not None and restore_after_warmup) else None
         side = torch.cuda.Stream()
@@ -61,7 +71,7 @@ class GraphedTrainStep:
         with torch.cuda.stream(side), sequenced_block():   # warm up what the capture records, not the eager fast path
             for _ in range(max(1, warmup)):          # lazy inits (cuBLAS handles, func attributes) happen here
                 zero_grad()
-                loss = step_fn(self.static_x)
+                loss = step_fn(*args)
                 loss.backward()
                 if post_backward is not None:
                     post_backward()
@@ -80,16 +90,21 @@ class GraphedTrainStep:
             capture_error_mode = "thread_local" if dist.is_available() and dist.is_initialized() else "global"
         with torch.cuda.graph(self.graph, capture_error_mode=capture_error_mode):
             zero_grad()
-            self.static_loss = step_fn(self.static_x)
+            self.static_loss = step_fn(*args)
             self.static_loss.backward()
             if post_backward is not None:
                 post_backward()
             if optimizer is not None:
                 optimizer.step()
 
-    def run(self, x: Optional[torch.Tensor] = None) -> torch.Tensor:
+    def run(self, x: Optional[torch.Tensor] = None, lengths=None) -> torch.Tensor:
         if x is not None:
             self.static_x.copy_(x, non_blocking=True)
+        if lengths is not None:
+            if self.static_lengths is None:
+                raise ValueError("this step was captured without lengths")
+            B, T = self.static_x.shape[:2]
+            self.static_lengths.copy_(seqlens_tensor(lengths, B, T, self.static_x.device), non_blocking=True)
         self.graph.replay()
         return self.static_loss
 

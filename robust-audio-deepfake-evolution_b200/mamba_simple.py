@@ -70,11 +70,11 @@ class Mamba(nn.Module):
         self.D._no_weight_decay = True
         self.out_proj = nn.Linear(self.d_inner, self.d_model, bias=False, **factory)
 
-    def _run(self, hidden_states, bidirectional, lengths=None):
+    def _run(self, hidden_states, bidirectional, lengths=None, mask_padding=False):
         return bimamba_inner_fn(
             hidden_states, self.in_proj.weight, self.conv1d.weight, self.conv1d.bias, self.x_proj.weight,
             self.dt_proj.weight, self.dt_proj.bias, self.A_log, self.D, self.out_proj.weight,
-            bidirectional=bidirectional, lengths=lengths)
+            bidirectional=bidirectional, lengths=lengths, mask_padding=mask_padding)
 
     def forward(self, hidden_states, inference_params=None):
         """hidden_states (B, L, d_model) -> (B, L, d_model); one (causal) direction, as upstream."""
@@ -82,11 +82,13 @@ class Mamba(nn.Module):
             raise NotImplementedError("step-wise decoding is not part of the reference's path")
         return self._run(hidden_states, False)
 
-    def forward_bidirectional(self, hidden_states, lengths=None):
+    def forward_bidirectional(self, hidden_states, lengths=None, *, mask_padding=False):
         """M(x) + flip(M(flip(x))) with these weights in one fused pass
         (src/models/DualStreamSEMamba.py:473-481).
 
         lengths (B,) (list, CPU or CUDA tensor; scoring only): utterance b is frames 0 .. lengths[b]-1 of the
         right-padded batch, and its flip is taken over those frames alone, so each valid output frame equals that of
-        the utterance run by itself.  Output frames at padded positions are unspecified."""
-        return self._run(hidden_states, True, lengths)
+        the utterance run by itself.  Output frames at padded positions are unspecified.
+        mask_padding=True (with lengths) trains on the padded batch: padded input frames are replaced by zeros, padded
+        output frames are zero, and the loss and gradients are those of each utterance run alone (bimamba_inner_fn)."""
+        return self._run(hidden_states, True, lengths, mask_padding)

@@ -151,7 +151,46 @@ def seqlens_tensor(lengths, Bsz: int, T: int, device) -> Optional[torch.Tensor]:
 
 def _forward_only(seqlens, *ts) -> None:
     if seqlens is not None and _wants_grad(*ts):
-        raise NotImplementedError("lengths are supported for scoring only: run under torch.no_grad() / inference_mode()")
+        raise NotImplementedError("lengths without mask_padding=True are supported for scoring only: pass "
+                                  "mask_padding=True to train on a right-padded batch, or run under torch.no_grad()")
+
+
+def _check_mask_padding(lengths, mask_padding: bool) -> None:
+    if mask_padding and lengths is None:
+        raise ValueError("mask_padding=True needs lengths (the per-utterance frame counts of the padded batch)")
+
+
+def mask_frames_raw(x: torch.Tensor, seqlens: torch.Tensor, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """(B, T, C) -> a copy (or `out`, which may be x) with the frames t >= seqlens[b] set to zero by selection (padded
+    frames are never read: NaN padding cannot pass).  One launch."""
+    lib = _lib.load()
+    x = x if x.is_contiguous() else x.contiguous()
+    out = torch.empty_like(x) if out is None else out
+    Bsz, T, C_ = x.shape
+    with _timed("mask"):
+        _lib.check(lib.bimamba_mask_frames(_ptr(x), _ptr(out), _ptr(seqlens), Bsz, T, C_, _dt(x), _stream()),
+                   "bimamba_mask_frames")
+    return out
+
+
+class MaskFramesFn(torch.autograd.Function):
+    """The frame mask of variable-length training, forward and backward: padded frames of the value and of its
+    gradient are zero."""
+
+    @staticmethod
+    def forward(ctx, x, seqlens):
+        _require_cuda(x)
+        ctx.seqlens = seqlens
+        return mask_frames_raw(x.detach(), seqlens)
+
+    @staticmethod
+    def backward(ctx, g):
+        return mask_frames_raw(g, ctx.seqlens), None
+
+
+def mask_frames(x: torch.Tensor, seqlens: torch.Tensor) -> torch.Tensor:
+    """x (B, T, C) with the frames at or past each utterance's length zeroed, as an autograd op (seqlens_tensor)."""
+    return MaskFramesFn.apply(x, seqlens)
 
 
 def _f32c(t: Optional[torch.Tensor]) -> Optional[torch.Tensor]:
@@ -189,11 +228,13 @@ def conv_fwd_raw(x, weight, bias, out, silu: bool, seqlens: Optional[torch.Tenso
         _lib.check(rc, "bimamba_causal_conv1d_fwd_varlen")
 
 
-def conv_bwd_raw(x, weight, bias, dout, dx, silu: bool, dz_in=None, dz_out=None, defer: Optional[list] = None):
+def conv_bwd_raw(x, weight, bias, dout, dx, silu: bool, dz_in=None, dz_out=None, defer: Optional[list] = None,
+                 seqlens: Optional[torch.Tensor] = None):
     """dout (B, ndir, L, D) view; dx (B, L, D) (may be a strided view).  Optionally folds the sum of the
     per-direction gate gradients dz_in (same strides as dout) into dz_out (same strides as dx).
     Returns dwb (D, K+1) fp32 [dw | dbias]; with `defer` (a list) its fixed-order sum over the CTAs' partials runs on
-    the side stream and the fork is appended to the list (join() before using dwb)."""
+    the side stream and the fork is appended to the list (join() before using dwb).
+    seqlens: the backward of conv_fwd_raw with the same frame counts; dx and dz_out are zero at padded frames."""
     lib = _lib.load()
     Bsz, L, D = x.shape
     ndir = dout.shape[1]
@@ -207,11 +248,11 @@ def conv_bwd_raw(x, weight, bias, dout, dx, silu: bool, dz_in=None, dz_out=None,
     nsl = lib.bimamba_conv_bwd_slices(Bsz, L, D)
     part = torch.empty((max(nsl, 1), D, K + 1), device=x.device, dtype=torch.float32)
     with _timed("conv_bwd"):
-        rc = lib.bimamba_causal_conv1d_bwd(
-            _ptr(x), _ptr(weight), _ptr(bias), _ptr(dout), _ptr(dx), _ptr(dz_in), _ptr(dz_out), _ptr(part),
+        rc = lib.bimamba_causal_conv1d_bwd_varlen(
+            _ptr(x), _ptr(weight), _ptr(bias), _ptr(dout), _ptr(dx), _ptr(dz_in), _ptr(dz_out), _ptr(part), _ptr(seqlens),
             Bsz, ndir, D, L, K, x.stride(0), x.stride(1), gbs, gds, gts, dx.stride(0), dx.stride(1), _dt(x),
             _lib.FLAG_SILU if silu else 0, _stream())
-        _lib.check(rc, "bimamba_causal_conv1d_bwd")
+        _lib.check(rc, "bimamba_causal_conv1d_bwd_varlen")
     dwb = torch.empty((D, K + 1), device=x.device, dtype=torch.float32)
     if Bsz * L == 0:
         return dwb.zero_()
@@ -258,11 +299,10 @@ def scan_fwd_raw(u, z, delta, bc, dtr, Wdt, A, D, delta_bias, softplus: bool, wa
     """All activations are (B, ndir, L, C) views with unit channel stride (z may be expanded over
     dir).  Returns (out, ckpt, ypre): out / ypre are (B, ndir, L, dim) views of (B, L, ndir, dim).
     seqlens: (B,) int32 device frame counts (seqlens_tensor) or None.  With them each utterance walks its own frames
-    (direction 1 from its last valid one), padded frames of out are zeros, and the serial walk is used: the time-split
-    forward has no variable-length form.  Forward only (want_ckpt must be False)."""
+    (direction 1 from its last valid one), padded frames of out (and ypre) are zeros, and the serial walk is used: the
+    time-split forward has no variable-length form.  With want_ckpt the checkpoints keep the padded layout
+    (ceil(L / 8) per channel) for scan_bwd_raw with the same seqlens."""
     lib = _lib.load()
-    if seqlens is not None and want_ckpt:
-        raise NotImplementedError("variable-length scan is forward-only (no checkpoints for a backward)")
     Bsz, ndir, L, dim = u.shape
     G, ngroups, nchunks = _lib.scan_plan(L, dim, Bsz * ndir, False)
     out = per_dir(Bsz, L, ndir, dim, u.device, u.dtype)
@@ -284,21 +324,23 @@ def scan_fwd_raw(u, z, delta, bc, dtr, Wdt, A, D, delta_bias, softplus: bool, wa
                        "bimamba_selective_scan_fwd_split")
         _lib.launch_count += 1   # two kernels per call
         return out, ckpt, ypre
+    fwd = lib.bimamba_selective_scan_fwd_varlen_train if want_ckpt else lib.bimamba_selective_scan_fwd_varlen
     with _timed("scan_fwd"):
-        _lib.check(lib.bimamba_selective_scan_fwd_varlen(C.byref(d), _ptr(seqlens), _stream()),
-                   "bimamba_selective_scan_fwd_varlen")
+        _lib.check(fwd(C.byref(d), _ptr(seqlens), _stream()), "bimamba_selective_scan_fwd_varlen")
     return out, ckpt, ypre
 
 
 def scan_bwd_raw(u, z, delta, bc, dtr, Wdt, A, D, delta_bias, softplus: bool, dout, ckpt, ypre,
                  dtr_padded: bool = False, bc_out_dtype=None, defer: Optional[list] = None,
-                 dbc_rows: Optional[torch.Tensor] = None):
+                 dbc_rows: Optional[torch.Tensor] = None, seqlens: Optional[torch.Tensor] = None):
     """Returns (du, ddelta, dz, dbc, dA, dD, dbias): du / ddelta / dz are (B, ndir, L, dim) views of
     (B, L, ndir, dim) storage; dbc is (B, ndir, L, 32) = [dB | dC] likewise; dA (dim, N), dD, dbias (dim).
     With `defer` (a list) the parameter-gradient sums dA / dD / dbias are enqueued on the side stream and the fork is
     appended to the list: the caller must join() it before using them.
     With `dbc_rows` (a (B*L*ndir, >= 32) row matrix, rows ordered (b, t, dir)) the group sum of [dB | dC] is written
-    into its first 32 columns and the returned dbc is None."""
+    into its first 32 columns and the returned dbc is None.
+    seqlens: the backward of scan_fwd_raw with the same frame counts: du, ddelta, dz and [dB | dC] are zero at padded
+    frames, dout there is never read, and dA / dD / dbias sum over valid steps only."""
     lib = _lib.load()
     Bsz, ndir, L, dim = u.shape
     N = A.shape[1]
@@ -324,7 +366,8 @@ def scan_bwd_raw(u, z, delta, bc, dtr, Wdt, A, D, delta_bias, softplus: bool, do
     d.du, d.ddelta, d.dz = _ptr(du), _ptr(ddelta), _ptr(dz)
     d.dbc_part, d.dA_part, d.dD_part, d.dbias_part = _ptr(dbc_part), _ptr(dA_part), _ptr(dD_part), _ptr(db_part)
     with _timed("scan_bwd"):
-        _lib.check(lib.bimamba_selective_scan_bwd(C.byref(d), _stream()), "bimamba_selective_scan_bwd")
+        _lib.check(lib.bimamba_selective_scan_bwd_varlen(C.byref(d), _ptr(seqlens), _stream()),
+                   "bimamba_selective_scan_bwd_varlen")
 
     if dbc_rows is not None:
         dbc = None
@@ -820,7 +863,7 @@ class HeadPoolFn(torch.autograd.Function):
     launch backward (+ the fixed-order sum of the per-utterance parameter-gradient rows)."""
 
     @staticmethod
-    def forward(ctx, x, norm_w, norm_b, att_w, att_b, eps, needs_bwd=True):
+    def forward(ctx, x, norm_w, norm_b, att_w, att_b, eps, needs_bwd=True, seqlens=None):
         _require_cuda(x, norm_w, norm_b, att_w, att_b)
         lib = _lib.load()
         xc = x.detach()
@@ -833,10 +876,12 @@ class HeadPoolFn(torch.autograd.Function):
         gw, gb, aw, ab = _f32c(norm_w), _f32c(norm_b), _f32c(att_w).reshape(-1), _f32c(att_b)
         feats = torch.empty((Bsz, C_), device=x.device, dtype=torch.float32)
         with _timed("head_fwd"):
-            _lib.check(lib.bimamba_head_fwd(_ptr(xc), _ptr(gw), _ptr(gb), _ptr(aw), _ptr(ab), None, None, _ptr(feats), None,
-                                            Bsz, T, C_, 0, float(eps), _dt(xc), _stream()), "bimamba_head_fwd")
+            _lib.check(lib.bimamba_head_fwd_varlen(_ptr(xc), _ptr(gw), _ptr(gb), _ptr(aw), _ptr(ab), None, None, _ptr(feats),
+                                                   None, _ptr(seqlens), Bsz, T, C_, 0, float(eps), _dt(xc), _stream()),
+                       "bimamba_head_fwd_varlen")
         if needs_bwd:
             ctx.save_for_backward(xc, gw, gb, aw, ab if ab is not None else torch.empty(0))
+            ctx.seqlens = seqlens
             ctx.meta = (eps, x.dtype, norm_w.dtype, norm_b.dtype, att_w.dtype, tuple(att_w.shape),
                         None if att_b is None else att_b.dtype)
         return feats
@@ -852,17 +897,19 @@ class HeadPoolFn(torch.autograd.Function):
         dx = torch.empty_like(xc)
         part = torch.empty((Bsz, 4, C_), device=xc.device, dtype=torch.float32)
         with _timed("head_bwd"):
-            _lib.check(lib.bimamba_head_pool_bwd(_ptr(xc), _ptr(gw), _ptr(gb), _ptr(aw), _ptr(ab), _ptr(df), _ptr(dx),
-                                                 _ptr(part), Bsz, T, C_, float(eps), _dt(xc), _stream()),
-                       "bimamba_head_pool_bwd")
+            _lib.check(lib.bimamba_head_pool_bwd_varlen(_ptr(xc), _ptr(gw), _ptr(gb), _ptr(aw), _ptr(ab), _ptr(df), _ptr(dx),
+                                                        _ptr(part), _ptr(ctx.seqlens), Bsz, T, C_, float(eps), _dt(xc),
+                                                        _stream()), "bimamba_head_pool_bwd_varlen")
         sums = torch.empty((4, C_), device=xc.device, dtype=torch.float32)
         reduce_raw(part, sums, groups=1, rows=Bsz, cols=4 * C_, part_gs=0, row_stride=4 * C_, out_gs=0)
         return (dx.to(xdt), sums[0].to(nwdt), sums[1].to(nbdt), sums[2].reshape(awshape).to(awdt),
-                None if abdt is None else sums[3, :1].to(abdt), None, None)
+                None if abdt is None else sums[3, :1].to(abdt), None, None, None)
 
 
-def head_pool_fn(x, norm_w, norm_b, att_w, att_b, eps=1e-5):
-    return HeadPoolFn.apply(x, norm_w, norm_b, att_w, att_b, eps, _wants_grad(x, norm_w, norm_b, att_w, att_b))
+def head_pool_fn(x, norm_w, norm_b, att_w, att_b, eps=1e-5, seqlens=None):
+    """seqlens (seqlens_tensor): pool, and take the gradient of, each utterance's first seqlens[b] frames only; dx is
+    zero at padded frames and a zero-length utterance gets zero features and zero gradients."""
+    return HeadPoolFn.apply(x, norm_w, norm_b, att_w, att_b, eps, _wants_grad(x, norm_w, norm_b, att_w, att_b), seqlens)
 
 
 class LinearFn(torch.autograd.Function):
@@ -1011,6 +1058,7 @@ class BiMambaInnerFn(torch.autograd.Function):
                 ctx.meta = (Bsz, L, ndir, R, x.dtype,
                             tuple(t.dtype for t in (W_in, conv_w, conv_b, W_x, W_dt, b_dt, A_log, Dp, W_out)),
                             tuple(conv_w.shape))
+                ctx.seqlens = seqlens
             return out
 
     @staticmethod
@@ -1042,7 +1090,7 @@ class BiMambaInnerFn(torch.autograd.Function):
             dxdbl = torch.empty((M * ndir, XW), device=xz.device, dtype=cd)   # [dB | dC | ddt_r | 0], rows (b, t, dir)
             du, ddelta, dz, _, dA, dD, dbdt = scan_bwd_raw(
                 xc, z.unsqueeze(1).expand(Bsz, ndir, L, D), None, xd4[..., :2 * N], xd4[..., 2 * N:], Wd32,
-                A32, D32, bdt32, True, dyb, ckpt, ypre, dtr_padded=True, defer=forks, dbc_rows=dxdbl)
+                A32, D32, bdt32, True, dyb, ckpt, ypre, dtr_padded=True, defer=forks, dbc_rows=dxdbl, seqlens=ctx.seqlens)
             # dt_proj (weight gradient in fp32; the data gradient is written next to dB | dC: no concatenation)
             dd2 = rows2d(ddelta)                                              # (M*ndir, D)
             gemm_nt(dd2, WdT, out=dxdbl[:, 2 * N:])                           # (M*ndir, 16)
@@ -1056,7 +1104,8 @@ class BiMambaInnerFn(torch.autograd.Function):
             # conv (writes dx into the x half and dz_fwd + dz_rev into the z half of dxz)
             dxz = torch.empty_like(xz)
             dxz3 = dxz.view(Bsz, L, 2 * D)
-            dwb = conv_bwd_raw(xs, cw32, cb32, dxc4, dxz3[:, :, :D], True, dz_in=dz, dz_out=dxz3[:, :, D:], defer=forks)
+            dwb = conv_bwd_raw(xs, cw32, cb32, dxc4, dxz3[:, :, :D], True, dz_in=dz, dz_out=dxz3[:, :, D:], defer=forks,
+                               seqlens=ctx.seqlens)
             K = cw32.shape[1]
             # in_proj
             with _Fork() as f_in:                                             # in_proj weight gradient || its data gradient
@@ -1140,18 +1189,25 @@ class BiMambaNativeFn(torch.autograd.Function):
 
 
 def bimamba_inner_fn(x, W_in, conv_w, conv_b, W_x, W_dt, b_dt, A_log, Dp, W_out, bidirectional=True,
-                     compute_dtype=None, lengths=None):
+                     compute_dtype=None, lengths=None, *, mask_padding=False):
     """x (B, L, d_model) -> (B, L, d_model).  compute_dtype: activation dtype of the kernels and
     GEMMs (default: the autocast dtype when autocast is on, else x.dtype); scan state is fp32.
     lengths (B,): utterance b is frames 0 .. lengths[b]-1 of the right-padded x (seqlens_tensor); each valid output frame
     equals that of the utterance run alone at its own length, output frames at padded positions are unspecified.
-    Scoring only: with lengths and autograd recording this raises NotImplementedError."""
+    Without mask_padding this is scoring only: with lengths and autograd recording it raises NotImplementedError.
+    mask_padding=True (with lengths) is the training form: the padded frames of x are replaced by zeros (selection, so
+    NaN padding cannot pass), padded output frames are exactly zero, the gradient at padded input frames is zero, and
+    the loss and every gradient are those of each utterance run alone, parameter gradients summed over utterances."""
     if compute_dtype is None:
         compute_dtype = torch.get_autocast_dtype("cuda") if torch.is_autocast_enabled("cuda") else x.dtype
+    _check_mask_padding(lengths, mask_padding)
     seqlens = seqlens_tensor(lengths, x.shape[0], x.shape[1], x.device)
     _require_cuda(x, W_in, conv_w, conv_b, W_x, W_dt, b_dt, A_log, Dp, W_out)
     ps = (x, W_in, conv_w, conv_b, W_x, W_dt, b_dt, A_log, Dp, W_out)
-    _forward_only(seqlens, *ps)
+    if mask_padding:
+        ps = (mask_frames(x, seqlens),) + ps[1:]
+    else:
+        _forward_only(seqlens, *ps)
     fn = BiMambaNativeFn if _native_block_ok(x, W_in, compute_dtype) else BiMambaInnerFn
     return fn.apply(*ps, bool(bidirectional), compute_dtype, _wants_grad(*ps), seqlens)
 
@@ -1195,7 +1251,9 @@ class NativeBlock:
         d.batch, d.seqlen, d.d_model, d.d_inner, d.dt_rank, d.d_conv, d.ndir = Bsz, L, dm, D, R, K, ndir
         d.io_dtype, d.save_for_backward = _dt(x), int(save_for_backward)
         self.desc = d
-        _lib.check(lib.bimamba_block_fwd_varlen(C.byref(d), _ptr(seqlens), _stream()), "bimamba_block_fwd_varlen")
+        self.seqlens = seqlens
+        fwd = lib.bimamba_block_fwd_varlen_train if save_for_backward else lib.bimamba_block_fwd_varlen
+        _lib.check(fwd(C.byref(d), _ptr(seqlens), _stream()), "bimamba_block_fwd_varlen")
         _lib.launch_count += 4           # the call enqueues 5 kernels (3 GEMMs, conv, scan)
 
     def backward(self, dout):
@@ -1217,7 +1275,8 @@ class NativeBlock:
         g.WiT, g.WxpT, g.WoT, g.WdT = _ptr(WiT), _ptr(WxpT), _ptr(WoT), _ptr(WdT)
         (g.dW_in, g.dconv_w, g.dconv_b, g.dW_x, g.dW_dt, g.db_dt, g.dA_log, g.dD, g.dW_out) = [_ptr(t) for t in grads]
         g.workspace, g.workspace_bytes = _ptr(ws), nbytes
-        _lib.check(lib.bimamba_block_bwd(C.byref(self.desc), C.byref(g), _stream()), "bimamba_block_bwd")
+        _lib.check(lib.bimamba_block_bwd_varlen(C.byref(self.desc), C.byref(g), _ptr(self.seqlens), _stream()),
+                   "bimamba_block_bwd_varlen")
         _lib.launch_count += 19          # 20 kernels: 4 + 4 x 2 GEMMs, scan, conv, row sum, 4 partial sums, layout pass
         self._keep = (dout, ws)
         return (dx, *grads)
@@ -1262,7 +1321,9 @@ class NativeLayer:
         d.eps1, d.eps2, d.d_ff, d.x_dtype = float(eps1), float(eps2), dff, _dt(self.x)
         self.desc = d
         self._keep_fwd = (cw32,)
-        _lib.check(lib.bimamba_layer_fwd_varlen(C.byref(d), _ptr(seqlens), _stream()), "bimamba_layer_fwd_varlen")
+        self.seqlens = seqlens
+        fwd = lib.bimamba_layer_fwd_varlen_train if save_for_backward else lib.bimamba_layer_fwd_varlen
+        _lib.check(fwd(C.byref(d), _ptr(seqlens), _stream()), "bimamba_layer_fwd_varlen")
         _lib.launch_count += 11          # 12 kernels: 2 LayerNorm, 5 of the block, 2 weight casts, 2 GEMMs, GELU
 
     def backward(self, dout):
@@ -1287,7 +1348,8 @@ class NativeLayer:
         kg.WiT, kg.WxpT, kg.WoT, kg.WdT = _ptr(WiT), _ptr(WxpT), _ptr(WoT), _ptr(WdT)
         (kg.dW_in, kg.dconv_w, kg.dconv_b, kg.dW_x, kg.dW_dt, kg.db_dt, kg.dA_log, kg.dD, kg.dW_out) = [_ptr(t) for t in mg]
         g.workspace, g.workspace_bytes = _ptr(ws), nbytes
-        _lib.check(lib.bimamba_layer_bwd(C.byref(self.desc), C.byref(g), _stream()), "bimamba_layer_bwd")
+        _lib.check(lib.bimamba_layer_bwd_varlen(C.byref(self.desc), C.byref(g), _ptr(self.seqlens), _stream()),
+                   "bimamba_layer_bwd_varlen")
         _lib.launch_count += 35          # 36 kernels: 20 of the block, 11 of the feed-forward, 2 x 2 of the norms, the cast of dout
         self._keep = (dout, ws)
         return (dx, *lg, *mg)
@@ -1341,12 +1403,17 @@ def native_layer_ok(x, layer) -> bool:
             and m.dt_rank <= MAX_DT_RANK and not torch.cuda.is_current_stream_capturing())
 
 
-def encoder_layer_native(x, layer, seqlens=None):
-    """seqlens: (B,) int32 device frame counts (seqlens_tensor) or None; scoring only."""
+def encoder_layer_native(x, layer, seqlens=None, mask_padding=False):
+    """seqlens: (B,) int32 device frame counts (seqlens_tensor) or None; scoring only unless mask_padding, which masks
+    the layer's input and output (forward and backward, MaskFramesFn) as PN_BiMambas_Encoder.forward does."""
     cd = torch.get_autocast_dtype("cuda") if torch.is_autocast_enabled("cuda") else x.dtype
     m, ff = layer.mamba, layer.feed_forward
     ps = (layer.norm1.weight, layer.norm1.bias, layer.norm2.weight, layer.norm2.bias, ff[0].weight, ff[0].bias,
           ff[2].weight, ff[2].bias, m.in_proj.weight, m.conv1d.weight, m.conv1d.bias, m.x_proj.weight, m.dt_proj.weight,
           m.dt_proj.bias, m.A_log, m.D, m.out_proj.weight)
-    _forward_only(seqlens, x, *ps)
-    return EncoderLayerNativeFn.apply(x, *ps, layer.norm1.eps, layer.norm2.eps, cd, _wants_grad(x, *ps), seqlens)
+    if mask_padding:
+        x = mask_frames(x, seqlens)
+    else:
+        _forward_only(seqlens, x, *ps)
+    out = EncoderLayerNativeFn.apply(x, *ps, layer.norm1.eps, layer.norm2.eps, cd, _wants_grad(x, *ps), seqlens)
+    return mask_frames(out, seqlens) if mask_padding else out
