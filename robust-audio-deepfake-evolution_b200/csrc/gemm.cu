@@ -267,7 +267,8 @@ gemm_nt_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
           if (n + j < N) {
             float v = __uint_as_float(r[j]);
             if (bias != nullptr) v += __ldg(bias + n + j);
-            if (src != nullptr) v += to_f(src[j]);
+            // round the Linear output to TOut before the addend, as the staged epilogue does: same bits on both paths
+            if (src != nullptr) v = to_f(from_f<TOut>(v)) + to_f(src[j]);
             dst[j] = from_f<TOut>(v);
           }
         }

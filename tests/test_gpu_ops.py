@@ -208,7 +208,7 @@ def test_layer_norm(C, dtype, out_dtype):
 
 # ---------------------------------------------------------------- tcgen05 GEMM
 @pytest.mark.parametrize("M,N,K", [(128, 48, 288), (12864, 576, 144), (25728, 48, 288), (12864, 144, 576),
-                                   (201, 288, 48), (1, 16, 8), (300, 41 + 7, 144), (257, 640, 72)])
+                                   (201, 288, 48), (1, 16, 8), (300, 41 + 7, 144), (257, 640, 72), (129, 45, 72)])
 @pytest.mark.parametrize("dtype", [torch.bfloat16, torch.float16])
 def test_gemm_nt_tensor_cores(M, N, K, dtype):
     """nn.Linear products of the block (mamba_block.py:48, :73, :62) on the tcgen05 kernel against an fp64 product
