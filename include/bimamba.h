@@ -180,6 +180,37 @@ int bimamba_selective_scan_bwd_varlen(const bimamba_scan_desc* d, const int32_t*
 int bimamba_mask_frames(const void* x, void* out, const int32_t* seqlens, int batch, int seqlen, int channels, int dtype,
                         bimamba_stream_t stream);
 
+/* ---- Variable-length DualStreamFusion (DualStreamSEMamba.py:580-637 run on each utterance alone).  Two streams, two
+ * length vectors: seqlens_dst (batch) are the WavLM frame counts n1 of a batch padded to dst_frames, seqlens_src the
+ * SincNet frame counts n2 of a batch padded to src_frames (device int32, clamped to [0, frames]).  Activations
+ * (batch, frames, channels) contiguous in `dtype`; arithmetic fp32 with one rounding; frames at or past an utterance's
+ * length are never read and are written as zeros.  NULL operand -1, bad sizes -3, empty batch a no-op 0.
+ *
+ * Interpolation of the projected SincNet branch onto the WavLM frames, per utterance (:601-626, F.interpolate):
+ * n1 == n2 copies (bit-identical), n1 > 4 n2 is nearest, otherwise linear with align_corners=False, on ATen's fp32
+ * index rule (scale = (float)n2 / n1; see DESIGN.md 4.8).  The backward is a gather: each source frame sums the weighted
+ * cotangents of the destination frames that read it in increasing frame order (deterministic). */
+int bimamba_interp_frames_fwd(const void* src, void* dst, const int32_t* seqlens_dst, const int32_t* seqlens_src,
+                              int batch, int dst_frames, int src_frames, int channels, int dtype, bimamba_stream_t stream);
+int bimamba_interp_frames_bwd(const void* ddst, void* dsrc, const int32_t* seqlens_dst, const int32_t* seqlens_src,
+                              int batch, int dst_frames, int src_frames, int channels, int dtype, bimamba_stream_t stream);
+/* SELayer's squeeze (:524-526, AdaptiveAvgPool1d): mean (batch, channels) fp32 = sum_{t < n} x / n in a fixed order;
+ * 0 for a zero-length utterance.  Backward: dx = dmean / n at valid frames. */
+int bimamba_frame_mean(const void* x, float* mean, const int32_t* seqlens, int batch, int seqlen, int channels,
+                       int dtype, bimamba_stream_t stream);
+int bimamba_frame_mean_bwd(const float* dmean, void* dx, const int32_t* seqlens, int batch, int seqlen, int channels,
+                           int dtype, bimamba_stream_t stream);
+/* SELayer's excitation product (:528): y = x * gate[b] (gate (batch, channels) fp32).  Backward in one pass:
+ * dx = dy * gate[b] and dgate_part (batch, nslices, channels) fp32, nslices = bimamba_frame_scale_bwd_slices(seqlen),
+ * the sums of dy * x over each slice's valid frames: finish with bimamba_reduce_partials(groups = batch, rows = nslices,
+ * cols = channels, part_gs = nslices * channels, row_stride = channels, out_gs = channels). */
+int bimamba_frame_scale(const void* x, const float* gate, void* y, const int32_t* seqlens, int batch, int seqlen,
+                        int channels, int dtype, bimamba_stream_t stream);
+int bimamba_frame_scale_bwd_slices(int seqlen);
+int bimamba_frame_scale_bwd(const void* x, const float* gate, const void* dy, void* dx, float* dgate_part,
+                            const int32_t* seqlens, int batch, int seqlen, int channels, int dtype,
+                            bimamba_stream_t stream);
+
 /* Time-parallel forward scan for long sequences at small batches (the scan as an associative operator on pairs,
  * (a2, b2) o (a1, b1) = (a2 a1, a2 b1 + b2); mamba_block.py:92-117 is the serial loop).  Scan time is cut into nseg
  * segments of seg_len steps: a carry pass computes every segment's end state from zero and its decay exponent

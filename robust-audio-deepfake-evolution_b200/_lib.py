@@ -35,6 +35,8 @@ EXPORTS = (
     "bimamba_selective_scan_fwd_varlen_train", "bimamba_selective_scan_bwd_varlen", "bimamba_causal_conv1d_bwd_varlen",
     "bimamba_head_pool_bwd_varlen", "bimamba_block_fwd_varlen_train", "bimamba_block_bwd_varlen",
     "bimamba_layer_fwd_varlen_train", "bimamba_layer_bwd_varlen", "bimamba_mask_frames",
+    "bimamba_interp_frames_fwd", "bimamba_interp_frames_bwd", "bimamba_frame_mean", "bimamba_frame_mean_bwd",
+    "bimamba_frame_scale", "bimamba_frame_scale_bwd_slices", "bimamba_frame_scale_bwd",
 )
 
 
@@ -248,6 +250,20 @@ def load() -> C.CDLL:
         lib.bimamba_layer_bwd_varlen.argtypes = [C.POINTER(LayerDesc), C.POINTER(LayerGrads), vp, vp]
         lib.bimamba_mask_frames.restype = i32
         lib.bimamba_mask_frames.argtypes = [vp, vp, vp, i32, i32, i32, i32, vp]
+        for name in ("bimamba_interp_frames_fwd", "bimamba_interp_frames_bwd"):
+            fn = getattr(lib, name)
+            fn.restype = i32
+            fn.argtypes = [vp, vp, vp, vp, i32, i32, i32, i32, i32, vp]
+        lib.bimamba_frame_mean.restype = i32
+        lib.bimamba_frame_mean.argtypes = [vp, vp, vp, i32, i32, i32, i32, vp]
+        lib.bimamba_frame_mean_bwd.restype = i32
+        lib.bimamba_frame_mean_bwd.argtypes = [vp, vp, vp, i32, i32, i32, i32, vp]
+        lib.bimamba_frame_scale.restype = i32
+        lib.bimamba_frame_scale.argtypes = [vp, vp, vp, vp, i32, i32, i32, i32, vp]
+        lib.bimamba_frame_scale_bwd_slices.restype = i32
+        lib.bimamba_frame_scale_bwd_slices.argtypes = [i32]
+        lib.bimamba_frame_scale_bwd.restype = i32
+        lib.bimamba_frame_scale_bwd.argtypes = [vp, vp, vp, vp, vp, vp, i32, i32, i32, i32, vp]
         got = lib.bimamba_abi_version()
         if got != ABI_VERSION:
             raise RuntimeError(f"libbimamba ABI {got} != expected {ABI_VERSION}; rebuild the library")

@@ -12,7 +12,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libbimamba_sm100.so")
-SOURCES = ("api.cu", "scan_fwd.cu", "scan_fwd1.cu", "scan_fwd_split.cu", "scan_bwd1.cu", "conv.cu", "layernorm.cu", "gemm.cu", "pack.cu", "optim.cu", "head.cu", "eltwise.cu", "block.cu")
+SOURCES = ("api.cu", "scan_fwd.cu", "scan_fwd1.cu", "scan_fwd_split.cu", "scan_bwd1.cu", "conv.cu", "layernorm.cu", "gemm.cu", "pack.cu", "optim.cu", "head.cu", "eltwise.cu", "block.cu", "fusion.cu")
 HEADERS = ("common.cuh", os.path.join("..", "..", "include", "bimamba.h"))
 
 NVCC_FLAGS = [

@@ -193,6 +193,128 @@ def mask_frames(x: torch.Tensor, seqlens: torch.Tensor) -> torch.Tensor:
     return MaskFramesFn.apply(x, seqlens)
 
 
+# ----------------------------------------------------------------------------------------
+# variable-length DualStreamFusion (DualStreamSEMamba.py:601-628 per utterance): interpolation of the projected SincNet
+# branch onto each utterance's WavLM frames, SELayer's masked mean and channel scale.  One launch each way.
+# ----------------------------------------------------------------------------------------
+def _c3(t: torch.Tensor) -> torch.Tensor:
+    t = t.detach()
+    if t.dtype not in _DT:
+        t = t.float()
+    return t if t.is_contiguous() else t.contiguous()
+
+
+class InterpFramesFn(torch.autograd.Function):
+    """src (B, T2, C) -> (B, T1, C): utterance b's first seqlens_src[b] frames interpolated onto seqlens_dst[b] frames
+    (copy, nearest or linear by the reference's rule, chosen per utterance on the device); zero at padded frames."""
+
+    @staticmethod
+    def forward(ctx, src, seqlens_dst, seqlens_src, T1):
+        _require_cuda(src)
+        lib = _lib.load()
+        s = _c3(src)
+        Bsz, T2, C_ = s.shape
+        out = torch.empty((Bsz, T1, C_), device=s.device, dtype=s.dtype)
+        with _timed("interp_fwd"):
+            _lib.check(lib.bimamba_interp_frames_fwd(_ptr(s), _ptr(out), _ptr(seqlens_dst), _ptr(seqlens_src), Bsz, T1, T2,
+                                                     C_, _dt(s), _stream()), "bimamba_interp_frames_fwd")
+        ctx.seqlens = (seqlens_dst, seqlens_src)
+        ctx.meta = (T2, src.dtype)
+        return out
+
+    @staticmethod
+    def backward(ctx, g):
+        lib = _lib.load()
+        T2, sdt = ctx.meta
+        gc = _c3(g)
+        Bsz, T1, C_ = gc.shape
+        dsrc = torch.empty((Bsz, T2, C_), device=gc.device, dtype=gc.dtype)
+        with _timed("interp_bwd"):
+            _lib.check(lib.bimamba_interp_frames_bwd(_ptr(gc), _ptr(dsrc), _ptr(ctx.seqlens[0]), _ptr(ctx.seqlens[1]), Bsz, T1,
+                                                     T2, C_, _dt(gc), _stream()), "bimamba_interp_frames_bwd")
+        return dsrc.to(sdt), None, None, None
+
+
+def interp_frames(src: torch.Tensor, seqlens_dst: torch.Tensor, seqlens_src: torch.Tensor, T1: int) -> torch.Tensor:
+    """(B, T2, C) -> (B, T1, C) per-utterance interpolation (seqlens_tensor for both streams), autograd op."""
+    return InterpFramesFn.apply(src, seqlens_dst, seqlens_src, int(T1))
+
+
+class FrameMeanFn(torch.autograd.Function):
+    """x (B, T, C) -> (B, C) fp32 mean over each utterance's first seqlens[b] frames (0 for a zero-length one)."""
+
+    @staticmethod
+    def forward(ctx, x, seqlens):
+        _require_cuda(x)
+        lib = _lib.load()
+        xc = _c3(x)
+        Bsz, T, C_ = xc.shape
+        mean = torch.empty((Bsz, C_), device=xc.device, dtype=torch.float32)
+        with _timed("frame_mean"):
+            _lib.check(lib.bimamba_frame_mean(_ptr(xc), _ptr(mean), _ptr(seqlens), Bsz, T, C_, _dt(xc), _stream()),
+                       "bimamba_frame_mean")
+        ctx.seqlens = seqlens
+        ctx.meta = (xc.shape, xc.dtype, x.dtype)
+        return mean
+
+    @staticmethod
+    def backward(ctx, g):
+        lib = _lib.load()
+        (Bsz, T, C_), cdt, xdt = ctx.meta
+        g32 = g.detach().to(torch.float32).contiguous()
+        dx = torch.empty((Bsz, T, C_), device=g.device, dtype=cdt)
+        with _timed("frame_mean_bwd"):
+            _lib.check(lib.bimamba_frame_mean_bwd(_ptr(g32), _ptr(dx), _ptr(ctx.seqlens), Bsz, T, C_, _dt(dx), _stream()),
+                       "bimamba_frame_mean_bwd")
+        return dx.to(xdt), None
+
+
+def frame_mean(x: torch.Tensor, seqlens: torch.Tensor) -> torch.Tensor:
+    return FrameMeanFn.apply(x, seqlens)
+
+
+class FrameScaleFn(torch.autograd.Function):
+    """y = x * gate[b] (gate (B, C) fp32) on each utterance's first seqlens[b] frames, zero at padded frames.  Backward in
+    one launch (dx and the fixed-order dgate partials) + the fixed-order sum of the partials."""
+
+    @staticmethod
+    def forward(ctx, x, gate, seqlens):
+        _require_cuda(x, gate)
+        lib = _lib.load()
+        xc, g32 = _c3(x), gate.detach().to(torch.float32).contiguous()
+        Bsz, T, C_ = xc.shape
+        y = torch.empty_like(xc)
+        with _timed("frame_scale"):
+            _lib.check(lib.bimamba_frame_scale(_ptr(xc), _ptr(g32), _ptr(y), _ptr(seqlens), Bsz, T, C_, _dt(xc), _stream()),
+                       "bimamba_frame_scale")
+        ctx.save_for_backward(xc, g32)
+        ctx.seqlens = seqlens
+        ctx.meta = (x.dtype, gate.dtype)
+        return y
+
+    @staticmethod
+    def backward(ctx, dy):
+        xc, g32 = ctx.saved_tensors
+        xdt, gdt = ctx.meta
+        lib = _lib.load()
+        Bsz, T, C_ = xc.shape
+        dyc = dy.detach().to(xc.dtype).contiguous()
+        dx = torch.empty_like(xc)
+        nsl = lib.bimamba_frame_scale_bwd_slices(T)
+        part = torch.empty((Bsz, nsl, C_), device=xc.device, dtype=torch.float32)
+        with _timed("frame_scale_bwd"):
+            _lib.check(lib.bimamba_frame_scale_bwd(_ptr(xc), _ptr(g32), _ptr(dyc), _ptr(dx), _ptr(part), _ptr(ctx.seqlens),
+                                                   Bsz, T, C_, _dt(xc), _stream()), "bimamba_frame_scale_bwd")
+        dg = torch.empty((Bsz, C_), device=xc.device, dtype=torch.float32)
+        if Bsz and C_:
+            reduce_raw(part, dg, groups=Bsz, rows=nsl, cols=C_, part_gs=nsl * C_, row_stride=C_, out_gs=C_)
+        return dx.to(xdt), dg.to(gdt), None
+
+
+def frame_scale(x: torch.Tensor, gate: torch.Tensor, seqlens: torch.Tensor) -> torch.Tensor:
+    return FrameScaleFn.apply(x, gate, seqlens)
+
+
 def _f32c(t: Optional[torch.Tensor]) -> Optional[torch.Tensor]:
     return None if t is None else t.detach().to(torch.float32).contiguous()
 
