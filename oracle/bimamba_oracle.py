@@ -115,6 +115,25 @@ def selective_scan_ref(u: Tensor, delta: Tensor, A: Tensor, B: Tensor, C: Tensor
     return (y, h) if return_last_state else y
 
 
+def scan_inputs(Bsz: int, D: int, L: int, N: int = 16, seed: int = 0, dtype=torch.float32):
+    """Seeded scan operands with SURVEY 8(d) config-5 distributions (trained-like A, mamba's dt-bias range):
+    [u, delta, z, B, C] in `dtype` ((B, D, L) and (B, N, L)), then A (D, N), D (D) and delta_bias (D) in fp32."""
+    g = torch.Generator().manual_seed(seed)
+    u = torch.randn(Bsz, D, L, generator=g)
+    delta = 0.5 * torch.randn(Bsz, D, L, generator=g)
+    z = torch.randn(Bsz, D, L, generator=g)
+    Bm = torch.randn(Bsz, N, L, generator=g)
+    Cm = torch.randn(Bsz, N, L, generator=g)
+    A = -torch.exp(torch.log(torch.arange(1, N + 1, dtype=torch.float32)).repeat(D, 1)
+                   + 0.1 * torch.randn(D, N, generator=g))
+    Dp = 1 + 0.1 * torch.randn(D, generator=g)
+    dt = torch.exp(torch.rand(D, generator=g) * (torch.log(torch.tensor(0.1)) - torch.log(torch.tensor(1e-3)))
+                   + torch.log(torch.tensor(1e-3)))
+    bias = dt + torch.log(-torch.expm1(-dt))
+    act = [t.to(dtype) for t in (u, delta, z, Bm, Cm)]
+    return act + [A, Dp, bias]
+
+
 def selective_scan_split_ref(u: Tensor, delta: Tensor, A: Tensor, B: Tensor, C: Tensor,
                              D: Optional[Tensor] = None, z: Optional[Tensor] = None,
                              delta_bias: Optional[Tensor] = None, delta_softplus: bool = False,

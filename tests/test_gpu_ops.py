@@ -1,44 +1,29 @@
 """GPU parity of the op-level kernels (through the C ABI) against the CPU oracle.
 
-Tolerances are the ones BASELINE.json's north_star states: <= 1e-4 relative in fp32,
-<= 2e-2 in bf16 (fp32 state), measured as max|a-b| / max|b| against the fp64 oracle.
+Tolerances are the ones BASELINE.json's north_star states: <= 1e-4 relative in fp32, <= 2e-2 in bf16 (fp32 state),
+measured per slice against the fp64 oracle (oracle/compare.py): every state, channel, 8-step chunk and utterance of a
+tensor against its own magnitude.
 """
 import pytest
 import torch
 
 import bimamba_b200 as bm
 from oracle import bimamba_oracle as orc
+from oracle import compare as cmp
 
 pytestmark = pytest.mark.gpu
 
-TOL = {torch.float32: 1e-4, torch.bfloat16: 2e-2, torch.float16: 5e-3}
-
-
-def rel(a, b):
-    a = a.detach().double().cpu()
-    b = b.detach().double().cpu()
-    return float((a - b).abs().max() / b.abs().max().clamp_min(1e-30))
-
-
-def _scan_inputs(Bsz, D, L, N=16, seed=0, dtype=torch.float32):
-    """SURVEY 8(d) config-5 distributions (trained-like A, mamba dt-bias range)."""
-    g = torch.Generator().manual_seed(seed)
-    u = torch.randn(Bsz, D, L, generator=g)
-    delta = 0.5 * torch.randn(Bsz, D, L, generator=g)
-    z = torch.randn(Bsz, D, L, generator=g)
-    Bm = torch.randn(Bsz, N, L, generator=g)
-    Cm = torch.randn(Bsz, N, L, generator=g)
-    A = -torch.exp(torch.log(torch.arange(1, N + 1, dtype=torch.float32)).repeat(D, 1)
-                   + 0.1 * torch.randn(D, N, generator=g))
-    Dp = 1 + 0.1 * torch.randn(D, generator=g)
-    dt = torch.exp(torch.rand(D, generator=g) * (torch.log(torch.tensor(0.1)) - torch.log(torch.tensor(1e-3)))
-                   + torch.log(torch.tensor(1e-3)))
-    bias = dt + torch.log(-torch.expm1(-dt))
-    act = [t.to(dtype) for t in (u, delta, z, Bm, Cm)]
-    return act + [A, Dp, bias]
+TOL = cmp.TOL
+# (B, D, L) scan activations and data gradients, (B, N, L) dB / dC, then the parameter gradients
+SLICES = {"out": cmp.scan_act(0, 1, 2), "du": cmp.scan_act(0, 1, 2), "ddelta": cmp.scan_act(0, 1, 2),
+          "dz": cmp.scan_act(0, 1, 2), "dB": cmp.scan_state(0, 1), "dC": cmp.scan_state(0, 1),
+          "dA": cmp.CHANNEL_STATE, "dD": cmp.CHANNELS, "dbias": cmp.CHANNELS}
+_scan_inputs = orc.scan_inputs
 
 
 def _run_both(Bsz, D, L, dtype, with_z=True, with_D=True, with_bias=True, softplus=True, seed=0):
+    """The scan forward and backward on the GPU against the fp64 oracle on the same (dtype-rounded) inputs: the output
+    and every gradient, per slice at TOL[dtype]."""
     u, delta, z, Bm, Cm, A, Dp, bias = _scan_inputs(Bsz, D, L, seed=seed, dtype=dtype)
     if not softplus:          # a raw delta must be a positive step size
         delta = (0.2 * delta.float().abs()).to(dtype)
@@ -56,45 +41,40 @@ def _run_both(Bsz, D, L, dtype, with_z=True, with_D=True, with_bias=True, softpl
     assert out.dtype == dtype and out.shape == ref.shape
     out.backward(cot.cuda())
     torch.cuda.synchronize()
-    errs = {"out": rel(out, ref)}
+    tag = f"L={L} D={D} "
+    cmp.check(tag + "out", out, ref, TOL[dtype], SLICES["out"])
     for n, a, b in zip(names, dev_in, ref_in):
         if a is not None:
-            errs["d" + n] = rel(a.grad, b.grad)
-    return errs
+            cmp.check(tag + "d" + n, a.grad, b.grad, TOL[dtype], SLICES["d" + n])
 
 
 @pytest.mark.parametrize("L", [1, 5, 32, 33, 64, 201, 224, 256])
 def test_scan_single_chunk_fp32(L):
-    errs = _run_both(2, 40, L, torch.float32)
-    assert max(errs.values()) < TOL[torch.float32], errs
+    _run_both(2, 40, L, torch.float32)
 
 
 @pytest.mark.parametrize("L", [257, 300, 499, 777, 1024])
 def test_scan_multi_chunk_fp32(L):
-    errs = _run_both(2, 24, L, torch.float32, seed=L)
-    assert max(errs.values()) < TOL[torch.float32], errs
+    _run_both(2, 24, L, torch.float32, seed=L)
 
 
 @pytest.mark.parametrize("dtype", [torch.bfloat16, torch.float16])
 @pytest.mark.parametrize("L", [201, 499])
 def test_scan_half_precision_io(dtype, L):
-    errs = _run_both(2, 48, L, dtype, seed=3)
-    assert max(errs.values()) < TOL[dtype], errs
+    _run_both(2, 48, L, dtype, seed=3)
 
 
 @pytest.mark.parametrize("with_z,with_D,with_bias,softplus", [
     (False, True, True, True), (True, False, True, True), (True, True, False, True),
     (True, True, True, False), (False, False, False, False)])
 def test_scan_optional_operands(with_z, with_D, with_bias, softplus):
-    errs = _run_both(3, 17, 77, torch.float32, with_z, with_D, with_bias, softplus, seed=5)
-    assert max(errs.values()) < TOL[torch.float32], errs
+    _run_both(3, 17, 77, torch.float32, with_z, with_D, with_bias, softplus, seed=5)
 
 
 def test_scan_wide_and_ragged_channels():
     # dim = 288 (Phase 6) and a dim that is not a multiple of the channel group
     for D in (288, 37):
-        errs = _run_both(2, D, 201, torch.float32, seed=D)
-        assert max(errs.values()) < TOL[torch.float32], (D, errs)
+        _run_both(2, D, 201, torch.float32, seed=D)
 
 
 def test_scan_empty():
@@ -111,7 +91,7 @@ def test_scan_long_against_oracle_on_gpu():
     dev = [t.cuda() for t in (u, delta, A, Bm, Cm, Dp, z, bias)]
     ref = orc.selective_scan_ref(*[t.double() for t in dev], delta_softplus=True)
     out = bm.selective_scan_fn(*dev, delta_softplus=True)
-    assert rel(out, ref) < TOL[torch.float32]
+    cmp.check("out", out, ref, TOL[torch.float32], SLICES["out"])
 
 
 def test_scan_rejects_cpu_and_bad_state():
@@ -141,10 +121,10 @@ def test_causal_conv1d(dtype, L, act):
     out = bm.causal_conv1d_fn(xd, wd, bd, activation=act)
     out.backward(cot.cuda())
     tol = TOL[dtype]
-    assert rel(out, ref) < tol
-    assert rel(xd.grad, xr.grad) < tol
-    assert rel(wd.grad, wr.grad) < tol
-    assert rel(bd.grad, br.grad) < tol
+    cmp.check("out", out, ref, tol, cmp.scan_act(0, 1, 2))
+    cmp.check("dx", xd.grad, xr.grad, tol, cmp.scan_act(0, 1, 2))
+    cmp.check("conv1d.weight", wd.grad, wr.grad, tol, cmp.param("conv1d.weight", wr.shape))
+    cmp.check("conv1d.bias", bd.grad, br.grad, tol, cmp.CHANNELS)
 
 
 @pytest.mark.parametrize("D,force_tile", [(20, True), (18, False), (288, True)])
@@ -166,9 +146,9 @@ def _conv_bwd_case(D):
     (orc.causal_conv1d_ref(xr, wr, br, "silu") * cot.double()).sum().backward()
     xd, wd, bd = (t.cuda().requires_grad_(True) for t in (x, w, b))
     bm.causal_conv1d_fn(xd, wd, bd, activation="silu").backward(cot.cuda())
-    assert rel(xd.grad, xr.grad) < 1e-5
-    assert rel(wd.grad, wr.grad) < 1e-5
-    assert rel(bd.grad, br.grad) < 1e-5
+    cmp.check("dx", xd.grad, xr.grad, 1e-5, cmp.scan_act(0, 1, 2))
+    cmp.check("conv1d.weight", wd.grad, wr.grad, 1e-5, cmp.param("conv1d.weight", wr.shape))
+    cmp.check("conv1d.bias", bd.grad, br.grad, 1e-5, cmp.CHANNELS)
 
 
 @pytest.mark.parametrize("K", [2, 3, 4])
@@ -178,7 +158,7 @@ def test_causal_conv1d_widths_no_bias(K):
     w = torch.randn(9, K, generator=g)
     ref = orc.causal_conv1d_ref(x.double(), w.double(), None, "silu")
     out = bm.causal_conv1d_fn(x.cuda(), w.cuda(), None, activation="silu")
-    assert rel(out, ref) < 1e-5
+    cmp.check("out", out, ref, 1e-5, cmp.scan_act(0, 1, 2))
 
 
 # ---------------------------------------------------------------- layer norm
@@ -200,10 +180,10 @@ def test_layer_norm(C, dtype, out_dtype):
     assert out.dtype == out_dtype and out.shape == x.shape
     out.backward(cot.cuda())
     tol = 1e-5 if (dtype == torch.float32 and out_dtype == torch.float32) else 2e-2
-    assert rel(out, ref) < tol
-    assert rel(xd.grad, xr.grad) < tol
-    assert rel(wd.grad, wr.grad) < tol
-    assert rel(bd.grad, br.grad) < tol
+    cmp.check("out", out, ref, tol, cmp.frames())
+    cmp.check("dx", xd.grad, xr.grad, tol, cmp.frames())
+    cmp.check("weight", wd.grad, wr.grad, tol, cmp.CHANNELS)
+    cmp.check("bias", bd.grad, br.grad, tol, cmp.CHANNELS)
 
 
 # ---------------------------------------------------------------- tcgen05 GEMM
@@ -222,11 +202,11 @@ def test_gemm_nt_tensor_cores(M, N, K, dtype):
     Ad, Bd = A.cuda(), B.cuda()
     out = bm.ops.gemm_nt(Ad, Bd)
     assert out.dtype == dtype and out.shape == (M, N)
-    assert rel(out, ref) < (4e-3 if dtype == torch.bfloat16 else 1e-3)
+    assert cmp.rel(out, ref) < (4e-3 if dtype == torch.bfloat16 else 1e-3)
     out32 = bm.ops.gemm_nt(Ad, Bd, bias=bias.cuda(), out_dtype=torch.float32)
-    assert rel(out32, ref + bias.double()) < 1e-5          # fp32 accumulation, exact operands
+    assert cmp.rel(out32, ref + bias.double()) < 1e-5          # fp32 accumulation, exact operands
     out_add = bm.ops.gemm_nt(Ad, Bd, addend=add.cuda())          # product rounded to dtype, then + addend, rounded again
-    assert rel(out_add, ref + add.double()) < (8e-3 if dtype == torch.bfloat16 else 2e-3)
+    assert cmp.rel(out_add, ref + add.double()) < (8e-3 if dtype == torch.bfloat16 else 2e-3)
 
 
 def test_gemm_nt_strided_operand():
@@ -235,7 +215,7 @@ def test_gemm_nt_strided_operand():
     big = torch.randn(500, 576, generator=g).to(torch.bfloat16).cuda()
     W = (torch.randn(48, 288, generator=g) / 17).to(torch.bfloat16).cuda()
     out = bm.ops.gemm_nt(big[:, :288], W, out_dtype=torch.float32)
-    assert rel(out, big[:, :288].double() @ W.double().t()) < 1e-5
+    assert cmp.rel(out, big[:, :288].double() @ W.double().t()) < 1e-5
 
 
 # ---------------------------------------------------------------- feed-forward + column sums
@@ -259,9 +239,15 @@ def test_feed_forward_fn(dtype):
     assert out.dtype == torch.float32                      # the residual stream stays fp32
     out.backward(cot.cuda())
     tol = 1e-5 if dtype == torch.float32 else 2e-2
-    assert rel(out, ref) < tol
-    for a, b in zip(dev_in, ref_in):
-        assert rel(a.grad, b.grad) < tol
+    cmp.check("out", out, ref, tol, cmp.frames())
+    names = ["dx", "feed_forward.0.weight", "feed_forward.0.bias", "feed_forward.2.weight", "feed_forward.2.bias",
+             "dresidual"]
+    for n, a, b in zip(names, dev_in, ref_in):
+        # fp32 dx keeps the whole-tensor rule at this test's 1e-5 (rho 1): on a B200, dx[2, 32:40], at 0.71 of the
+        # tensor's largest element, is 1.1e-5 off (7.8e-6 of max|ref|), the rounding of the fp32 products on split-bf16
+        # operands through both GEMMs
+        rho = 1.0 if n == "dx" and dtype == torch.float32 else None
+        cmp.check(n, a.grad, b.grad, tol, cmp.frames() if n.startswith("d") else cmp.param(n, b.shape), rho=rho)
 
 
 @pytest.mark.parametrize("rows,cols", [(12864, 576), (1, 7), (300, 144)])
@@ -269,7 +255,7 @@ def test_colsum(rows, cols):
     g = torch.Generator().manual_seed(rows)
     x = torch.randn(rows, cols, generator=g).to(torch.bfloat16)
     out = bm.ops.colsum(x.cuda())
-    assert rel(out, x.double().sum(0)) < 1e-5
+    assert cmp.rel(out, x.double().sum(0)) < 1e-5
 
 
 @pytest.mark.parametrize("variant", [1, 3])
@@ -280,8 +266,7 @@ def test_scan_forward_variants(variant, dtype):
     rounding."""
     with bm._lib.tuning(bm._lib.TUNE_SCAN_FWD, variant):
         for L, D in ((201, 288), (37, 40), (499, 17)):
-            errs = _run_both(2, D, L, dtype, seed=L + D)
-            assert max(errs.values()) < TOL[dtype], (variant, L, D, errs)
+            _run_both(2, D, L, dtype, seed=L + D)
 
 
 @pytest.mark.parametrize("dtype", [torch.float32, torch.bfloat16])
@@ -289,10 +274,8 @@ def test_scan_backward_shapes(dtype):
     """The backward kernel on ragged shapes: channel counts that are not multiples of the 32-channel group or of the
     vector width, a single 8-step chunk, and every optional operand absent."""
     for L, D in ((201, 288), (37, 40), (499, 17), (8, 33)):
-        errs = _run_both(2, D, L, dtype, seed=L + D)
-        assert max(errs.values()) < TOL[dtype], (L, D, errs)
-    errs = _run_both(2, 40, 77, dtype, with_z=False, with_D=False, with_bias=False, softplus=False, seed=5)
-    assert max(errs.values()) < TOL[dtype], errs
+        _run_both(2, D, L, dtype, seed=L + D)
+    _run_both(2, 40, 77, dtype, with_z=False, with_D=False, with_bias=False, softplus=False, seed=5)
 
 
 @pytest.mark.parametrize("kernel", [1, 2])
@@ -307,7 +290,7 @@ def test_gemm_nt_kernel_variants(kernel):
             bias = torch.randn(N, generator=g).cuda()
             out = bm.ops.gemm_nt(A, B, bias=bias, out_dtype=torch.float32)
             ref = A.double() @ B.double().t() + bias.double()
-            assert rel(out, ref) < 1e-5, (kernel, M, N, K)
+            assert cmp.rel(out, ref) < 1e-5, (kernel, M, N, K)
 
 
 @pytest.mark.parametrize("M,N1,N2", [(12864, 576, 144), (25728, 288, 48), (12864, 576, 144), (130, 128, 16), (1000, 144, 576),
@@ -321,7 +304,7 @@ def test_gemm_tn_weight_gradient(M, N1, N2, dtype):
     out = bm.ops.gemm_tn(A, B)
     assert out.dtype == torch.float32 and out.shape == (N1, N2)
     ref = A.double().t() @ B.double()
-    assert rel(out, ref) < 1e-5
+    assert cmp.rel(out, ref) < 1e-5
     assert torch.equal(out, bm.ops.gemm_tn(A, B))
 
 
@@ -342,8 +325,8 @@ def test_head_forward_fused(T, dtype):
     logits_ref = feats_ref @ cw.double().t() + cb.double()
     feats, logits = bm.ops.head_fwd(x.cuda(), gw.cuda(), gb.cuda(), aw.cuda(), ab.cuda(), cw.cuda(), cb.cuda(), 1e-5)
     assert feats.dtype == torch.float32 and logits.shape == (Bsz, 2)
-    assert rel(feats, feats_ref) < 1e-5
-    assert rel(logits, logits_ref) < 1e-5
+    cmp.check("feats", feats, feats_ref, 1e-5, cmp.UTT)
+    cmp.check("logits", logits, logits_ref, 1e-5, cmp.UTT)
 
 
 def test_scan_long_backward_against_oracle_on_gpu():
@@ -361,9 +344,10 @@ def test_scan_long_backward_against_oracle_on_gpu():
         dev_in = [t.cuda().requires_grad_(True) for t in cpu]
         out = bm.selective_scan_fn(*dev_in, delta_softplus=True)
         out.backward(cot)
-        assert rel(out, ref) < TOL[dtype]
+        tag = f"{str(dtype)[6:]} "
+        cmp.check(tag + "out", out, ref, TOL[dtype], SLICES["out"])
         for n, a, b in zip(names, dev_in, ref_in):
-            assert rel(a.grad, b.grad) < TOL[dtype], (dtype, n)
+            cmp.check(tag + "d" + n, a.grad, b.grad, TOL[dtype], SLICES["d" + n])
 
 
 def test_gelu_kernels():
@@ -374,8 +358,8 @@ def test_gelu_kernels():
         xr = x.double().requires_grad_(True)
         yr = torch.nn.functional.gelu(xr)
         yr.backward(dy.double())
-        assert rel(bm.ops.gelu_fwd(x), yr) < tol
-        assert rel(bm.ops.gelu_bwd(dy, x), xr.grad) < tol
+        assert cmp.rel(bm.ops.gelu_fwd(x), yr) < tol
+        assert cmp.rel(bm.ops.gelu_bwd(dy, x), xr.grad) < tol
 
 
 @pytest.mark.parametrize("C_", [1024, 64, 300])
@@ -392,9 +376,9 @@ def test_layernorm_wide_rows(C_):
     dev_in = [t.cuda().requires_grad_(True) for t in (x, w, b)]
     out = bm.ops.layer_norm_fn(*dev_in, 1e-5)
     out.backward(cot.cuda())
-    assert rel(out, ref) < 1e-5
-    for a, r in zip(dev_in, ref_in):
-        assert rel(a.grad, r.grad) < 1e-5
+    cmp.check("out", out, ref, 1e-5, cmp.frames())
+    for n, a, r in zip(("dx", "weight", "bias"), dev_in, ref_in):
+        cmp.check(n, a.grad, r.grad, 1e-5, cmp.frames() if n == "dx" else cmp.CHANNELS)
 
 
 def test_fp32_products_on_the_tensor_cores():
@@ -409,16 +393,16 @@ def test_fp32_products_on_the_tensor_cores():
         add = torch.randn(M, N, generator=g).cuda()
         out = bm.ops.gemm_nt(A, B, bias=bias, addend=add)
         assert out.dtype == torch.float32
-        assert rel(out, A.double() @ B.double().t() + bias.double() + add.double()) < 2e-5, (M, N, K)   # fp32 accumulation over 6 K terms
+        assert cmp.rel(out, A.double() @ B.double().t() + bias.double() + add.double()) < 2e-5, (M, N, K)   # fp32 accumulation over 6 K terms
     buf = torch.zeros(515, 48, device="cuda")
     A = torch.randn(515, 288, generator=g).cuda()
     W = (torch.randn(16, 288, generator=g) / 17).cuda()
     bm.ops.gemm_nt(A, W, out=buf[:, 32:])
-    assert rel(buf[:, 32:], A.double() @ W.double().t()) < 2e-5 and float(buf[:, :32].abs().max()) == 0.0
+    assert cmp.rel(buf[:, 32:], A.double() @ W.double().t()) < 2e-5 and float(buf[:, :32].abs().max()) == 0.0
     for M, N1, N2 in ((12864, 576, 144), (25728, 288, 48), (130, 128, 16)):
         A = torch.randn(M, N1, generator=g).cuda()
         B = torch.randn(M, N2, generator=g).cuda()
-        assert rel(bm.ops.gemm_tn(A, B), A.double().t() @ B.double()) < 5e-5, (M, N1, N2)   # up to 154 k fp32-accumulated terms
+        assert cmp.rel(bm.ops.gemm_tn(A, B), A.double().t() @ B.double()) < 5e-5, (M, N1, N2)   # up to 154 k fp32-accumulated terms
 
 
 def test_cast_and_mean_square_loss_kernels():
@@ -433,10 +417,10 @@ def test_cast_and_mean_square_loss_kernels():
         loss = bm.ops.mean_square_loss(x)
         ref_in = x.detach().double().requires_grad_(True)
         ref = ref_in.square().mean()
-        assert loss.dtype == torch.float32 and loss.ndim == 0 and rel(loss, ref) < tol
+        assert loss.dtype == torch.float32 and loss.ndim == 0 and cmp.rel(loss, ref) < tol
         (3.0 * loss).backward()
         (3.0 * ref).backward()
-        assert rel(x.grad, ref_in.grad) < (1e-6 if dtype == torch.float32 else 1e-2)
+        assert cmp.rel(x.grad, ref_in.grad) < (1e-6 if dtype == torch.float32 else 1e-2)
 
 
 @pytest.mark.parametrize("nseg", [2, 3, 5])
@@ -449,10 +433,8 @@ def test_scan_forward_time_split(nseg, dtype):
     with bm._lib.tuning(bm._lib.TUNE_SCAN_SPLIT, nseg):
         for L, D in ((201, 288), (37, 40), (499, 17), (1024, 24)):
             assert bm._lib.scan_split_plan(2, 1, L, D, bm._lib.F32)[0] >= 2
-            errs = _run_both(2, D, L, dtype, seed=L + D)
-            assert max(errs.values()) < TOL[dtype], (nseg, L, D, errs)
-        errs = _run_both(2, 40, 77, dtype, with_z=False, with_D=False, with_bias=False, softplus=False, seed=5)
-        assert max(errs.values()) < TOL[dtype], errs
+            _run_both(2, D, L, dtype, seed=L + D)
+        _run_both(2, 40, 77, dtype, with_z=False, with_D=False, with_bias=False, softplus=False, seed=5)
 
 
 def test_scan_time_split_is_automatic_at_long_lengths_and_matches_the_serial_walk():
@@ -473,7 +455,7 @@ def test_scan_time_split_is_automatic_at_long_lengths_and_matches_the_serial_wal
                 out_split = bm.selective_scan_fn(*dev, delta_softplus=True)
             with bm._lib.tuning(bm._lib.TUNE_SCAN_SPLIT, 1):
                 out_serial = bm.selective_scan_fn(*dev, delta_softplus=True)
-        assert rel(out_split, out_serial) < tol_pair
+        assert cmp.rel(out_split, out_serial) < tol_pair
         ref = orc.selective_scan_ref(*[t.double() for t in dev], delta_softplus=True)
-        assert rel(out_split, ref) < TOL[dtype]
-        assert rel(out_serial, ref) < TOL[dtype]
+        cmp.check("split out", out_split, ref, TOL[dtype], SLICES["out"])
+        cmp.check("serial out", out_serial, ref, TOL[dtype], SLICES["out"])

@@ -16,7 +16,8 @@ stream (parallel graph branches) and reads the AdamW hyper-parameters from devic
     torch.optim.AdamW in fp64.
   * bimamba_reduce_partials: each of its three variants, on both sides of the switch points, against an fp64 sum.
 
-The oracle (oracle/bimamba_oracle.py) runs on the GPU in fp64, one layer at a time: a forward without autograd keeps
+Every comparison is per slice (oracle/compare.py): activations per utterance and per 8-frame chunk, each parameter
+gradient per its own blocks.  The oracle (oracle/bimamba_oracle.py) runs on the GPU in fp64, one layer at a time: a forward without autograd keeps
 each layer's input, then every layer's forward is redone under autograd while the cotangent walks back through it.
 """
 import pytest
@@ -24,17 +25,12 @@ import torch
 
 import bimamba_b200 as bm
 from oracle import bimamba_oracle as orc
+from oracle import compare as cmp
 
 pytestmark = pytest.mark.gpu
 
 B, L, D_MODEL, N_LAYERS, D_STATE = 64, 201, 144, 4, 16      # bench.py's workload (BASELINE.json configs[1])
 D_INNER, NDIR = 2 * D_MODEL, 2
-
-
-def rel(a, b):
-    a = torch.as_tensor(a).detach().double().cpu()
-    b = torch.as_tensor(b).detach().double().cpu()
-    return float((a - b).abs().max() / b.abs().max().clamp_min(1e-30))
 
 
 def _model():
@@ -133,11 +129,10 @@ def test_fp32_captured_step_vs_oracle(oracle):
     torch.cuda.synchronize()
     named = _named(model)
     assert len(named) == 68
-    errs = {"loss": rel(loss, ref_loss)}
-    errs.update({n: rel(p.grad, ref_grads[n]) for n, p in named})
-    print("fp32 captured step, worst rel err vs oracle:", _worst(errs), "loss", errs["loss"])
-    bad = {n: e for n, e in errs.items() if not e < 1e-4}
-    assert not bad, bad
+    loss_err = cmp.rel(loss, ref_loss)
+    ratios = {n: cmp.check(n, p.grad, ref_grads[n], 1e-4, cmp.param(n, p.shape)) for n, p in named}
+    print("fp32 captured step, worst slice ratio vs oracle:", _worst(ratios), "loss rel err", loss_err)
+    assert loss_err < 1e-4
 
 
 class _Recorder:
@@ -182,8 +177,8 @@ def test_bf16_step_captured_sequenced_native_bitwise_and_vs_oracle(oracle):
     oracle on that layer's own input and output cotangent, and end to end (loss 2e-2, gradients 5e-2: the bars of the
     4-layer bf16 chain in test_model_tail_vs_reference_fixture).
 
-    Per layer, the output and dx keep one layer's bf16 bar, 2e-2.  The parameter gradients get 3e-2.  On a B200 the
-    largest of the 68 is 2.4e-2, layer 2's x_proj.weight, in its C rows: a sum over 25 728 rows whose operands, dC and the
+    Per layer, the output and dx keep one layer's bf16 bar, 2e-2.  The parameter gradients get 3e-2, per slice.  On a
+    B200 the largest of the 68 over the whole tensor is 2.4e-2, layer 2's x_proj.weight, in its C rows: a sum over 25 728 rows whose operands, dC and the
     conv output, are stored in bf16.  The next largest is 1.8e-2 (layer 1's dt_proj.bias), and the same step in fp32 is within 3e-5 of the oracle on every gradient (the fp32 test above), so the
     excess is the rounding of the stored bf16 operands, not the arithmetic."""
     ref_loss, ref_grads = oracle
@@ -222,27 +217,28 @@ def test_bf16_step_captured_sequenced_native_bitwise_and_vs_oracle(oracle):
         assert not diff, (other, diff)
 
     # (c) layer by layer: the oracle fed the layer's recorded input and output cotangent
-    errs = {}
+    ratios = {}
     for i in range(N_LAYERS):
         out_ref, dx_ref, gp_ref = _layer_ref(sds[i], rec.x[i], rec.cot[i])
-        errs[f"out.{i}"] = rel(rec.out[i], out_ref)
+        ratios[f"out.{i}"] = cmp.check(f"out.{i}", rec.out[i], out_ref, 2e-2, cmp.frames())
         if i > 0:                          # the gradient w.r.t. layer i's input arrives at layer i - 1's output
-            errs[f"dx.{i}"] = rel(rec.cot[i - 1], dx_ref)
+            ratios[f"dx.{i}"] = cmp.check(f"dx.{i}", rec.cot[i - 1], dx_ref, 2e-2, cmp.frames())
         for k, g in gp_ref.items():
-            errs[f"backbone_layers.{i}.{k}"] = rel(grads[f"backbone_layers.{i}.{k}"], g)
+            n = f"backbone_layers.{i}.{k}"
+            # x_proj.weight keeps the whole-tensor rule (rho 1): on a B200 its column group [:, 128:160] in layer 2,
+            # at 0.53 of the tensor's largest element, is 4.3e-2 off, 2.3e-2 of max|ref| - the rounding of its
+            # bf16-stored operands described above, on a slice too large for any floor to cover
+            rho = 1.0 if k.endswith("x_proj.weight") else None
+            ratios[n] = cmp.check(n, grads[n], g, 3e-2, cmp.param(n, g.shape), rho=rho)
         del out_ref, dx_ref, gp_ref
-    assert len(errs) == N_LAYERS * 18 + N_LAYERS - 1
-    print("bf16 step, per layer, worst rel err vs oracle:", _worst(errs))
-    bad = {n: e for n, e in errs.items() if not e < (3e-2 if n.startswith("backbone_layers.") else 2e-2)}
-    assert not bad, bad
+    assert len(ratios) == N_LAYERS * 18 + N_LAYERS - 1
+    print("bf16 step, per layer, worst slice ratio vs oracle:", _worst(ratios))
 
     # end to end against the 4-layer oracle
-    e2e = {n: rel(g, ref_grads[n]) for n, g in grads.items()}
-    loss_err = rel(runs["native"]["loss"], ref_loss)
-    print("bf16 step, end to end: loss rel err", loss_err, "worst gradient", _worst(e2e))
+    e2e = {n: cmp.check("e2e " + n, g, ref_grads[n], 5e-2, cmp.param(n, g.shape)) for n, g in grads.items()}
+    loss_err = cmp.rel(runs["native"]["loss"], ref_loss)
+    print("bf16 step, end to end: loss rel err", loss_err, "worst gradient slice ratio", _worst(e2e))
     assert loss_err < 2e-2
-    bad = {n: e for n, e in e2e.items() if not e < 5e-2}
-    assert not bad, bad
 
 
 def test_adamw_inside_the_captured_step_vs_torch_adamw():
@@ -287,12 +283,12 @@ def test_adamw_inside_the_captured_step_vs_torch_adamw():
             ulp = (torch.nextafter(big, torch.full_like(big, float("inf"))) - big).double()
             excess = ((d_ours - d_ref).abs() - ulp).clamp_min(0.0)
             errs[n] = float(excess.max() / d_ref.abs().max())
-            worst.setdefault("raw", {})[(k, n)] = rel(d_ours, d_ref)
+            worst.setdefault("raw", {})[(k, n)] = cmp.rel(d_ours, d_ref)
         errs_m = {}
         sd = opt.state_dict()["state"]
         for i, (n, r) in enumerate(zip(names, ref_p)):
-            errs_m["exp_avg." + n] = rel(sd[i]["exp_avg"], ref.state[r]["exp_avg"])
-            errs_m["exp_avg_sq." + n] = rel(sd[i]["exp_avg_sq"], ref.state[r]["exp_avg_sq"])
+            errs_m["exp_avg." + n] = cmp.rel(sd[i]["exp_avg"], ref.state[r]["exp_avg"])
+            errs_m["exp_avg_sq." + n] = cmp.rel(sd[i]["exp_avg_sq"], ref.state[r]["exp_avg_sq"])
             assert float(sd[i]["step"]) == k + 1
         print(f"AdamW replay {k + 1} (lr {lr:g}): update beyond 1 ulp", _worst(errs), "moments", _worst(errs_m))
         bad = {n: e for n, e in {**errs, **errs_m}.items() if not e < 1e-6}

@@ -1,26 +1,22 @@
 """Variable-length scoring on the GPU: right-padded batches with per-utterance frame counts against the oracle run on
 every utterance at its own length; padding never leaks; lengths == T is bit-identical to the fixed-length path.
 
-Tolerances as elsewhere: <= 1e-4 relative in fp32, <= 2e-2 in bf16 (fp32 state), against the fp64 oracle."""
+Tolerances as elsewhere: <= 1e-4 relative in fp32, <= 2e-2 in bf16 (fp32 state), against the fp64 oracle, per slice
+(oracle/compare.py): every utterance, and every 8-frame chunk of it, against its own magnitude."""
 import numpy as np
 import pytest
 import torch
 
 import bimamba_b200 as bm
 from oracle import bimamba_oracle as orc
+from oracle import compare as cmp
 from oracle.varlen_oracle import backend_varlen_ref
 
 pytestmark = pytest.mark.gpu
 
-TOL = {torch.float32: 1e-4, torch.bfloat16: 2e-2}
+TOL = cmp.TOL
 # shorter than the conv width, around the 8-step checkpoint and 16-step chunk boundaries, and the full padded length
 LENGTHS = [1, 2, 3, 7, 8, 9, 15, 16, 17, 40]
-
-
-def rel(a, b):
-    a = torch.as_tensor(a).detach().double().cpu()
-    b = torch.as_tensor(b).detach().double().cpu()
-    return float((a - b).abs().max() / b.abs().max().clamp_min(1e-30))
 
 
 def _mamba(d_model, seed):
@@ -45,12 +41,10 @@ def _autocast(dtype):
 
 
 def _check_block(m, pr, x, lengths, out, tol):
-    got, ref = [], []
     for n in sorted(set(lengths)):
         idx = [b for b, v in enumerate(lengths) if v == n]
-        ref.append(orc.bimamba_ref(pr, x[idx, :n].double().cuda()).reshape(-1))
-        got.append(out[idx, :n].reshape(-1))
-    assert rel(torch.cat(got), torch.cat(ref)) < tol
+        ref = orc.bimamba_ref(pr, x[idx, :n].double().cuda())
+        cmp.check(f"out(n={n})", out[idx, :n], ref, tol, cmp.frames())
 
 
 @pytest.mark.parametrize("variant", [1, 3])
@@ -86,8 +80,8 @@ def test_backend_varlen_vs_oracle(dtype):
     f_ref, s_ref = backend_varlen_ref(lay, head, x.double().cuda(), lengths)
     with torch.no_grad(), _autocast(dtype):
         feats, logits = net(x.cuda(), lengths)
-    assert rel(feats, f_ref) < TOL[dtype]
-    assert rel(logits, s_ref) < TOL[dtype]
+    cmp.check("feats", feats, f_ref, TOL[dtype], cmp.UTT)
+    cmp.check("logits", logits, s_ref, TOL[dtype], cmp.UTT)
 
 
 @pytest.mark.parametrize("dtype", [torch.float32, torch.bfloat16])
@@ -107,8 +101,8 @@ def test_graphed_forward_serves_every_length_mix(dtype):
         x = torch.randn(B, T, 144, generator=g)
         feats, logits = runner.run(x.cuda(), lengths)
         f_ref, s_ref = backend_varlen_ref(lay, head, x.double().cuda(), [int(v) for v in lengths])
-        assert rel(feats, f_ref) < TOL[dtype]
-        assert rel(logits, s_ref) < TOL[dtype]
+        cmp.check("feats", feats, f_ref, TOL[dtype], cmp.UTT)
+        cmp.check("logits", logits, s_ref, TOL[dtype], cmp.UTT)
 
 
 def _padded(x, lengths, value):
@@ -155,7 +149,7 @@ def test_zero_length_utterance_scores_as_zero_features():
         f2, l2 = net(x[[0, 2]], [24, 11])
     assert torch.equal(feats[1], torch.zeros_like(feats[1]))
     assert torch.equal(logits[1], net.classifier.bias.detach())
-    assert rel(feats[[0, 2]], f2) < 1e-6 and rel(logits[[0, 2]], l2) < 1e-6
+    assert cmp.rel(feats[[0, 2]], f2) < 1e-6 and cmp.rel(logits[[0, 2]], l2) < 1e-6
 
 
 @pytest.mark.parametrize("path", ["fp32", "bf16_native", "bf16_sequenced"])

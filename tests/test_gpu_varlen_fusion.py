@@ -3,7 +3,8 @@ utterance alone, the module with lengths (scoring and mask_padding=True training
 utterance, the model tail (fusion -> 4-layer backend -> head) with lengths from real clip sample counts, full lengths
 against the reference fixtures and the fixed-length module, and one captured graph serving every length mix.
 
-Tolerances as elsewhere: 1e-4 fp32, 2e-2 bf16 (5e-2 for bf16 gradients that cross the whole tail)."""
+Tolerances as elsewhere: 1e-4 fp32, 2e-2 bf16 (5e-2 for bf16 gradients that cross the whole tail), measured per slice
+(oracle/compare.py) against the oracle: every utterance and 8-frame chunk, every parameter gradient per its blocks."""
 import os
 
 import numpy as np
@@ -13,6 +14,7 @@ import torch.nn.functional as F
 
 import bimamba_b200 as bm
 from bimamba_b200 import ops
+from oracle import compare as cmp
 from oracle.varlen_fusion_oracle import (fusion_loss_and_grads_ref, fusion_one_ref, fusion_varlen_ref, tail_fn,
                                          tail_varlen_ref)
 
@@ -24,12 +26,6 @@ EPS = {torch.float32: 2.0 ** -23, torch.bfloat16: 2.0 ** -7, torch.float16: 2.0 
 # a linear downsample (n1 < n2), the full padded shape (nearest), and (110, 16): a 2.21 s clip, where fp32 and fp64
 # nearest rules pick different frames
 PAIRS = [(30, 30), (1, 1), (120, 30), (121, 30), (5, 30), (125, 30), (110, 16), (7, 3)]
-
-
-def rel(a, b):
-    a = torch.as_tensor(a).detach().double().cpu()
-    b = torch.as_tensor(b).detach().double().cpu()
-    return float((a - b).abs().max() / b.abs().max().clamp_min(1e-30))
 
 
 def wavlm_frames(S):
@@ -110,7 +106,7 @@ def test_interp_backward_matches_autograd_and_is_repeatable(dtype):
     for b, (n1, n2) in enumerate(PAIRS):
         x = src[b, :n2].float().cpu().requires_grad_(True)
         _interp_torch(x, n1).backward(cot[b, :n1].float().cpu())
-        assert rel(d1[b, :n2], x.grad) < tol, (n1, n2)
+        assert cmp.rel(d1[b, :n2], x.grad) < tol, (n1, n2)
         assert bool((d1[b, n2:] == 0).all())
 
 
@@ -134,16 +130,16 @@ def test_frame_mean_and_scale_match_torch_per_utterance(dtype):
     tol = 1e-5 if dtype == torch.float32 else 2 * EPS[dtype]
     for b, n in enumerate(lengths):
         xb = x[b, :n].float()
-        assert rel(mean[b], xb.mean(0) if n else torch.zeros(C)) < 1e-5
+        assert cmp.rel(mean[b], xb.mean(0) if n else torch.zeros(C)) < 1e-5
         assert torch.equal(y[b, :n], (xb * gate[b]).to(dtype))
         assert bool((y[b, n:] == 0).all())
     torch.autograd.backward([mean, y], [dmean, dy])
     for b, n in enumerate(lengths):
         dgr = (dy[b, :n].float() * x[b, :n].float()).sum(0)
-        assert (rel(gr.grad[b], dgr) < 1e-5) if n else bool((gr.grad[b] == 0).all())
+        assert (cmp.rel(gr.grad[b], dgr) < 1e-5) if n else bool((gr.grad[b] == 0).all())
         if n:
             dxr = dy[b, :n].float() * gate[b] + dmean[b] / n
-            assert rel(xr.grad[b, :n], dxr) < tol
+            assert cmp.rel(xr.grad[b, :n], dxr) < tol
         assert bool((xr.grad[b, n:] == 0).all())
     g1 = gr.grad.clone()
     gr.grad = None
@@ -188,7 +184,7 @@ def test_module_scoring_matches_oracle(dtype):
     ref = fusion_varlen_ref(_p64(fus), fw.double().cpu(), fs.double().cpu(), l1, l2)
     tol = 1e-4 if dtype == torch.float32 else 2e-2
     for b, n1 in enumerate(l1):
-        assert rel(out[b, :n1], ref[b, :n1]) < tol, PAIRS[b]
+        cmp.check(f"out{PAIRS[b]}", out[b, :n1], ref[b, :n1], tol, [{0: cmp.CHUNK}])
 
 
 @pytest.mark.parametrize("fill", [float("nan"), 1e4])
@@ -217,11 +213,12 @@ def test_module_mask_padding_training_matches_oracle(dtype, fill):
     gtol = 1e-4 if dtype == torch.float32 else 5e-2
     for b, (n1, n2) in enumerate(PAIRS):
         assert bool((out[b, n1:] == 0).all()) and bool((fwr.grad[b, n1:] == 0).all()) and bool((fsr.grad[b, n2:] == 0).all())
-    assert rel(out, ref) < tol
-    assert rel(fwr.grad, dfw) < gtol and rel(fsr.grad, dfs) < gtol
+    cmp.check("out", out, ref, tol, cmp.frames())
+    cmp.check("d f_wavlm", fwr.grad, dfw, gtol, cmp.frames())
+    cmp.check("d f_sinc", fsr.grad, dfs, gtol, cmp.frames())
     for name, p in fus.named_parameters():
         assert torch.isfinite(p.grad).all(), name
-        assert rel(p.grad, grads[name]) < gtol, name
+        cmp.check(name, p.grad, grads[name], gtol, cmp.param(name, p.shape))
 
 
 def test_module_full_lengths_match_fixed_length_path():
@@ -239,7 +236,7 @@ def test_module_full_lengths_match_fixed_length_path():
             mode = "nearest" if T1 / T2 > 4.0 else "linear"
             kw = {} if mode == "nearest" else {"align_corners": False}
             theirs = F.interpolate(s2.transpose(1, 2), size=T1, mode=mode, **kw).transpose(1, 2)
-        assert rel(b, a) < 1e-6
+        assert cmp.rel(b, a) < 1e-6
         if mode == "nearest":
             assert torch.equal(mine, theirs)
 
@@ -260,15 +257,15 @@ def test_module_full_lengths_vs_reference_fixture(golden_dir, tag, dtype):
     tol = 1e-4 if dtype == torch.float32 else 2e-2
     with torch.autocast("cuda", dtype=dtype, enabled=dtype != torch.float32):
         out = fus(fw, fs, [T1] * B, [T2] * B, mask_padding=True)
-    assert rel(out, g["f_fused"]) < tol
+    cmp.check("out", out, g["f_fused"], tol, cmp.frames())
     out.backward(torch.tensor(g["grad.f_fused"], device="cuda", dtype=torch.float32))
     if tag == "linear":
-        assert rel(fw.grad, g["grad.f_wavlm"]) < tol
-    else:
-        assert rel(fw.grad.reshape(-1)[::5], g["grad5.f_wavlm"]) < tol
-    assert rel(fs.grad, g["grad.f_sinc"]) < tol
+        cmp.check("d f_wavlm", fw.grad, g["grad.f_wavlm"], tol, cmp.frames())
+    else:                                      # every 5th element of the flattened gradient: no structure to slice
+        cmp.check("d f_wavlm[::5]", fw.grad.reshape(-1)[::5], g["grad5.f_wavlm"], tol)
+    cmp.check("d f_sinc", fs.grad, g["grad.f_sinc"], tol, cmp.frames())
     for name, p in fus.named_parameters():
-        assert rel(p.grad, g["grad.fusion." + name]) < tol, name
+        cmp.check(name, p.grad, g["grad.fusion." + name], tol, cmp.param(name, p.shape))
 
 
 # ---------------------------------------------------------------------------------------------------------------- tail
@@ -304,7 +301,8 @@ def test_tail_scoring_matches_oracle(tail_case, dtype):
     with torch.no_grad(), torch.autocast("cuda", dtype=dtype, enabled=dtype != torch.float32):
         feats, logits = net(fus(c["fw"], c["fs"], c["l1"], c["l2"]), c["l1"])
     tol = 1e-4 if dtype == torch.float32 else 2e-2
-    assert rel(feats, c["feats"]) < tol and rel(logits, c["logits"]) < tol
+    cmp.check("feats", feats, c["feats"], tol, cmp.UTT)
+    cmp.check("logits", logits, c["logits"], tol, cmp.UTT)
 
 
 @pytest.mark.parametrize("dtype", [torch.float32, torch.bfloat16])
@@ -325,7 +323,8 @@ def test_tail_training_matches_oracle(tail_case, dtype):
     tol = 1e-4 if dtype == torch.float32 else 2e-2
     gtol = 1e-4 if dtype == torch.float32 else 5e-2
     assert abs(float(loss.detach()) - float(c["loss"])) <= tol * abs(float(c["loss"])) + tol
-    assert rel(fw.grad, c["dfw"]) < gtol and rel(fs.grad, c["dfs"]) < gtol
+    cmp.check("d f_wavlm", fw.grad, c["dfw"], gtol, cmp.frames())
+    cmp.check("d f_sinc", fs.grad, c["dfs"], gtol, cmp.frames())
     for b, (n1, n2) in enumerate(zip(c["l1"], c["l2"])):
         assert bool((fw.grad[b, n1:] == 0).all()) and bool((fs.grad[b, n2:] == 0).all())
     named = [("fusion." + n, p) for n, p in fus.named_parameters()] + list(net.named_parameters())
@@ -334,7 +333,11 @@ def test_tail_training_matches_oracle(tail_case, dtype):
         if name == "attention_pool.bias":           # exact gradient 0 (softmax shift invariance): on the weight's scale
             assert float(p.grad.abs().max()) <= gtol * float(c["grads"]["attention_pool.weight"].abs().max()), name
         else:
-            assert rel(p.grad, ref) < gtol, name
+            # bf16: x_proj.weight keeps the whole-tensor rule (rho 1).  On a B200 its column group [:, 256:288] in
+            # layer 2, at 0.33 of the tensor's largest element, is 7.4e-2 off, 2.4e-2 of max|ref|: the rounding of its
+            # bf16-stored operands (dC and the conv output) after four layers, on a slice too large for a floor
+            rho = 1.0 if dtype != torch.float32 and name.endswith("x_proj.weight") else None
+            cmp.check(name, p.grad, ref, gtol, cmp.param(name, p.shape), rho=rho)
 
 
 def test_tail_captured_once_serves_every_length_mix(tail_case):

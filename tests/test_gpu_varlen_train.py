@@ -3,7 +3,8 @@ and the block, encoder layer and backend with mask_padding=True, against the fp6
 own length (parameter gradients summed over utterances).  Padding never leaks; lengths == T gives the bits of the
 fixed-length path; one captured training step serves every length mix.
 
-Tolerances as elsewhere: 1e-4 fp32, 2e-2 bf16, 5e-3 fp16 at op level; 5e-2 for bf16 end-to-end gradients."""
+Tolerances as elsewhere: 1e-4 fp32, 2e-2 bf16, 5e-3 fp16 at op level; 5e-2 for bf16 end-to-end gradients; measured per
+slice (oracle/compare.py), every utterance against its own magnitude."""
 import pytest
 import torch
 import torch.nn.functional as F
@@ -11,31 +12,27 @@ import torch.nn.functional as F
 import bimamba_b200 as bm
 from bimamba_b200 import ops
 from oracle import bimamba_oracle as orc
+from oracle import compare as cmp
 from oracle.varlen_train_oracle import backend_logits_fn, block_fn, layer_fn, varlen_loss_and_grads_ref
 
 pytestmark = pytest.mark.gpu
 
-TOL = {torch.float32: 1e-4, torch.bfloat16: 2e-2, torch.float16: 5e-3}
+TOL = cmp.TOL
 # shorter than the conv width, around the 8-step checkpoint and 16-step chunk boundaries, and the full padded length
 LENGTHS = [1, 2, 3, 7, 8, 9, 15, 16, 17, 40]
 LONG = [201, 150, 77, 9, 201, 33]
 N, XW = 16, 48
 
 
-def rel(a, b):
-    a = torch.as_tensor(a).detach().double().cpu()
-    b = torch.as_tensor(b).detach().double().cpu()
-    return float((a - b).abs().max() / b.abs().max().clamp_min(1e-30))
-
-
-def grad_err(name, got, grads_ref):
-    """Relative error of a parameter gradient; the attention-pool bias gets an exact gradient of zero (the softmax does
-    not change when every logit moves by the same amount), so it is measured on the scale of the attention weight's."""
-    ref = grads_ref[name]
+def check_grad(name, got, grads_ref, tol):
+    """A parameter gradient per slice; the attention-pool bias gets an exact gradient of zero (the softmax does not
+    change when every logit moves by the same amount), so it is measured on the scale of the attention weight's."""
     if "attention_pool.bias" in name or name == "ab":
         w = name.replace("bias", "weight") if name != "ab" else "aw"
-        return float(got.detach().double().abs().max().cpu() / grads_ref[w].abs().max().clamp_min(1e-30).cpu())
-    return rel(got, ref)
+        err = float(got.detach().double().abs().max().cpu() / grads_ref[w].abs().max().clamp_min(1e-30).cpu())
+        assert err < tol, (name, err)
+        return
+    cmp.check(name, got, grads_ref[name], tol, cmp.param(name, got.shape))
 
 
 def _pad_mask(lengths, T, dev="cuda"):
@@ -90,7 +87,7 @@ def _scan_case(mode, dtype, lengths, D=40, ndir=2, seed=0):
     A64 = A.double().cpu().requires_grad_(True)
     D64 = Dp.double().cpu().requires_grad_(True)
     b64 = bias.double().cpu().requires_grad_(True)
-    errs = {}
+    tol, act, state = TOL[dtype], cmp.scan_act(0, 2, 1), cmp.scan_state(0, 2)     # (1, n, D) / (1, n, 2N) pieces
     for b, n in enumerate(lengths):
         for di in range(ndir):
             fl = (lambda t: t.flip(-1)) if di else (lambda t: t)
@@ -103,16 +100,15 @@ def _scan_case(mode, dtype, lengths, D=40, ndir=2, seed=0):
             bc_d = fl(cut(bc[:, di])).requires_grad_(True)
             y = orc.selective_scan_ref(u_d, dl_d, A64, bc_d[:, :N], bc_d[:, N:], D64, z_d, b64, delta_softplus=True)
             k = f"{b}.{di}"
-            errs["out" + k] = rel(out[b:b + 1, di, :n].transpose(1, 2), fl(y))
+            cmp.check("out" + k, out[b:b + 1, di, :n], fl(y).transpose(1, 2), tol, act)
             (y * fl(cut(dout[:, di]))).sum().backward()
-            errs["du" + k] = rel(du[b:b + 1, di, :n], fl(u_d.grad).transpose(1, 2))
-            errs["ddelta" + k] = rel(ddelta[b:b + 1, di, :n], fl(dl_d.grad).transpose(1, 2))
-            errs["dz" + k] = rel(dz[b:b + 1, di, :n], fl(z_d.grad).transpose(1, 2))
-            errs["dbc" + k] = rel(dbc[b:b + 1, di, :n], fl(bc_d.grad).transpose(1, 2))
-    errs["dA"] = rel(dA, A64.grad)
-    errs["dD"] = rel(dD, D64.grad)
-    errs["dbias"] = rel(dbias, b64.grad)
-    return errs
+            cmp.check("du" + k, du[b:b + 1, di, :n], fl(u_d.grad).transpose(1, 2), tol, act)
+            cmp.check("ddelta" + k, ddelta[b:b + 1, di, :n], fl(dl_d.grad).transpose(1, 2), tol, act)
+            cmp.check("dz" + k, dz[b:b + 1, di, :n], fl(z_d.grad).transpose(1, 2), tol, act)
+            cmp.check("dB|dC" + k, dbc[b:b + 1, di, :n], fl(bc_d.grad).transpose(1, 2), tol, state)
+    cmp.check("dA", dA, A64.grad, tol, cmp.CHANNEL_STATE)
+    cmp.check("dD", dD, D64.grad, tol, cmp.CHANNELS)
+    cmp.check("dbias", dbias, b64.grad, tol, cmp.CHANNELS)
 
 
 @pytest.mark.parametrize("variant", [1, 3])
@@ -122,13 +118,11 @@ def test_scan_varlen_forward_and_backward(mode, dtype, variant):
     """Checkpointed forward (both forward kernels, forced) and backward with lengths against the oracle per utterance;
     the padding holds NaN; padded gradients are exactly zero and a second backward gives the same bits."""
     with bm._lib.tuning(bm._lib.TUNE_SCAN_FWD, variant):
-        errs = _scan_case(mode, dtype, LENGTHS, seed=10 * mode + variant)
-    assert max(errs.values()) < TOL[dtype], {k: v for k, v in errs.items() if v >= TOL[dtype]}
+        _scan_case(mode, dtype, LENGTHS, seed=10 * mode + variant)
 
 
 def test_scan_varlen_long_mixed():
-    errs = _scan_case(9, torch.bfloat16, LONG, seed=5)
-    assert max(errs.values()) < TOL[torch.bfloat16]
+    _scan_case(9, torch.bfloat16, LONG, seed=5)
 
 
 # ---------------------------------------------------------------------------------------------------------------- conv
@@ -158,17 +152,16 @@ def test_conv_varlen_backward(kernel, width, dtype):
     assert bool((dx[pad.cuda()] == 0).all()) and bool((dz[pad.cuda()] == 0).all())
     w64 = w.double().cpu().requires_grad_(True)
     b64 = b.double().cpu().requires_grad_(True)
-    errs = {}
+    tol, act = TOL[dtype], [{1: 1}, {0: cmp.CHUNK}]               # (n, D) pieces: per channel, per 8-step chunk
     for i, n in enumerate(lengths):
         xi = x[i, :n].double().cpu().t().unsqueeze(0).requires_grad_(True)       # (1, D, n)
         o0 = orc.causal_conv1d_ref(xi, w64, b64, "silu")
         o1 = orc.causal_conv1d_ref(xi.flip(-1), w64, b64, "silu").flip(-1)
         (o0 * dout[i, 0, :n].double().cpu().t() + o1 * dout[i, 1, :n].double().cpu().t()).sum().backward()
-        errs[f"dx{i}"] = rel(dx[i, :n], xi.grad[0].t())
-        errs[f"dz{i}"] = rel(dz[i, :n], dz_in[i, :, :n].double().sum(0))
-    errs["dw"] = rel(dwb[:, :width], w64.grad)
-    errs["db"] = rel(dwb[:, width], b64.grad)
-    assert max(errs.values()) < TOL[dtype], {k: v for k, v in errs.items() if v >= TOL[dtype]}
+        cmp.check(f"dx{i}", dx[i, :n], xi.grad[0].t(), tol, act)
+        cmp.check(f"dz{i}", dz[i, :n], dz_in[i, :, :n].double().sum(0), tol, act)
+    cmp.check("conv1d.weight", dwb[:, :width], w64.grad, tol, cmp.param("conv1d.weight", w64.shape))
+    cmp.check("conv1d.bias", dwb[:, width], b64.grad, tol, cmp.CHANNELS)
 
 
 # ---------------------------------------------------------------------------------------------------------------- head
@@ -193,9 +186,9 @@ def test_head_pool_varlen_backward_and_zero_length():
     params = {"w": nw, "b": nb, "aw": aw, "ab": ab}
     _, gr, dx = varlen_loss_and_grads_ref(fn, params, x.detach(), lengths,
                                           lambda f, idx, n: (f * df[idx].double()).sum())
-    assert rel(x.grad, dx) < 1e-4
+    cmp.check("dx", x.grad, dx, 1e-4, cmp.frames())
     for k, t in params.items():
-        assert grad_err(k, t.grad, gr) < 1e-4, k
+        check_grad(k, t.grad, gr, 1e-4)
 
     # a zero-length utterance (a device vector is trusted and clamped): zero gradient, no NaN, no contribution
     x2 = x.detach().clone().requires_grad_(True)
@@ -208,7 +201,8 @@ def test_head_pool_varlen_backward_and_zero_length():
     _, gr0, _ = varlen_loss_and_grads_ref(fn, params, x.detach(), [0] + lengths[1:],
                                           lambda f, idx, n: (f * df[idx].double()).sum())
     for k, t in params.items():
-        assert torch.isfinite(t.grad).all() and grad_err(k, t.grad, gr0) < 1e-4, k
+        assert torch.isfinite(t.grad).all(), k
+        check_grad(k, t.grad, gr0, 1e-4)
 
 
 # -------------------------------------------------------------------------------------------------- block / layer / net
@@ -248,11 +242,11 @@ def test_block_mask_padding_vs_oracle(dtype, sequenced):
     loss_ref, gr, dx_ref = varlen_loss_and_grads_ref(block_fn, p64, x, lengths,
                                                      lambda o, idx, n: (o * wout[idx, :n].double()).sum())
     tol = TOL[dtype] if dtype == torch.float32 else 5e-2
-    assert rel(loss, loss_ref) < TOL[dtype]
-    assert rel(dx, dx_ref) < tol
+    assert cmp.rel(loss, loss_ref) < TOL[dtype]
+    cmp.check("dx", dx, dx_ref, tol, cmp.frames())
     assert len(grads) == 9
     for k, t in grads.items():
-        assert rel(t, gr[k]) < tol, k
+        check_grad(k, t, gr, tol)
 
 
 def test_block_native_and_sequenced_are_bit_identical_with_lengths():
@@ -313,10 +307,10 @@ def test_layer_mask_padding_vs_oracle(dtype):
     loss_ref, gr, dx_ref = varlen_loss_and_grads_ref(layer_fn, p64, x, lengths,
                                                      lambda o, idx, n: (o * wout[idx, :n].double()).sum())
     tol = 1e-4 if dtype == torch.float32 else 5e-2
-    assert rel(loss, loss_ref) < (1e-4 if dtype == torch.float32 else 2e-2)
-    assert rel(xg.grad, dx_ref) < tol
+    assert cmp.rel(loss, loss_ref) < (1e-4 if dtype == torch.float32 else 2e-2)
+    cmp.check("dx", xg.grad, dx_ref, tol, cmp.frames())
     for k, t in layer.named_parameters():
-        assert rel(t.grad, gr[k]) < tol, k
+        check_grad(k, t.grad, gr, tol)
 
 
 @pytest.mark.parametrize("dtype", [torch.float32, torch.bfloat16])
@@ -333,10 +327,10 @@ def test_backend_mask_padding_vs_oracle(dtype):
     loss_ref, gr, dx_ref = varlen_loss_and_grads_ref(
         backend_logits_fn(2), p64, x, lengths, lambda lg, idx, n: F.cross_entropy(lg, labels[idx], reduction="sum"))
     tol = 1e-4 if dtype == torch.float32 else 5e-2
-    assert rel(loss, loss_ref) < (1e-4 if dtype == torch.float32 else 2e-2)
-    assert rel(dx, dx_ref) < tol
+    assert cmp.rel(loss, loss_ref) < (1e-4 if dtype == torch.float32 else 2e-2)
+    cmp.check("dx", dx, dx_ref, tol, cmp.frames())
     for k, t in grads.items():
-        assert grad_err(k, t, gr) < tol, k
+        check_grad(k, t, gr, tol)
 
 
 @pytest.mark.parametrize("dtype,sequenced", [(torch.float32, True), (torch.bfloat16, False), (torch.bfloat16, True)])
@@ -455,7 +449,7 @@ def test_graphed_train_step_with_lengths():
                 backend_logits_fn(2), p64, xs[i], lens[1],
                 lambda lg, idx, n: F.cross_entropy(lg, labels[idx], reduction="sum"))
             for k, t in grads_g.items():
-                assert grad_err(k, t, gr) < 5e-2, k
+                check_grad(k, t, gr, 5e-2)
 
 
 def test_mask_padding_under_no_grad_scores_with_zero_padding():
@@ -469,4 +463,4 @@ def test_mask_padding_under_no_grad_scores_with_zero_padding():
         s_mask = net(x, lengths, mask_padding=True)[1]
         s_score = net(x, lengths)[1]
     assert bool((f[_pad_mask(lengths, T)] == 0).all())
-    assert rel(s_mask, s_score) < 1e-5
+    assert cmp.rel(s_mask, s_score) < 1e-5

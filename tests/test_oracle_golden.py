@@ -8,18 +8,13 @@ import pytest
 import torch
 
 from oracle import bimamba_oracle as orc
+from oracle.compare import rel as _rel
 
 RTOL = 2e-6   # fixtures store gradients as fp32 (6e-8 rounding); oracle runs in fp64
 
 
 def _load(golden_dir, name):
     return dict(np.load(os.path.join(golden_dir, name)))
-
-
-def _rel(a, b):
-    a = np.asarray(a, dtype=np.float64)
-    b = np.asarray(b, dtype=np.float64)
-    return np.abs(a - b).max() / max(np.abs(b).max(), 1e-30)
 
 
 @pytest.mark.parametrize("tag", ["small", "phase6"])
