@@ -485,6 +485,23 @@ int bimamba_block_fwd_varlen_train(const bimamba_block_desc* d, const int32_t* s
 int bimamba_block_bwd_varlen(const bimamba_block_desc* d, const bimamba_block_grads* g, const int32_t* seqlens,
                              bimamba_stream_t stream);
 
+/* ---- A second stream for the work that depends on the parameters only or produces parameter gradients.  The
+ * *_side calls fork it from `stream` with cudaEventRecord / cudaStreamWaitEvent and join it before they return, so
+ * they are safe under stream capture and their results are bitwise those of the single-stream calls (same kernels, same
+ * inputs).  `stream` NULL, or a NULL pointer to this struct: everything runs on `stream` in the single-stream order.
+ * The three events are the caller's (cudaEventCreateWithFlags(.., cudaEventDisableTiming)); calls that share them must
+ * not run concurrently from different host threads. */
+typedef struct bimamba_side_stream {
+  bimamba_stream_t stream; /* a cudaStream_t on the same device, not `stream` itself                     */
+  void* events[3];         /* cudaEvent_t                                                                */
+} bimamba_side_stream;
+
+/* The block backward with its parameter gradients on the side stream: the four weight-gradient products, the scan's and
+ * the conv's parameter sums and the layout pass run beside the data chain (in_proj / x_proj / dt_proj data gradients,
+ * scan and conv backward).  The block forward has no such call: its first product needs the packed weights. */
+int bimamba_block_bwd_side(const bimamba_block_desc* d, const bimamba_block_grads* g, const int32_t* seqlens,
+                           const bimamba_side_stream* side, bimamba_stream_t stream);
+
 /* ---- The whole encoder layer in one call each way: PN_BiMambas_Encoder.forward (DualStreamSEMamba.py:467-486)
  *   out = FFN(LN2(M(LN1 x) + flip(M(flip(LN1 x))))) + x,   FFN = Linear(d_model, d_ff) -> GELU (erf) -> Linear(d_ff, d_model)
  * and its complete backward.  x / out / dout / dx have x_dtype: fp32 (the reference's autocast arrangement: fp32
@@ -542,6 +559,34 @@ int bimamba_layer_bwd(const bimamba_layer_desc* d, const bimamba_layer_grads* g,
 int bimamba_layer_fwd_varlen_train(const bimamba_layer_desc* d, const int32_t* seqlens, bimamba_stream_t stream);
 int bimamba_layer_bwd_varlen(const bimamba_layer_desc* d, const bimamba_layer_grads* g, const int32_t* seqlens,
                              bimamba_stream_t stream);
+
+/* The block's per-step weight pack (bimamba_pack_weights): fp32 masters in, the arrangements the kernels read out. */
+typedef struct bimamba_block_pack {
+  const float* W_in;       /* (2*d_inner, d_model)  in_proj.weight                                       */
+  const float* W_x;        /* (dt_rank + 32, d_inner) x_proj.weight                                      */
+  const float* W_dt;       /* (d_inner, dt_rank)     dt_proj.weight                                      */
+  const float* A_log;      /* (d_inner, 16)                                                              */
+  const float* W_out;      /* (d_model, d_inner)     out_proj.weight                                     */
+  void* Wi;                /* outputs in block.io_dtype, layouts of bimamba_pack_weights                 */
+  void* WiT;
+  void* Wxp;
+  void* WxpT;
+  void* Wo2;
+  void* WoT;
+  void* WdT;
+  float* A;                /* (d_inner, 16) fp32 = -exp(A_log)                                           */
+} bimamba_block_pack;
+
+/* bimamba_layer_fwd_varlen_train (seqlens may be NULL) with the weight preparation inside the call.  pack != NULL: the
+ * call packs the block's weights first and uses pack->Wi, Wxp, Wo2 and A in place of d->block's (the transposed outputs
+ * are the backward's WiT, WxpT, WoT, WdT).  With a side stream the pack and the feed-forward weight casts run there,
+ * beside norm1, and the main stream waits for each just before the first product that reads it. */
+int bimamba_layer_fwd_side(const bimamba_layer_desc* d, const bimamba_block_pack* pack, const int32_t* seqlens,
+                           const bimamba_side_stream* side, bimamba_stream_t stream);
+/* bimamba_layer_bwd_varlen with every parameter gradient (bias column sums, weight-gradient products, both norms'
+ * dgamma / dbeta sums, the block's, see bimamba_block_bwd_side) on the side stream, joined once at the end. */
+int bimamba_layer_bwd_side(const bimamba_layer_desc* d, const bimamba_layer_grads* g, const int32_t* seqlens,
+                           const bimamba_side_stream* side, bimamba_stream_t stream);
 
 #ifdef __cplusplus
 }

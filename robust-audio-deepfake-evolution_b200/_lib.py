@@ -37,6 +37,7 @@ EXPORTS = (
     "bimamba_layer_fwd_varlen_train", "bimamba_layer_bwd_varlen", "bimamba_mask_frames",
     "bimamba_interp_frames_fwd", "bimamba_interp_frames_bwd", "bimamba_frame_mean", "bimamba_frame_mean_bwd",
     "bimamba_frame_scale", "bimamba_frame_scale_bwd_slices", "bimamba_frame_scale_bwd",
+    "bimamba_block_bwd_side", "bimamba_layer_fwd_side", "bimamba_layer_bwd_side",
 )
 
 
@@ -91,6 +92,17 @@ class LayerGrads(C.Structure):
         [(n, C.c_void_p) for n in ("dout", "dx", "dnorm1", "dnorm2", "dff_w1", "dff_b1", "dff_w2", "dff_b2")]
         + [("block", BlockGrads), ("workspace", C.c_void_p), ("workspace_bytes", C.c_size_t)]
     )
+
+
+class SideStream(C.Structure):
+    """Mirror of `struct bimamba_side_stream` (include/bimamba.h): the second stream of the *_side calls."""
+    _fields_ = [("stream", C.c_void_p), ("events", C.c_void_p * 3)]
+
+
+class BlockPack(C.Structure):
+    """Mirror of `struct bimamba_block_pack` (include/bimamba.h): the block's weight pack inside bimamba_layer_fwd_side."""
+    _fields_ = [(n, C.c_void_p) for n in ("W_in", "W_x", "W_dt", "A_log", "W_out", "Wi", "WiT", "Wxp", "WxpT", "Wo2", "WoT",
+                                          "WdT", "A")]
 
 
 _lib = None
@@ -248,6 +260,12 @@ def load() -> C.CDLL:
         lib.bimamba_layer_fwd_varlen_train.argtypes = [C.POINTER(LayerDesc), vp, vp]
         lib.bimamba_layer_bwd_varlen.restype = i32
         lib.bimamba_layer_bwd_varlen.argtypes = [C.POINTER(LayerDesc), C.POINTER(LayerGrads), vp, vp]
+        lib.bimamba_block_bwd_side.restype = i32
+        lib.bimamba_block_bwd_side.argtypes = [C.POINTER(BlockDesc), C.POINTER(BlockGrads), vp, C.POINTER(SideStream), vp]
+        lib.bimamba_layer_fwd_side.restype = i32
+        lib.bimamba_layer_fwd_side.argtypes = [C.POINTER(LayerDesc), C.POINTER(BlockPack), vp, C.POINTER(SideStream), vp]
+        lib.bimamba_layer_bwd_side.restype = i32
+        lib.bimamba_layer_bwd_side.argtypes = [C.POINTER(LayerDesc), C.POINTER(LayerGrads), vp, C.POINTER(SideStream), vp]
         lib.bimamba_mask_frames.restype = i32
         lib.bimamba_mask_frames.argtypes = [vp, vp, vp, i32, i32, i32, i32, vp]
         for name in ("bimamba_interp_frames_fwd", "bimamba_interp_frames_bwd"):

@@ -16,6 +16,52 @@ namespace bimamba {
 
 static inline size_t up256(size_t v) { return (v + 255) & ~(size_t)255; }
 
+// The caller's second stream (bimamba_side_stream).  Without one every launch goes to the main stream, in the order of
+// the single-stream calls.  Event 0 forks, events 1 and 2 join; a wait is issued after its record, so recording the same
+// event again later in the call does not disturb it.
+struct Fork {
+  cudaStream_t main = nullptr, side = nullptr;
+  cudaEvent_t ev[3] = {};
+
+  // The stream for work that may run beside the main chain from here on: the side stream, once it has waited for
+  // everything enqueued on the main stream so far; without a side stream the main stream itself.
+  int branch(cudaStream_t* st) {
+    *st = main;
+    if (!side) return 0;
+    if (cudaEventRecord(ev[0], main) != cudaSuccess || cudaStreamWaitEvent(side, ev[0], 0) != cudaSuccess) {
+      set_err("side stream: fork failed");
+      return -11;
+    }
+    *st = side;
+    return 0;
+  }
+  // mark(k) records what the side stream holds so far; wait(k) makes the main stream wait for that mark.
+  int mark(int k) {
+    if (side && cudaEventRecord(ev[k], side) != cudaSuccess) { set_err("side stream: event record failed"); return -11; }
+    return 0;
+  }
+  int wait(int k) {
+    if (side && cudaStreamWaitEvent(main, ev[k], 0) != cudaSuccess) { set_err("side stream: join failed"); return -11; }
+    return 0;
+  }
+  int join() {
+    const int rc = mark(1);
+    return rc ? rc : wait(1);
+  }
+};
+
+static int make_fork(const bimamba_side_stream* s, bimamba_stream_t stream, Fork* f) {
+  f->main = reinterpret_cast<cudaStream_t>(stream);
+  if (!s || !s->stream) return 0;
+  if (s->stream == stream) { set_err("side stream: must differ from the main stream"); return -11; }
+  for (int i = 0; i < 3; ++i) {
+    if (!s->events[i]) { set_err("side stream: three events are required"); return -11; }
+    f->ev[i] = reinterpret_cast<cudaEvent_t>(s->events[i]);
+  }
+  f->side = reinterpret_cast<cudaStream_t>(s->stream);
+  return 0;
+}
+
 struct FwdCarve {
   size_t xz, xc, xdbl, y, ckpt, ypre, total;
   int nck;
@@ -199,8 +245,13 @@ extern "C" int bimamba_block_bwd(const bimamba_block_desc* d, const bimamba_bloc
 
 // seqlens != NULL: the backward of bimamba_block_fwd_varlen_train (same seqlens).  The scan and the conv walk each
 // utterance's own frames and write zero gradients at padded frames, so every product over the rows sees zeros there.
-extern "C" int bimamba_block_bwd_varlen(const bimamba_block_desc* d, const bimamba_block_grads* g, const int32_t* seqlens,
-                                        bimamba_stream_t stream) {
+namespace bimamba {
+
+// The block backward.  Parameter-gradient work (the four weight-gradient products, the scan's and the conv's parameter
+// sums, the layout pass) goes to f.branch(), the data chain to the main stream; the side stream is not joined here.
+static int block_bwd(const bimamba_block_desc* d, const bimamba_block_grads* g, const int32_t* seqlens, Fork& f) {
+  bimamba_stream_t stream = f.main;
+  cudaStream_t side = nullptr;
   int rc = check_block(d);
   if (rc) return rc;
   if (!g) { set_err("block_bwd: null gradient descriptor"); return -1; }
@@ -246,7 +297,8 @@ extern "C" int bimamba_block_bwd_varlen(const bimamba_block_desc* d, const bimam
 #define BIMAMBA_TRY(call) do { rc = (call); if (rc) return rc; } while (0)
   // out_proj: weight gradient over [y_fwd | y_rev] (folded over the directions by the layout pass) and dy, which both
   // directions share
-  BIMAMBA_TRY(bimamba_gemm_tn(g->dout, dm, y, (int64_t)nd * D, dWo2, tn_part, M, dm, nd * D, dt, stream));
+  BIMAMBA_TRY(f.branch(&side));
+  BIMAMBA_TRY(bimamba_gemm_tn(g->dout, dm, y, (int64_t)nd * D, dWo2, tn_part, M, dm, nd * D, dt, side));
   BIMAMBA_TRY(bimamba_gemm_nt(g->dout, dm, g->WoT, dm, dy, D, nullptr, nullptr, M, D, dm, dt, dt, stream));
   // scan backward, both directions in one launch
   bimamba_scan_desc s;
@@ -260,14 +312,16 @@ extern "C" int bimamba_block_bwd_varlen(const bimamba_block_desc* d, const bimam
   BIMAMBA_TRY(bimamba_selective_scan_bwd_varlen(&s, seqlens, stream));
   // [dB | dC]: fixed-order sum over the channel groups, written next to where ddt_r goes (no concatenation)
   BIMAMBA_TRY(bimamba_reduce_rows32(dbc_part, dxdbl, B, w.ngroups, L * nd, kXW, dt, stream));
-  BIMAMBA_TRY(bimamba_reduce_partials(dA_part, dA, 1, B * nd, (int64_t)D * kN, 0, (int64_t)D * kN, 0, BIMAMBA_F32, 0, stream));
-  BIMAMBA_TRY(bimamba_reduce_partials(dD_part, g->dD, 1, B * nd, D, 0, D, 0, BIMAMBA_F32, 0, stream));
-  BIMAMBA_TRY(bimamba_reduce_partials(db_part, g->db_dt, 1, B * nd, D, 0, D, 0, BIMAMBA_F32, 0, stream));
+  BIMAMBA_TRY(f.branch(&side));
+  BIMAMBA_TRY(bimamba_reduce_partials(dA_part, dA, 1, B * nd, (int64_t)D * kN, 0, (int64_t)D * kN, 0, BIMAMBA_F32, 0, side));
+  BIMAMBA_TRY(bimamba_reduce_partials(dD_part, g->dD, 1, B * nd, D, 0, D, 0, BIMAMBA_F32, 0, side));
+  BIMAMBA_TRY(bimamba_reduce_partials(db_part, g->db_dt, 1, B * nd, D, 0, D, 0, BIMAMBA_F32, 0, side));
   // dt_proj: data gradient into columns 32..47 of the same rows; weight gradient against the saved x_proj rows
   BIMAMBA_TRY(bimamba_gemm_nt(ddelta, D, g->WdT, D, static_cast<unsigned char*>(dxdbl) + (size_t)2 * kN * es, kXW, nullptr, nullptr,
                               M * nd, BIMAMBA_MAX_DT_RANK, D, dt, dt, stream));
-  BIMAMBA_TRY(bimamba_gemm_tn(ddelta, D, xdbl, kXW, dWdtf, tn_part, M * nd, D, kXW, dt, stream));
-  BIMAMBA_TRY(bimamba_gemm_tn(dxdbl, kXW, xc, D, dWxp, tn_part, M * nd, kXW, D, dt, stream));
+  BIMAMBA_TRY(f.branch(&side));
+  BIMAMBA_TRY(bimamba_gemm_tn(ddelta, D, xdbl, kXW, dWdtf, tn_part, M * nd, D, kXW, dt, side));
+  BIMAMBA_TRY(bimamba_gemm_tn(dxdbl, kXW, xc, D, dWxp, tn_part, M * nd, kXW, D, dt, side));
   // x_proj data gradient + the scan's du
   BIMAMBA_TRY(bimamba_gemm_nt(dxdbl, kXW, g->WxpT, kXW, dxc, D, nullptr, du, M * nd, D, kXW, dt, dt, stream));
   // conv backward: dx into the x half and dz_fwd + dz_rev into the z half of one [dx | dz] matrix
@@ -275,16 +329,35 @@ extern "C" int bimamba_block_bwd_varlen(const bimamba_block_desc* d, const bimam
                                                static_cast<unsigned char*>(dxz) + (size_t)D * es, conv_part, seqlens, (int)B, nd,
                                                D, (int)L, K, L * 2 * D, 2 * D, L * nd * D, D, (int64_t)nd * D, L * 2 * D, 2 * D,
                                                dt, BIMAMBA_FLAG_SILU, stream));
+  BIMAMBA_TRY(f.branch(&side));
   BIMAMBA_TRY(bimamba_reduce_partials(conv_part, dwb, 1, w.conv_slices, (int64_t)D * (K + 1), 0, (int64_t)D * (K + 1), 0,
-                                      BIMAMBA_F32, 0, stream));
+                                      BIMAMBA_F32, 0, side));
   // in_proj
-  BIMAMBA_TRY(bimamba_gemm_tn(dxz, 2 * D, d->x, dm, g->dW_in, tn_part, M, 2 * D, dm, dt, stream));
+  BIMAMBA_TRY(bimamba_gemm_tn(dxz, 2 * D, d->x, dm, g->dW_in, tn_part, M, 2 * D, dm, dt, side));
   BIMAMBA_TRY(bimamba_gemm_nt(dxz, 2 * D, g->WiT, 2 * D, g->dx, dm, nullptr, nullptr, M, dm, 2 * D, dt, dt, stream));
   // the reference's parameter layouts (dA_log = dA * A, x_proj row order, dt_proj slice, out_proj fold, conv split)
   BIMAMBA_TRY(bimamba_finalize_param_grads(dA, d->A, dWxp, dWdtf, dWo2, dwb, g->dA_log, g->dW_x, g->dW_dt, g->dW_out,
-                                           g->dconv_w, g->dconv_b, dm, D, kN, R, nd, K, stream));
+                                           g->dconv_w, g->dconv_b, dm, D, kN, R, nd, K, side));
 #undef BIMAMBA_TRY
   return 0;
+}
+
+}  // namespace bimamba
+
+extern "C" int bimamba_block_bwd_varlen(const bimamba_block_desc* d, const bimamba_block_grads* g, const int32_t* seqlens,
+                                        bimamba_stream_t stream) {
+  return bimamba_block_bwd_side(d, g, seqlens, nullptr, stream);
+}
+
+// side != NULL with a stream: the parameter-gradient work runs on side->stream beside the data chain, joined before the
+// call returns.  Same kernels, same inputs: results are bitwise those of the single-stream call.
+extern "C" int bimamba_block_bwd_side(const bimamba_block_desc* d, const bimamba_block_grads* g, const int32_t* seqlens,
+                                      const bimamba_side_stream* side, bimamba_stream_t stream) {
+  Fork f;
+  int rc = make_fork(side, stream, &f);
+  if (!rc) rc = block_bwd(d, g, seqlens, f);
+  const int rj = f.join();     // also after an error: no fork is left open
+  return rc ? rc : rj;
 }
 
 
@@ -323,7 +396,7 @@ static LayerFwdCarve carve_layer_fwd(int64_t B, int64_t L, int dm, int D, int df
 }
 
 struct LayerBwdCarve {
-  size_t g, da, dh, dmn, dmo, dxn, cs_part, ln_part, tn_part, block, total;
+  size_t g, da, dh, dmn, dmo, dxn, cs_part, ln_part1, ln_part2, tn_part, block, total;
   int cs_slices, ln_blocks;
 };
 
@@ -341,7 +414,10 @@ static LayerBwdCarve carve_layer_bwd(int64_t B, int64_t L, int dm, int D, int df
   c.dmo = take(M * dm * es);
   c.dxn = take(M * dm * es);
   c.cs_part = take((size_t)(c.cs_slices > 0 ? c.cs_slices : 1) * dff * 4);
-  c.ln_part = take((size_t)(c.ln_blocks > 0 ? c.ln_blocks : 1) * 2 * dm * 4);
+  // one partial buffer per norm: norm1's backward (main stream) may run while norm2's sum (side stream) still reads its
+  // own.  The column sums and the products share theirs: they all run on the one side queue, in order.
+  c.ln_part1 = take((size_t)(c.ln_blocks > 0 ? c.ln_blocks : 1) * 2 * dm * 4);
+  c.ln_part2 = take((size_t)(c.ln_blocks > 0 ? c.ln_blocks : 1) * 2 * dm * 4);
   size_t tn = (size_t)bimamba_gemm_tn_splits((int64_t)M, dm, dff) * dm * dff * 4;
   const size_t tn2 = (size_t)bimamba_gemm_tn_splits((int64_t)M, dff, dm) * dm * dff * 4;
   if (tn2 > tn) tn = tn2;
@@ -401,22 +477,55 @@ extern "C" int bimamba_layer_fwd_varlen(const bimamba_layer_desc* d, const int32
 }
 
 extern "C" int bimamba_layer_fwd_varlen_train(const bimamba_layer_desc* d, const int32_t* seqlens, bimamba_stream_t stream) {
+  return bimamba_layer_fwd_side(d, nullptr, seqlens, nullptr, stream);
+}
+
+// pack != NULL: the block's weights are packed from the fp32 masters first (bimamba_pack_weights), so the call needs
+// nothing prepared per step.  With a side stream the pack and the two feed-forward weight casts run there, beside norm1,
+// and the main stream waits for each just before its first product.
+extern "C" int bimamba_layer_fwd_side(const bimamba_layer_desc* d, const bimamba_block_pack* pack, const int32_t* seqlens,
+                                      const bimamba_side_stream* side, bimamba_stream_t stream) {
   int rc = check_layer(d);
   if (rc) return rc;
   bimamba_block_desc k = d->block;
   if (k.batch == 0 || k.seqlen == 0) return 0;
+  if (pack && (!pack->W_in || !pack->W_x || !pack->W_dt || !pack->A_log || !pack->W_out || !pack->Wi || !pack->WiT ||
+               !pack->Wxp || !pack->WxpT || !pack->Wo2 || !pack->WoT || !pack->WdT || !pack->A)) {
+    set_err("layer_fwd: null operand in the weight pack");
+    return -7;
+  }
   const int es = 2, cd = k.io_dtype, xd = d->x_dtype;
   const int64_t B = k.batch, L = k.seqlen, M = B * L;
   const int dm = k.d_model, D = k.d_inner, dff = d->d_ff, nd = k.ndir;
   const bool save = k.save_for_backward != 0;
   const LayerFwdCarve c = carve_layer_fwd(B, L, dm, D, dff, nd, es, save);
   if (d->workspace_bytes < c.total) { set_err("layer_fwd: workspace too small (bimamba_layer_fwd_workspace_bytes)"); return -10; }
+  if (pack) { k.Wi = pack->Wi; k.Wxp = pack->Wxp; k.Wo2 = pack->Wo2; k.A = pack->A; }
+  Fork f;
+  rc = make_fork(side, stream, &f);
+  if (rc) return rc;
   unsigned char* ws = static_cast<unsigned char*>(d->workspace);
   void *xn = ws + c.xn, *mo = ws + c.mo, *mn = ws + c.mn, *h = ws + c.h, *a = ws + c.a;
   float* st = reinterpret_cast<float*>(ws + c.stats);
   float *mean1 = save ? st : nullptr, *rstd1 = save ? st + M : nullptr, *mean2 = save ? st + 2 * M : nullptr,
         *rstd2 = save ? st + 3 * M : nullptr;
-#define BIMAMBA_TRY(call) do { rc = (call); if (rc) return rc; } while (0)
+  cudaStream_t wst = nullptr;
+#define BIMAMBA_TRY(call) do { rc = (call); if (rc) { f.join(); return rc; } } while (0)
+  // the weights: they depend on the parameters only (one branch, forked before anything of this layer)
+  BIMAMBA_TRY(f.branch(&wst));
+  if (pack) {
+    BIMAMBA_TRY(bimamba_pack_weights(pack->W_in, pack->W_x, pack->W_dt, pack->A_log, pack->W_out, pack->Wi, pack->WiT, pack->Wxp,
+                                     pack->WxpT, pack->Wo2, pack->WoT, pack->WdT, pack->A, dm, D, kN, k.dt_rank, nd, cd, wst));
+  }
+  BIMAMBA_TRY(f.mark(1));
+  // feed-forward weights cast (and transposed for the backward); on one stream they stay where the single-stream call
+  // has always issued them, after norm2
+  auto ff_weights = [&]() {
+    int r = bimamba_cast_transpose(d->ff_w1, ws + c.w1c, ws + c.w1t, dff, dm, cd, wst);
+    return r ? r : bimamba_cast_transpose(d->ff_w2, ws + c.w2c, ws + c.w2t, dm, dff, cd, wst);
+  };
+  if (f.side) BIMAMBA_TRY(ff_weights());
+  BIMAMBA_TRY(f.mark(2));
   // norm1, written in the compute dtype (DualStreamSEMamba.py:472)
   BIMAMBA_TRY(bimamba_layernorm_fwd(d->x, d->norm1_w, d->norm1_b, xn, mean1, rstd1, M, dm, d->eps1, xd, cd, stream));
   // the bidirectional block (:473-481)
@@ -424,13 +533,14 @@ extern "C" int bimamba_layer_fwd_varlen_train(const bimamba_layer_desc* d, const
   k.out = mo;
   k.workspace = ws + c.block;
   k.workspace_bytes = d->workspace_bytes - c.block;
+  BIMAMBA_TRY(f.wait(1));
   BIMAMBA_TRY(bimamba_block_fwd_varlen_train(&k, seqlens, stream));
   // norm2 (:482)
   BIMAMBA_TRY(bimamba_layernorm_fwd(mo, d->norm2_w, d->norm2_b, mn, mean2, rstd2, M, dm, d->eps2, cd, cd, stream));
-  // feed-forward + residual (:483-485): weights cast (and transposed for the backward), two products with the bias and
-  // the residual in their epilogues, exact GELU in between
-  BIMAMBA_TRY(bimamba_cast_transpose(d->ff_w1, ws + c.w1c, ws + c.w1t, dff, dm, cd, stream));
-  BIMAMBA_TRY(bimamba_cast_transpose(d->ff_w2, ws + c.w2c, ws + c.w2t, dm, dff, cd, stream));
+  if (!f.side) BIMAMBA_TRY(ff_weights());
+  // feed-forward + residual (:483-485): two products with the bias and the residual in their epilogues, exact GELU in
+  // between
+  BIMAMBA_TRY(f.wait(2));
   BIMAMBA_TRY(bimamba_gemm_nt(mn, dm, ws + c.w1c, dm, h, dff, d->ff_b1, nullptr, M, dff, dm, cd, cd, stream));
   BIMAMBA_TRY(bimamba_gelu_fwd(h, a, M * dff, cd, stream));
   BIMAMBA_TRY(bimamba_gemm_nt(a, dff, ws + c.w2c, dff, d->out, dm, d->ff_b2, d->x, M, dm, dff, cd, xd, stream));
@@ -446,6 +556,16 @@ extern "C" int bimamba_layer_bwd(const bimamba_layer_desc* d, const bimamba_laye
 // The norms and the feed-forward are per row: for the masked contract dout must be zero at padded frames.
 extern "C" int bimamba_layer_bwd_varlen(const bimamba_layer_desc* d, const bimamba_layer_grads* g, const int32_t* seqlens,
                                         bimamba_stream_t stream) {
+  return bimamba_layer_bwd_side(d, g, seqlens, nullptr, stream);
+}
+
+namespace bimamba {
+
+// The layer backward: the data chain on the main stream; every parameter gradient (bias column sums, weight-gradient
+// products, both norms' dgamma / dbeta sums and the block's, see block_bwd) on f.branch(), joined by the caller.
+static int layer_bwd(const bimamba_layer_desc* d, const bimamba_layer_grads* g, const int32_t* seqlens, Fork& f) {
+  bimamba_stream_t stream = f.main;
+  cudaStream_t side = nullptr;
   int rc = check_layer(d);
   if (rc) return rc;
   if (!g) { set_err("layer_bwd: null gradient descriptor"); return -1; }
@@ -470,8 +590,8 @@ extern "C" int bimamba_layer_bwd_varlen(const bimamba_layer_desc* d, const bimam
   const float* st = reinterpret_cast<const float*>(fs + c.stats);
   const float *mean1 = st, *rstd1 = st + M, *mean2 = st + 2 * M, *rstd2 = st + 3 * M;
   void *da = bs + w.da, *dh = bs + w.dh, *dmn = bs + w.dmn, *dmo = bs + w.dmo, *dxn = bs + w.dxn;
-  float *cs_part = reinterpret_cast<float*>(bs + w.cs_part), *ln_part = reinterpret_cast<float*>(bs + w.ln_part),
-        *tn_part = reinterpret_cast<float*>(bs + w.tn_part);
+  float *cs_part = reinterpret_cast<float*>(bs + w.cs_part), *ln_part1 = reinterpret_cast<float*>(bs + w.ln_part1),
+        *ln_part2 = reinterpret_cast<float*>(bs + w.ln_part2), *tn_part = reinterpret_cast<float*>(bs + w.tn_part);
 #define BIMAMBA_TRY(call) do { rc = (call); if (rc) return rc; } while (0)
   // feed-forward backward; its incoming gradient is also the residual branch's (added inside norm1's backward below)
   const void* gy = g->dout;
@@ -479,18 +599,21 @@ extern "C" int bimamba_layer_bwd_varlen(const bimamba_layer_desc* d, const bimam
     BIMAMBA_TRY(bimamba_cast(g->dout, bs + w.g, M * dm, xd, cd, stream));
     gy = bs + w.g;
   }
-  BIMAMBA_TRY(bimamba_colsum(gy, cs_part, M, dm, dm, cd, stream));
-  BIMAMBA_TRY(bimamba_reduce_partials(cs_part, g->dff_b2, 1, w.cs_slices, dm, 0, dm, 0, BIMAMBA_F32, 0, stream));
-  BIMAMBA_TRY(bimamba_gemm_tn(gy, dm, a, dff, g->dff_w2, tn_part, M, dm, dff, cd, stream));
+  BIMAMBA_TRY(f.branch(&side));
+  BIMAMBA_TRY(bimamba_colsum(gy, cs_part, M, dm, dm, cd, side));
+  BIMAMBA_TRY(bimamba_reduce_partials(cs_part, g->dff_b2, 1, w.cs_slices, dm, 0, dm, 0, BIMAMBA_F32, 0, side));
+  BIMAMBA_TRY(bimamba_gemm_tn(gy, dm, a, dff, g->dff_w2, tn_part, M, dm, dff, cd, side));
   BIMAMBA_TRY(bimamba_gemm_nt(gy, dm, fs + c.w2t, dm, da, dff, nullptr, nullptr, M, dff, dm, cd, cd, stream));
   BIMAMBA_TRY(bimamba_gelu_bwd(h, da, dh, M * dff, cd, stream));
-  BIMAMBA_TRY(bimamba_colsum(dh, cs_part, M, dff, dff, cd, stream));
-  BIMAMBA_TRY(bimamba_reduce_partials(cs_part, g->dff_b1, 1, w.cs_slices, dff, 0, dff, 0, BIMAMBA_F32, 0, stream));
-  BIMAMBA_TRY(bimamba_gemm_tn(dh, dff, mn, dm, g->dff_w1, tn_part, M, dff, dm, cd, stream));
+  BIMAMBA_TRY(f.branch(&side));
+  BIMAMBA_TRY(bimamba_colsum(dh, cs_part, M, dff, dff, cd, side));
+  BIMAMBA_TRY(bimamba_reduce_partials(cs_part, g->dff_b1, 1, w.cs_slices, dff, 0, dff, 0, BIMAMBA_F32, 0, side));
+  BIMAMBA_TRY(bimamba_gemm_tn(dh, dff, mn, dm, g->dff_w1, tn_part, M, dff, dm, cd, side));
   BIMAMBA_TRY(bimamba_gemm_nt(dh, dff, fs + c.w1t, dff, dmn, dm, nullptr, nullptr, M, dm, dff, cd, cd, stream));
   // norm2 backward
-  BIMAMBA_TRY(bimamba_layernorm_bwd(mo, dmn, d->norm2_w, mean2, rstd2, nullptr, dmo, ln_part, M, dm, cd, cd, stream));
-  BIMAMBA_TRY(bimamba_reduce_partials(ln_part, g->dnorm2, 1, w.ln_blocks, 2 * dm, 0, 2 * dm, 0, BIMAMBA_F32, 0, stream));
+  BIMAMBA_TRY(bimamba_layernorm_bwd(mo, dmn, d->norm2_w, mean2, rstd2, nullptr, dmo, ln_part2, M, dm, cd, cd, stream));
+  BIMAMBA_TRY(f.branch(&side));
+  BIMAMBA_TRY(bimamba_reduce_partials(ln_part2, g->dnorm2, 1, w.ln_blocks, 2 * dm, 0, 2 * dm, 0, BIMAMBA_F32, 0, side));
   // the block
   k.x = xn;
   k.out = mo;
@@ -501,10 +624,25 @@ extern "C" int bimamba_layer_bwd_varlen(const bimamba_layer_desc* d, const bimam
   kg.dx = dxn;
   kg.workspace = bs + w.block;
   kg.workspace_bytes = g->workspace_bytes - w.block;
-  BIMAMBA_TRY(bimamba_block_bwd_varlen(&k, &kg, seqlens, stream));
+  BIMAMBA_TRY(block_bwd(&k, &kg, seqlens, f));
   // norm1 backward + the residual branch's gradient
-  BIMAMBA_TRY(bimamba_layernorm_bwd(d->x, dxn, d->norm1_w, mean1, rstd1, g->dout, g->dx, ln_part, M, dm, xd, cd, stream));
-  BIMAMBA_TRY(bimamba_reduce_partials(ln_part, g->dnorm1, 1, w.ln_blocks, 2 * dm, 0, 2 * dm, 0, BIMAMBA_F32, 0, stream));
+  BIMAMBA_TRY(bimamba_layernorm_bwd(d->x, dxn, d->norm1_w, mean1, rstd1, g->dout, g->dx, ln_part1, M, dm, xd, cd, stream));
+  BIMAMBA_TRY(f.branch(&side));
+  BIMAMBA_TRY(bimamba_reduce_partials(ln_part1, g->dnorm1, 1, w.ln_blocks, 2 * dm, 0, 2 * dm, 0, BIMAMBA_F32, 0, side));
 #undef BIMAMBA_TRY
   return 0;
+}
+
+}  // namespace bimamba
+
+// side != NULL with a stream: the parameter-gradient work of the feed-forward, the norms and the block runs on
+// side->stream beside the data chain, and the main stream waits for it once, before the call returns.  Same kernels,
+// same inputs: results are bitwise those of the single-stream call.
+extern "C" int bimamba_layer_bwd_side(const bimamba_layer_desc* d, const bimamba_layer_grads* g, const int32_t* seqlens,
+                                      const bimamba_side_stream* side, bimamba_stream_t stream) {
+  Fork f;
+  int rc = make_fork(side, stream, &f);
+  if (!rc) rc = layer_bwd(d, g, seqlens, f);
+  const int rj = f.join();     // also after an error: no fork is left open
+  return rc ? rc : rj;
 }

@@ -40,8 +40,8 @@ class PN_BiMambas_Encoder(nn.Module):
             if not mask_padding:
                 _forward_only(seqlens, x, *self.parameters())
         if native_layer_ok(x, self):
-            # eager mode: the whole layer in one native call each way (same kernels, same order, same bits; a captured
-            # step keeps the sequenced Functions below, which overlap the weight-gradient products on a second stream)
+            # the whole layer in one native call each way, eager and captured (same kernels, same bits as the sequenced
+            # Functions below; weight preparation and parameter gradients on a second stream)
             return encoder_layer_native(x, self, seqlens, mask_padding)
         if mask_padding:
             x = mask_frames(x, seqlens)

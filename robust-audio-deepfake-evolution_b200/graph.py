@@ -5,12 +5,20 @@ launch-latency bound (SURVEY 3.5, 7.2); capturing it once and replaying removes 
 loop.  This plays the role a tracing compiler would: explicit capture, static buffers."""
 from __future__ import annotations
 
+import contextlib
 import copy
 from typing import Callable, Optional
 
 import torch
 
-from .ops import seqlens_tensor, sequenced_block
+from . import ops
+from .ops import seqlens_tensor
+
+
+def _as_captured():
+    """The warm-up runs the arrangement the capture records: the native layer calls with their second stream, or, with
+    the side stream switched off (BIMAMBA_SIDE_STREAM=0), the sequenced Functions."""
+    return contextlib.nullcontext() if ops.SIDE_STREAM else ops.sequenced_block()
 
 
 def _snapshot(optimizer):
@@ -68,7 +76,7 @@ class GraphedTrainStep:
         snap = _snapshot(optimizer) if (optimizer is not None and restore_after_warmup) else None
         side = torch.cuda.Stream()
         side.wait_stream(torch.cuda.current_stream())
-        with torch.cuda.stream(side), sequenced_block():   # warm up what the capture records, not the eager fast path
+        with torch.cuda.stream(side), _as_captured():
             for _ in range(max(1, warmup)):          # lazy inits (cuBLAS handles, func attributes) happen here
                 zero_grad()
                 loss = step_fn(*args)
@@ -161,7 +169,7 @@ class GraphedForward:
             args = (self.static_x, self.static_lengths)
         side = torch.cuda.Stream()
         side.wait_stream(torch.cuda.current_stream())
-        with torch.cuda.stream(side), torch.no_grad(), sequenced_block():
+        with torch.cuda.stream(side), torch.no_grad(), _as_captured():
             for _ in range(max(1, warmup)):
                 fn(*args)
         torch.cuda.current_stream().wait_stream(side)

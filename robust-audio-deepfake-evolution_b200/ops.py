@@ -11,11 +11,12 @@ Public names mirror what the reference's path binds upstream:
 
 All arithmetic runs in the CUDA library (ops on CPU tensors raise: there is no fallback).
 
-Two arrangements of the same kernels, bit-identical in their results: outside CUDA-graph capture the block and the whole
-encoder layer go through the library's one-call entry points (``BiMambaNativeFn`` / ``EncoderLayerNativeFn`` ->
-bimamba_block_fwd/bwd, bimamba_layer_fwd/bwd: device-bound eager steps); under capture - and inside
-``sequenced_block()`` - the Functions below enqueue the kernels one by one and overlap the weight-gradient products on a
-second stream.
+Two arrangements of the same kernels, bit-identical in their results: the whole encoder layer goes through the
+library's one-call entry points (``EncoderLayerNativeFn`` -> bimamba_layer_fwd_side / bimamba_layer_bwd_side, which put
+the weight preparation and the parameter gradients on a second stream), eager and under CUDA-graph capture, and outside
+capture so does a lone block (``BiMambaNativeFn`` -> bimamba_block_fwd/bwd); inside ``sequenced_block()`` - and for
+fp32 compute - the Functions below enqueue the kernels one by one and overlap the weight-gradient products on a second
+stream.
 
 Layout.  The kernels are channel-last: every activation is (batch, time, channel) with unit channel
 stride, the layout the projections produce and consume, so the block has no transposes.  Tensors
@@ -121,6 +122,30 @@ class _Fork:
     def join(self):
         if self.side is not None:
             self.cur.wait_stream(self.side)
+
+
+_SIDE_ABI = {}
+
+
+def _side_stream(dev: int):
+    """The bimamba_side_stream of the native layer calls on device `dev`: the side stream of _Fork and three events, made
+    once per device (each event is recorded once here so that it exists before any call hands it to the library)."""
+    if dev not in _SIDE_ABI:
+        if dev not in _SIDE:
+            _SIDE[dev] = torch.cuda.Stream(device=dev)
+        evs = [torch.cuda.Event() for _ in range(3)]
+        for e in evs:
+            e.record(torch.cuda.current_stream(dev))
+        s = _lib.SideStream()
+        s.stream = _SIDE[dev].cuda_stream
+        for i, e in enumerate(evs):
+            s.events[i] = e.cuda_event
+        _SIDE_ABI[dev] = (s, evs)
+    return _SIDE_ABI[dev][0]
+
+
+def _side_ptr(side):
+    return None if side is None else C.byref(side)
 
 
 def _wants_grad(*ts) -> bool:
@@ -1091,6 +1116,21 @@ def layer_norm_fn(x, weight, bias, eps=1e-5, out_dtype=None, with_residual=False
 # ----------------------------------------------------------------------------------------
 # the fused block: both directions, shared weights
 # ----------------------------------------------------------------------------------------
+def _pack_buffers(W_in, A_log, ndir: int, dtype):
+    """Uninitialised outputs of bimamba_pack_weights: (Wi, WiT, Wxp, WxpT, Wo2, WoT, WdT) in `dtype` and A fp32."""
+    D2, dm = W_in.shape
+    D = D2 // 2
+    N = A_log.shape[1]
+    sizes = (D2 * dm, D2 * dm, XW * D, XW * D, dm * ndir * D, D * dm, MAX_DT_RANK * D)
+    flat = torch.empty((sum(sizes),), device=W_in.device, dtype=dtype)
+    shapes = ((D2, dm), (dm, D2), (XW, D), (D, XW), (dm, ndir * D), (D, dm), (MAX_DT_RANK, D))
+    outs, off = [], 0
+    for n_, sh in zip(sizes, shapes):       # every size is a multiple of 8 elements -> 16-byte aligned views
+        outs.append(flat[off:off + n_].view(sh))
+        off += n_
+    return (*outs, torch.empty((D, N), device=W_in.device, dtype=torch.float32))
+
+
 def pack_weights(W_in, W_x, W_dt, A_log, W_out, ndir: int, dtype):
     """One launch: fp32 master parameters -> (Wi, WiT, Wxp, WxpT, Wo2, WoT, WdT) in `dtype` and A = -exp(A_log) fp32
     (layouts in include/bimamba.h: bimamba_pack_weights)."""
@@ -1099,14 +1139,7 @@ def pack_weights(W_in, W_x, W_dt, A_log, W_out, ndir: int, dtype):
     D = D2 // 2
     N = A_log.shape[1]
     R = W_dt.shape[1]
-    sizes = (D2 * dm, D2 * dm, XW * D, XW * D, dm * ndir * D, D * dm, MAX_DT_RANK * D)
-    flat = torch.empty((sum(sizes),), device=W_in.device, dtype=dtype)
-    shapes = ((D2, dm), (dm, D2), (XW, D), (D, XW), (dm, ndir * D), (D, dm), (MAX_DT_RANK, D))
-    outs, off = [], 0
-    for n_, sh in zip(sizes, shapes):       # every size is a multiple of 8 elements -> 16-byte aligned views
-        outs.append(flat[off:off + n_].view(sh))
-        off += n_
-    A32 = torch.empty((D, N), device=W_in.device, dtype=torch.float32)
+    *outs, A32 = _pack_buffers(W_in, A_log, ndir, dtype)
     srcs = [_f32c(t) for t in (W_in, W_x, W_dt, A_log, W_out)]
     with _timed("pack"):
         _lib.check(lib.bimamba_pack_weights(*[_ptr(t) for t in srcs], *[_ptr(t) for t in outs], _ptr(A32),
@@ -1378,9 +1411,10 @@ class NativeBlock:
         _lib.check(fwd(C.byref(d), _ptr(seqlens), _stream()), "bimamba_block_fwd_varlen")
         _lib.launch_count += 4           # the call enqueues 5 kernels (3 GEMMs, conv, scan)
 
-    def backward(self, dout):
+    def backward(self, dout, two_stream=None):
         """-> (dx, dW_in, dconv_w, dconv_b, dW_x, dW_dt, db_dt, dA_log, dD, dW_out), fp32 parameter gradients in the
-        reference's shapes."""
+        reference's shapes.  two_stream (default: SIDE_STREAM): the parameter gradients run on a second stream
+        (bimamba_block_bwd_side); the same bits either way."""
         lib = _lib.load()
         Bsz, L, dm, D, R, ndir = self.shape
         K, N = self.K, D_STATE
@@ -1397,8 +1431,9 @@ class NativeBlock:
         g.WiT, g.WxpT, g.WoT, g.WdT = _ptr(WiT), _ptr(WxpT), _ptr(WoT), _ptr(WdT)
         (g.dW_in, g.dconv_w, g.dconv_b, g.dW_x, g.dW_dt, g.db_dt, g.dA_log, g.dD, g.dW_out) = [_ptr(t) for t in grads]
         g.workspace, g.workspace_bytes = _ptr(ws), nbytes
-        _lib.check(lib.bimamba_block_bwd_varlen(C.byref(self.desc), C.byref(g), _ptr(self.seqlens), _stream()),
-                   "bimamba_block_bwd_varlen")
+        side = _side_stream(dev.index) if (SIDE_STREAM if two_stream is None else two_stream) else None
+        _lib.check(lib.bimamba_block_bwd_side(C.byref(self.desc), C.byref(g), _ptr(self.seqlens), _side_ptr(side),
+                                              _stream()), "bimamba_block_bwd_side")
         _lib.launch_count += 19          # 20 kernels: 4 + 4 x 2 GEMMs, scan, conv, row sum, 4 partial sums, layout pass
         self._keep = (dout, ws)
         return (dx, *grads)
@@ -1412,7 +1447,10 @@ class NativeLayer:
     """One forward call of the native encoder layer: descriptor, saved-activation workspace, packed Mamba weights."""
 
     def __init__(self, x, norm1_w, norm1_b, eps1, norm2_w, norm2_b, eps2, W1, b1, W2, b2, W_in, conv_w, conv_b, W_x, W_dt,
-                 b_dt, A_log, Dp, W_out, cdtype, save_for_backward=True, seqlens=None):
+                 b_dt, A_log, Dp, W_out, cdtype, save_for_backward=True, seqlens=None, two_stream=None):
+        """two_stream (default: SIDE_STREAM): the weight preparation of the forward and the parameter gradients of the
+        backward run on a second stream beside the data chain (bimamba_layer_fwd_side / bimamba_layer_bwd_side); False:
+        one stream.  The results are the same bits either way."""
         _require_cuda(x, norm1_w, W1, W_in)
         lib = _lib.load()
         Bsz, L, dm = x.shape
@@ -1420,8 +1458,14 @@ class NativeLayer:
         self.x = x.detach().contiguous()
         self.shape = (Bsz, L, dm, D, R, dff)
         self.cdtype = cdtype
-        self.packed = pack_weights(W_in.detach(), W_x.detach(), W_dt.detach(), A_log.detach(), W_out.detach(), 2, cdtype)
+        self.side = _side_stream(self.x.device.index) if (SIDE_STREAM if two_stream is None else two_stream) else None
+        # packed inside the forward call (on the side stream when there is one)
+        self.packed = _pack_buffers(W_in, A_log, 2, cdtype)
         Wi, WiT, Wxp, WxpT, Wo2, WoT, WdT, A32 = self.packed
+        masters = [_f32c(t.detach()) for t in (W_in, W_x, W_dt, A_log, W_out)]
+        pk = _lib.BlockPack()
+        pk.W_in, pk.W_x, pk.W_dt, pk.A_log, pk.W_out = [_ptr(t) for t in masters]
+        pk.Wi, pk.WiT, pk.Wxp, pk.WxpT, pk.Wo2, pk.WoT, pk.WdT, pk.A = [_ptr(t) for t in self.packed]
         self.f32 = tuple(_f32c(t) for t in (W_dt, conv_w, conv_b, Dp, b_dt, norm1_w, norm1_b, norm2_w, norm2_b, W1, b1, W2, b2))
         Wd32, cw32, cb32, D32, bdt32, n1w, n1b, n2w, n2b, W1f, b1f, W2f, b2f = self.f32
         cw32 = cw32.reshape(D, -1)
@@ -1442,11 +1486,11 @@ class NativeLayer:
         d.workspace, d.workspace_bytes = _ptr(self.ws), nbytes
         d.eps1, d.eps2, d.d_ff, d.x_dtype = float(eps1), float(eps2), dff, _dt(self.x)
         self.desc = d
-        self._keep_fwd = (cw32,)
+        self._keep_fwd = (cw32, masters)
         self.seqlens = seqlens
-        fwd = lib.bimamba_layer_fwd_varlen_train if save_for_backward else lib.bimamba_layer_fwd_varlen
-        _lib.check(fwd(C.byref(d), _ptr(seqlens), _stream()), "bimamba_layer_fwd_varlen")
-        _lib.launch_count += 11          # 12 kernels: 2 LayerNorm, 5 of the block, 2 weight casts, 2 GEMMs, GELU
+        _lib.check(lib.bimamba_layer_fwd_side(C.byref(d), C.byref(pk), _ptr(seqlens), _side_ptr(self.side), _stream()),
+                   "bimamba_layer_fwd_side")
+        _lib.launch_count += 12          # 13 kernels: the pack, 2 LayerNorm, 5 of the block, 2 weight casts, 2 GEMMs, GELU
 
     def backward(self, dout):
         """-> (dx, dnorm1 (2, dm), dnorm2 (2, dm), dW1, db1, dW2, db2, then the nine Mamba gradients in the order
@@ -1470,8 +1514,8 @@ class NativeLayer:
         kg.WiT, kg.WxpT, kg.WoT, kg.WdT = _ptr(WiT), _ptr(WxpT), _ptr(WoT), _ptr(WdT)
         (kg.dW_in, kg.dconv_w, kg.dconv_b, kg.dW_x, kg.dW_dt, kg.db_dt, kg.dA_log, kg.dD, kg.dW_out) = [_ptr(t) for t in mg]
         g.workspace, g.workspace_bytes = _ptr(ws), nbytes
-        _lib.check(lib.bimamba_layer_bwd_varlen(C.byref(self.desc), C.byref(g), _ptr(self.seqlens), _stream()),
-                   "bimamba_layer_bwd_varlen")
+        _lib.check(lib.bimamba_layer_bwd_side(C.byref(self.desc), C.byref(g), _ptr(self.seqlens), _side_ptr(self.side),
+                                              _stream()), "bimamba_layer_bwd_side")
         _lib.launch_count += 35          # 36 kernels: 20 of the block, 11 of the feed-forward, 2 x 2 of the norms, the cast of dout
         self._keep = (dout, ws)
         return (dx, *lg, *mg)
@@ -1507,8 +1551,8 @@ class EncoderLayerNativeFn(torch.autograd.Function):
 
 
 def native_layer_ok(x, layer) -> bool:
-    """Eager-mode fast path of the encoder layer: CUDA, no graph capture, a 16-bit compute dtype (autocast, or 16-bit x),
-    x in fp32 or that dtype, exact GELU, widths the kernels take."""
+    """Fast path of the encoder layer, eager and captured: CUDA, a 16-bit compute dtype (autocast, or 16-bit x), x in fp32
+    or that dtype, exact GELU, widths the kernels take."""
     if not (USE_NATIVE_BLOCK and _lib.kernel_timer is None and x.is_cuda and x.dim() == 3 and x.numel() > 0):
         return False
     cd = torch.get_autocast_dtype("cuda") if torch.is_autocast_enabled("cuda") else x.dtype
@@ -1521,8 +1565,10 @@ def native_layer_ok(x, layer) -> bool:
         return False
     dm = x.shape[-1]
     m = layer.mamba
+    # under capture only with the second stream: single-stream native calls would lose the parameter-gradient overlap
+    # the sequenced Functions have there
     return (dm % 8 == 0 and dm <= 1024 and ff[0].out_features % 8 == 0 and m.d_inner % 8 == 0 and m.d_state == D_STATE
-            and m.dt_rank <= MAX_DT_RANK and not torch.cuda.is_current_stream_capturing())
+            and m.dt_rank <= MAX_DT_RANK and (SIDE_STREAM or not torch.cuda.is_current_stream_capturing()))
 
 
 def encoder_layer_native(x, layer, seqlens=None, mask_padding=False):
