@@ -322,6 +322,59 @@ int bimamba_adamw_chunk(void);
 int bimamba_adamw_step(const struct bimamba_adamw_tensor* table, const int32_t* block_map, int nblocks,
                        const float* hyper, float* state, bimamba_stream_t stream);
 
+/* The optimizer step of the fp16 recipe (src/main.py:1100-1117) on the device, capturable:
+ *   scaler.unscale_ -> clip_grad_norm_(max_norm) -> scaler.step (skipped when a gradient is inf / NaN) -> scaler.update
+ *   -> ema.update_parameters
+ * over the tables bimamba_adamw_step reads.  Per optimizer step, on one stream:
+ *   1. bimamba_amp_grad_stats over ONE table and block map holding every group's tensors;
+ *   2. bimamba_adamw_amp_step once per parameter group (and once more, without hyper / state / amp, for parameters the
+ *      optimizer does not hold but the average covers);
+ *   3. bimamba_amp_update.
+ * The gradients stay scaled: the step reads (g * inv_scale) * clip_coef and writes no gradient back.
+ *
+ * The loss-scaling record (device memory, 4-byte aligned).  scale and growth_tracker are the state of
+ * torch.amp.GradScaler (its `_scale` and `_growth_tracker`); the other fields are written by bimamba_amp_grad_stats. */
+typedef struct bimamba_amp {
+  float scale;            /* loss scale S: the loss is multiplied by S before backward; the step unscales by
+                             inv_scale = (float)(1.0 / (double)S), as GradScaler.unscale_ does                       */
+  int32_t growth_tracker; /* applied steps since the scale last changed                                              */
+  float found_inf;        /* 1 when any gradient element is inf or NaN (the step is then skipped), else 0            */
+  float total_norm;       /* 2-norm of the unscaled gradient over every tensor (clip_grad_norm_'s return value),
+                             summed in fp64 in a fixed order; NaN or inf when found_inf                              */
+  float clip_coef;        /* min(1, max_norm / (total_norm + 1e-6)) in fp32, 1 without clipping                      */
+  int32_t reserved[3];    /* unused; pads the record to 32 bytes                                                     */
+} bimamba_amp;
+
+/* Averaged copy of one parameter (torch.optim.swa_utils.AveragedModel with get_ema_multi_avg_fn): entry i goes with
+ * entry i of the AdamW table.  n = the parameter's element count, also when it has no gradient (table n = 0);
+ * n = 0: the parameter has no average. */
+struct bimamba_ema_tensor {
+  float* avg;
+  int64_t n;
+};
+
+/* Step 1.  One CTA per block-map entry sums (g * inv_scale)^2 of its chunk into partials[i] (device, nblocks doubles,
+ * caller-owned; NaN marks a chunk with a non-finite gradient); one more CTA adds them in a fixed order and writes
+ * found_inf, total_norm and clip_coef.  max_norm <= 0: no clipping (clip_coef = 1).  Entries with n = 0 are skipped.
+ * Deterministic: the same gradients give the same bits. */
+int bimamba_amp_grad_stats(const struct bimamba_adamw_tensor* table, const int32_t* block_map, int nblocks,
+                           float max_norm, double* partials, bimamba_amp* amp, bimamba_stream_t stream);
+/* Step 2.  bimamba_adamw_step on the gradient (g * amp->inv_scale) * amp->clip_coef (two fp32 roundings in that order,
+ * the .grad unscale_ then clip_grad_norm_ leave); when amp->found_inf is set p, m, v and the step counter are left as
+ * they are.  hyper, state and amp are given together or all NULL (then only the averages move).
+ * ema != NULL (with n_averaged, the AveragedModel's device counter): afterwards every average moves toward its
+ * parameter, also on a skipped step - a copy while *n_averaged == 0, else torch's lerp with weight ema_weight
+ * (= 1 - decay, in [0, 1]): avg + w (p - avg) for w < 0.5, bit for bit as torch._foreach_lerp_. */
+int bimamba_adamw_amp_step(const struct bimamba_adamw_tensor* table, const int32_t* block_map, int nblocks,
+                           const float* hyper, float* state, const bimamba_amp* amp,
+                           const struct bimamba_ema_tensor* ema, const int64_t* n_averaged, float ema_weight,
+                           bimamba_stream_t stream);
+/* Step 3.  amp != NULL: torch._amp_update_scale_ - found_inf: scale *= backoff_factor, growth_tracker = 0; else
+ * growth_tracker + 1, and at growth_interval scale *= growth_factor (kept if finite) and growth_tracker = 0.
+ * n_averaged != NULL: *n_averaged += 1.  At least one of the two. */
+int bimamba_amp_update(bimamba_amp* amp, double growth_factor, double backoff_factor, int growth_interval,
+                       int64_t* n_averaged, bimamba_stream_t stream);
+
 /* Column sums of a (rows, cols) matrix with row stride ld (elements): the bias gradients of the Linear layers.
  * Writes fp32 partials part (nslices, cols), nslices = bimamba_colsum_slices(rows); finish with
  * bimamba_reduce_partials. */

@@ -3,6 +3,7 @@ backend uses).  Import name: this directory is `robust-audio-deepfake-evolution_
 the hyphens import it with `importlib.import_module("robust-audio-deepfake-evolution_b200")` or
 through the top-level alias module `bimamba_b200`."""
 from . import _lib
+from .amp import DeviceGradScaler, FusedEMA
 from .dist import FlatGradBucket, shard_batch
 from .encoder import BiMambaBackend, PN_BiMambas_Encoder, backend_head
 from .fusion import DualStreamFusion, SELayer
@@ -18,6 +19,7 @@ __all__ = [
     "bimamba_inner_fn", "causal_conv1d_fn", "selective_scan_fn", "install_mamba_ssm_shim",
     "DualStreamFusion", "SELayer", "FGM", "LoRALinear", "Phase6TrainStep", "apply_lora", "freeze_batch_norm_stats", "mixup_batch", "mixup_loss",
     "FlatGradBucket", "shard_batch", "GraphedForward", "GraphedTrainStep", "FusedAdamW",
+    "DeviceGradScaler", "FusedEMA",
 ]
 
 

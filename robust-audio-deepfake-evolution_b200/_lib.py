@@ -38,6 +38,7 @@ EXPORTS = (
     "bimamba_interp_frames_fwd", "bimamba_interp_frames_bwd", "bimamba_frame_mean", "bimamba_frame_mean_bwd",
     "bimamba_frame_scale", "bimamba_frame_scale_bwd_slices", "bimamba_frame_scale_bwd",
     "bimamba_block_bwd_side", "bimamba_layer_fwd_side", "bimamba_layer_bwd_side",
+    "bimamba_amp_grad_stats", "bimamba_adamw_amp_step", "bimamba_amp_update",
 )
 
 
@@ -103,6 +104,12 @@ class BlockPack(C.Structure):
     """Mirror of `struct bimamba_block_pack` (include/bimamba.h): the block's weight pack inside bimamba_layer_fwd_side."""
     _fields_ = [(n, C.c_void_p) for n in ("W_in", "W_x", "W_dt", "A_log", "W_out", "Wi", "WiT", "Wxp", "WxpT", "Wo2", "WoT",
                                           "WdT", "A")]
+
+
+class AmpRecord(C.Structure):
+    """Mirror of `struct bimamba_amp` (include/bimamba.h): the loss-scaling record of the fp16 optimizer step."""
+    _fields_ = [("scale", C.c_float), ("growth_tracker", C.c_int32), ("found_inf", C.c_float), ("total_norm", C.c_float),
+                ("clip_coef", C.c_float), ("reserved", C.c_int32 * 3)]
 
 
 _lib = None
@@ -183,6 +190,12 @@ def load() -> C.CDLL:
         lib.bimamba_adamw_chunk.argtypes = []
         lib.bimamba_adamw_step.restype = i32
         lib.bimamba_adamw_step.argtypes = [vp, vp, i32, vp, vp, vp]
+        lib.bimamba_amp_grad_stats.restype = i32
+        lib.bimamba_amp_grad_stats.argtypes = [vp, vp, i32, C.c_float, vp, vp, vp]
+        lib.bimamba_adamw_amp_step.restype = i32
+        lib.bimamba_adamw_amp_step.argtypes = [vp, vp, i32, vp, vp, vp, vp, vp, C.c_float, vp]
+        lib.bimamba_amp_update.restype = i32
+        lib.bimamba_amp_update.argtypes = [vp, C.c_double, C.c_double, i32, vp, vp]
         lib.bimamba_gemm_tn_splits.restype = i32
         lib.bimamba_gemm_tn_splits.argtypes = [i64, i32, i32]
         lib.bimamba_gemm_tn.restype = i32

@@ -7,6 +7,7 @@ from __future__ import annotations
 
 import contextlib
 import copy
+import inspect
 from typing import Callable, Optional
 
 import torch
@@ -59,12 +60,26 @@ class GraphedTrainStep:
     The `warmup` iterations before the capture run real optimizer steps on the example batch (lazy initialisation of
     handles, function attributes and optimizer state must happen outside the capture); with restore_after_warmup
     (default) the parameters and the optimizer state are put back afterwards, so building the runner - e.g. right
-    after loading a checkpoint - does not change the model, the moments, or the step count."""
+    after loading a checkpoint - does not change the model, the moments, or the step count (nor the scaler's scale
+    and growth tracker, the averaged parameters or n_averaged).
+
+    The fp16 recipe (src/main.py:1049-1117), with a FusedAdamW:
+      * scaler (DeviceGradScaler), max_norm, ema (FusedEMA): the loss is multiplied by the device scale before
+        backward and the captured step is optimizer.step(scaler=..., max_norm=..., ema=...) - unscale, clip, the skip
+        of an overflowing step, the scale update and the EMA, with no host read;
+      * accumulation_steps = k > 1: the loss is divided by k and two graphs are captured, a micro-step (forward and
+        backward, accumulating into the gradients) and the optimizer step ([post_backward ->] step -> zero_grad).
+        `run` replays the micro-step, and the optimizer step after every k-th call.  The gradients must be static
+        buffers zeroed in place by `zero_grad` (FlatGradBucket(accumulate=True).zero).
+    `run` returns step_fn's loss, unscaled and undivided.  post_backward (e.g. the multi-GPU all-reduce) runs before the
+    optimizer step, so the inf check and the norm see the global gradient; an inf or NaN survives the all-reduce, so
+    every rank skips the same steps."""
 
     def __init__(self, step_fn: Callable[[torch.Tensor], torch.Tensor], example: torch.Tensor,
                  zero_grad: Callable[[], None], optimizer: Optional[torch.optim.Optimizer] = None,
                  warmup: int = 3, post_backward: Optional[Callable[[], None]] = None,
-                 capture_error_mode: Optional[str] = None, restore_after_warmup: bool = True, lengths=None):
+                 capture_error_mode: Optional[str] = None, restore_after_warmup: bool = True, lengths=None,
+                 scaler=None, max_norm: Optional[float] = None, ema=None, accumulation_steps: int = 1):
         self.static_x = torch.empty_like(example, device="cuda")
         self.static_x.copy_(example)
         self.static_lengths = None
@@ -73,37 +88,91 @@ class GraphedTrainStep:
             self.static_lengths = seqlens_tensor(lengths, example.shape[0], example.shape[1], self.static_x.device).clone()
             args = (self.static_x, self.static_lengths)
         self.optimizer = optimizer
+        k = self.accumulation_steps = int(accumulation_steps)
+        if k < 1:
+            raise ValueError("accumulation_steps must be >= 1")
+        if scaler is not None and not scaler.is_enabled():
+            scaler = None
+        step_kw = {}
+        if scaler is not None or max_norm is not None or ema is not None:
+            if optimizer is None or "scaler" not in inspect.signature(optimizer.step).parameters:
+                raise TypeError("scaler / max_norm / ema need an optimizer whose step takes them (FusedAdamW)")
+            step_kw = dict(scaler=scaler, max_norm=max_norm, ema=ema)
+            if scaler is not None:
+                scaler._lazy_init(self.static_x.device)         # the record exists before the snapshot and the capture
+        if k > 1 and optimizer is None:
+            raise ValueError("accumulation_steps > 1 needs the optimizer")
+        self._micro = 0
         snap = _snapshot(optimizer) if (optimizer is not None and restore_after_warmup) else None
+        amp_snap = None
+        if restore_after_warmup:
+            amp_snap = (scaler._record.clone() if scaler is not None else None,
+                        ema.snapshot() if ema is not None else None)
+
+        def forward_backward():
+            loss = step_fn(*args)
+            scaled = loss / k if k > 1 else loss
+            if scaler is not None:
+                scaled = scaler.scale(scaled)
+            scaled.backward()
+            return loss
+
+        def apply():
+            if post_backward is not None:
+                post_backward()
+            if optimizer is not None:
+                optimizer.step(**step_kw)
+
         side = torch.cuda.Stream()
         side.wait_stream(torch.cuda.current_stream())
         with torch.cuda.stream(side), _as_captured():
             for _ in range(max(1, warmup)):          # lazy inits (cuBLAS handles, func attributes) happen here
                 zero_grad()
-                loss = step_fn(*args)
-                loss.backward()
-                if post_backward is not None:
-                    post_backward()
-                if optimizer is not None:
-                    optimizer.step()
+                forward_backward()
+                apply()
         torch.cuda.current_stream().wait_stream(side)
         torch.cuda.synchronize()
         if snap is not None:
             _restore(optimizer, snap)
-            torch.cuda.synchronize()
+        if amp_snap is not None:
+            if amp_snap[0] is not None:
+                scaler._record.copy_(amp_snap[0])
+            if amp_snap[1] is not None:
+                ema.restore(amp_snap[1])
+        torch.cuda.synchronize()
         self.graph = torch.cuda.CUDAGraph()
+        self.apply_graph = None
         if capture_error_mode is None:
             # a process group's watchdog thread issues CUDA calls of its own: with NCCL collectives inside the capture
             # only this thread's calls may invalidate it
             import torch.distributed as dist
             capture_error_mode = "thread_local" if dist.is_available() and dist.is_initialized() else "global"
+        if k == 1:
+            with torch.cuda.graph(self.graph, capture_error_mode=capture_error_mode):
+                zero_grad()
+                self.static_loss = forward_backward()
+                apply()
+            return
+        zero_grad()
+        params = [p for g in optimizer.param_groups for p in g["params"] if p.requires_grad]
+        if any(p.grad is None for p in params):
+            raise ValueError("accumulation_steps > 1 accumulates into static gradient buffers: zero_grad must zero "
+                             "them in place (e.g. FlatGradBucket(accumulate=True).zero), not set them to None")
+        torch.cuda.synchronize()
         with torch.cuda.graph(self.graph, capture_error_mode=capture_error_mode):
+            self.static_loss = forward_backward()
+        self.apply_graph = torch.cuda.CUDAGraph()
+        with torch.cuda.graph(self.apply_graph, pool=self.graph.pool(), capture_error_mode=capture_error_mode):
+            apply()
             zero_grad()
-            self.static_loss = step_fn(*args)
-            self.static_loss.backward()
-            if post_backward is not None:
-                post_backward()
-            if optimizer is not None:
-                optimizer.step()
+
+    def _replay(self):
+        self.graph.replay()
+        if self.apply_graph is not None:
+            self._micro += 1
+            if self._micro == self.accumulation_steps:
+                self.apply_graph.replay()
+                self._micro = 0
 
     def run(self, x: Optional[torch.Tensor] = None, lengths=None) -> torch.Tensor:
         if x is not None:
@@ -113,7 +182,7 @@ class GraphedTrainStep:
                 raise ValueError("this step was captured without lengths")
             B, T = self.static_x.shape[:2]
             self.static_lengths.copy_(seqlens_tensor(lengths, B, T, self.static_x.device), non_blocking=True)
-        self.graph.replay()
+        self._replay()
         return self.static_loss
 
     def run_pipelined(self, host_batches):
@@ -147,7 +216,7 @@ class GraphedTrainStep:
                         copy.wait_event(self._consumed[1 - cur])
                     self._stage[1 - cur].copy_(nxt, non_blocking=True)
                     self._ready[1 - cur].record(copy)
-            self.graph.replay()
+            self._replay()
             yield float(self.static_loss.detach())
             idx += 1
 

@@ -160,7 +160,11 @@ class Phase6TrainStep:
 
     model(x) must return (features, logits) like the reference Model.forward.  `loss_fn(logits, feats, target)`.
     bucket: a FlatGradBucket(accumulate=True) over the trainable parameters when running data-parallel (its views ARE
-    the .grad tensors, so both backward passes of FGM and every micro-batch accumulate into it), else None."""
+    the .grad tensors, so both backward passes of FGM and every micro-batch accumulate into it), else None.
+
+    With a DeviceGradScaler and a FusedAdamW the tail is one FusedAdamW.step(scaler=, max_norm=, ema=) on the device,
+    with no host read in the step; ema_model is then a FusedEMA (the AveragedModel paired with the model) or None.
+    With torch's GradScaler the tail is torch's calls above."""
 
     def __init__(self, model: nn.Module, optimizer: torch.optim.Optimizer, loss_fn: Callable, *,
                  scaler: Optional[torch.amp.GradScaler] = None, autocast_dtype: Optional[torch.dtype] = torch.float16,
@@ -174,6 +178,14 @@ class Phase6TrainStep:
         self.max_norm, self.ema_model, self.scheduler, self.bucket = max_norm, ema_model, scheduler, bucket
         self.freeze_bn = freeze_bn
         self.model_kwargs = model_kwargs or {}
+        from .amp import DeviceGradScaler, FusedEMA
+        from .optim import FusedAdamW
+        self.fused = isinstance(self.scaler, DeviceGradScaler)
+        if self.fused:
+            if not isinstance(optimizer, FusedAdamW):
+                raise TypeError("a DeviceGradScaler unscales inside FusedAdamW.step: the optimizer must be a FusedAdamW")
+            if ema_model is not None and not isinstance(ema_model, FusedEMA):
+                raise TypeError("with a DeviceGradScaler, pass the AveragedModel as FusedEMA(averaged, model, decay)")
         self._zero()
 
     def _zero(self):
@@ -209,6 +221,12 @@ class Phase6TrainStep:
             total = loss.detach() if total is None else total + loss.detach()
         if self.bucket is not None:
             self.bucket.all_reduce_mean()                                             # global gradient before the clip
+        if self.fused:                                                                # main.py:1103-1113 on the device
+            self.optimizer.step(scaler=self.scaler, max_norm=self.max_norm, ema=self.ema_model)
+            self._zero()
+            if self.scheduler is not None:
+                self.scheduler.step()
+            return total
         self.scaler.unscale_(self.optimizer)                                          # main.py:1103
         params = [p for g in self.optimizer.param_groups for p in g["params"] if p.grad is not None]
         torch.nn.utils.clip_grad_norm_(params, max_norm=self.max_norm)                # main.py:1104
