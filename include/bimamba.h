@@ -32,6 +32,7 @@
  *                                       (per-utterance frame counts; see "Variable-length scoring" below)
  *   bimamba_*_varlen_train, *_bwd_varlen, bimamba_mask_frames
  *                                    <- training on such batches (see "Variable-length training" below)
+ *   bimamba_mixup_frames             <- Mixup of the training loop (src/main.py:1038-1046), fixed or variable length
  *
  * Ownership: the library never allocates or frees device memory.  All tensors and
  * workspaces are caller-allocated; pointers are borrowed for the duration of the
@@ -179,6 +180,17 @@ int bimamba_selective_scan_bwd_varlen(const bimamba_scan_desc* d, const int32_t*
  * (and, for the layer, the output after the forward: its feed-forward and residual make padded output rows non-zero). */
 int bimamba_mask_frames(const void* x, void* out, const int32_t* seqlens, int batch, int seqlen, int channels, int dtype,
                         bimamba_stream_t stream);
+
+/* Mixup of a right-padded batch (src/main.py:1038-1046), one launch.  x and out (batch, seqlen, channels) contiguous in
+ * `dtype`, out not x (rows read other rows); perm: device int32 (batch,) permutation p (values clamped to [0, batch));
+ * mix: device fp32 {lam, 1 - lam}, both formed in double on the host and rounded to fp32.  Each product is rounded to
+ * `dtype`, then their sum: out[b, t] = rn(rn(lam x[b, t]) + rn((1 - lam) x[p(b), t])), the bits of torch's
+ * `lam * x + (1.0 - lam) * x[perm]`.  seqlens_in (device int32, clamped to [0, seqlen]) or NULL = every frame valid: a
+ * term is taken only over its own utterance's frames (by selection, so padding is never read), out is exactly zero at
+ * t >= max(n_b, n_p(b)), and that mixed length goes to seqlens_out (required with seqlens_in, ignored without it).
+ * NULL operand -1, bad sizes / dtype -3, empty batch a no-op 0. */
+int bimamba_mixup_frames(const void* x, void* out, const int32_t* perm, const float* mix, const int32_t* seqlens_in,
+                         int32_t* seqlens_out, int batch, int seqlen, int channels, int dtype, bimamba_stream_t stream);
 
 /* ---- Variable-length DualStreamFusion (DualStreamSEMamba.py:580-637 run on each utterance alone).  Two streams, two
  * length vectors: seqlens_dst (batch) are the WavLM frame counts n1 of a batch padded to dst_frames, seqlens_src the

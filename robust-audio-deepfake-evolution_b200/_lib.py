@@ -39,6 +39,7 @@ EXPORTS = (
     "bimamba_frame_scale", "bimamba_frame_scale_bwd_slices", "bimamba_frame_scale_bwd",
     "bimamba_block_bwd_side", "bimamba_layer_fwd_side", "bimamba_layer_bwd_side",
     "bimamba_amp_grad_stats", "bimamba_adamw_amp_step", "bimamba_amp_update",
+    "bimamba_mixup_frames",
 )
 
 
@@ -281,6 +282,8 @@ def load() -> C.CDLL:
         lib.bimamba_layer_bwd_side.argtypes = [C.POINTER(LayerDesc), C.POINTER(LayerGrads), vp, C.POINTER(SideStream), vp]
         lib.bimamba_mask_frames.restype = i32
         lib.bimamba_mask_frames.argtypes = [vp, vp, vp, i32, i32, i32, i32, vp]
+        lib.bimamba_mixup_frames.restype = i32
+        lib.bimamba_mixup_frames.argtypes = [vp, vp, vp, vp, vp, vp, i32, i32, i32, i32, vp]
         for name in ("bimamba_interp_frames_fwd", "bimamba_interp_frames_bwd"):
             fn = getattr(lib, name)
             fn.restype = i32

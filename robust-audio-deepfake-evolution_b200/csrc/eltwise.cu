@@ -227,6 +227,47 @@ __global__ void __launch_bounds__(256) mask_frames_kernel(const T* x, T* out, co
   }
 }
 
+// Mixup of a right-padded batch: out[b, t] = rn(rn(lam * x[b, t]) + rn((1 - lam) * x[p, t])), p = perm[b], with each
+// product rounded to T as torch rounds `lam * x + (1.0 - lam) * x[perm]` (explicit _rn: no contraction into an FMA).
+// With seqlens each source adds only over its own frames (selection, so NaN padding is never read) and the mixed length
+// max(n_b, n_p) goes to seqlens_out; frames past it are zero.  perm values are clamped to [0, batch).
+template <typename T, bool kVec>
+__global__ void __launch_bounds__(256) mixup_frames_kernel(const T* __restrict__ x, T* __restrict__ out,
+                                                           const int32_t* __restrict__ perm, const float* __restrict__ mix,
+                                                           const int32_t* __restrict__ seqlens, int32_t* __restrict__ seqlens_out,
+                                                           int batch, int T_, int64_t C, int64_t n) {
+  pdl_prologue();
+  constexpr int kV = kVec ? 16 / sizeof(T) : 1;
+  const float lam = __ldg(mix), lam1 = __ldg(mix + 1);
+  auto len = [&](int b) { return seqlens ? min(max(__ldg(seqlens + b), 0), T_) : T_; };
+  if (seqlens_out && blockIdx.x == 0)
+    for (int b = threadIdx.x; b < batch; b += blockDim.x) seqlens_out[b] = max(len(b), len(min(max(__ldg(perm + b), 0), batch - 1)));
+  const int64_t nv = n / kV, cv = C / kV;
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < nv; i += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t row = i / cv, col = i - row * cv;
+    const int b = (int)(row / T_), t = (int)(row - (int64_t)b * T_);
+    const int p = min(max(__ldg(perm + b), 0), batch - 1);
+    const bool in_b = t < len(b), in_p = t < len(p);
+    T xb[kV], xp[kV], o[kV];
+    const int64_t jb = i, jp = ((int64_t)p * T_ + t) * cv + col;
+    if constexpr (kVec) {
+      *reinterpret_cast<uint4*>(xb) = in_b ? __ldg(reinterpret_cast<const uint4*>(x) + jb) : make_uint4(0u, 0u, 0u, 0u);
+      *reinterpret_cast<uint4*>(xp) = in_p ? __ldg(reinterpret_cast<const uint4*>(x) + jp) : make_uint4(0u, 0u, 0u, 0u);
+    } else {
+      xb[0] = in_b ? x[jb] : from_f<T>(0.f);
+      xp[0] = in_p ? x[jp] : from_f<T>(0.f);
+    }
+#pragma unroll
+    for (int k = 0; k < kV; ++k) {
+      const float a = in_b ? to_f(from_f<T>(__fmul_rn(lam, to_f(xb[k])))) : 0.f;
+      const float c = in_p ? to_f(from_f<T>(__fmul_rn(lam1, to_f(xp[k])))) : 0.f;
+      o[k] = from_f<T>(__fadd_rn(a, c));
+    }
+    if constexpr (kVec) *(reinterpret_cast<uint4*>(out) + i) = *reinterpret_cast<const uint4*>(o);
+    else out[i] = o[0];
+  }
+}
+
 }  // namespace bimamba
 
 using namespace bimamba;
@@ -390,6 +431,27 @@ extern "C" int bimamba_mask_frames(const void* x, void* out, const int32_t* seql
   const bool vec = channels % kV == 0 && aligned16(x) && aligned16(out);
   if (vec) EW_DISPATCH1(dtype, (launch_k(mask_frames_kernel<T, true>, ew_blocks(n / kV, 256), 256, 0, st, (const T*)x, (T*)out, seqlens, seqlen, (int64_t)channels, n)));
   else EW_DISPATCH1(dtype, (launch_k(mask_frames_kernel<T, false>, ew_blocks(n, 256), 256, 0, st, (const T*)x, (T*)out, seqlens, seqlen, (int64_t)channels, n)));
+  cudaError_t e = cudaGetLastError();
+  if (e != cudaSuccess) { set_err(cudaGetErrorString(e)); return (int)e; }
+  return 0;
+}
+
+extern "C" int bimamba_mixup_frames(const void* x, void* out, const int32_t* perm, const float* mix, const int32_t* seqlens_in,
+                                    int32_t* seqlens_out, int batch, int seqlen, int channels, int dtype,
+                                    bimamba_stream_t stream) {
+  if (batch < 0 || seqlen < 0 || channels < 0 || dtype < 0 || dtype > 2) { set_err("mixup_frames: bad sizes"); return -3; }
+  if (batch == 0) return 0;
+  if (!perm || !mix || (seqlens_in && !seqlens_out)) { set_err("mixup_frames: null operand"); return -1; }
+  const int64_t n = (int64_t)batch * seqlen * channels;
+  if (n && (!x || !out)) { set_err("mixup_frames: null operand"); return -1; }
+  if (n == 0 && !seqlens_in) return 0;
+  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+  const int kV = dtype == BIMAMBA_F32 ? 4 : 8;
+  const bool vec = channels % kV == 0 && aligned16(x) && aligned16(out);
+  const int32_t* sl = seqlens_in;
+  int32_t* so = seqlens_in ? seqlens_out : nullptr;
+  if (vec) EW_DISPATCH1(dtype, (launch_k(mixup_frames_kernel<T, true>, ew_blocks(n / kV, 256), 256, 0, st, (const T*)x, (T*)out, perm, mix, sl, so, batch, seqlen, (int64_t)channels, n)));
+  else EW_DISPATCH1(dtype, (launch_k(mixup_frames_kernel<T, false>, ew_blocks(n, 256), 256, 0, st, (const T*)x, (T*)out, perm, mix, sl, so, batch, seqlen, (int64_t)channels, n)));
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) { set_err(cudaGetErrorString(e)); return (int)e; }
   return 0;

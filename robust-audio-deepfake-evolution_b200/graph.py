@@ -73,13 +73,25 @@ class GraphedTrainStep:
         buffers zeroed in place by `zero_grad` (FlatGradBucket(accumulate=True).zero).
     `run` returns step_fn's loss, unscaled and undivided.  post_backward (e.g. the multi-GPU all-reduce) runs before the
     optimizer step, so the inf check and the norm see the global gradient; an inf or NaN survives the all-reduce, so
-    every rank skips the same steps."""
+    every rank skips the same steps.
+
+    Labels and Mixup (src/main.py:1038-1046, :1070-1073):
+      * labels (an example (B,) label vector) gives a static label buffer, and step_fn is then called as
+        step_fn(x, y, lengths, mix) - lengths the static frame counts or None, mix a training.MixState or None;
+      * mixup_alpha > 0 (needs labels) gives static perm and mix buffers: every `run` (every micro-step) draws lam ~
+        Beta(alpha, alpha) and a permutation on the host (training.draw_mixup, perm on `generator`), and copies them in
+        one 8 + 4B-byte copy, without a device sync, so each replay mixes with its own draw.  step_fn mixes with
+        training.mixup_batch(x, y, lam=mix.mix, lengths=lengths, index=mix.perm) and weights its loss with
+        training.mixup_loss(..., lam=mix.mix).  `last_lam` holds the last draw's lam.
+    run(x, lengths, y=y) copies whichever of them is given."""
 
     def __init__(self, step_fn: Callable[[torch.Tensor], torch.Tensor], example: torch.Tensor,
                  zero_grad: Callable[[], None], optimizer: Optional[torch.optim.Optimizer] = None,
                  warmup: int = 3, post_backward: Optional[Callable[[], None]] = None,
                  capture_error_mode: Optional[str] = None, restore_after_warmup: bool = True, lengths=None,
-                 scaler=None, max_norm: Optional[float] = None, ema=None, accumulation_steps: int = 1):
+                 scaler=None, max_norm: Optional[float] = None, ema=None, accumulation_steps: int = 1,
+                 labels: Optional[torch.Tensor] = None, mixup_alpha: float = 0.0,
+                 generator: Optional[torch.Generator] = None):
         self.static_x = torch.empty_like(example, device="cuda")
         self.static_x.copy_(example)
         self.static_lengths = None
@@ -87,6 +99,23 @@ class GraphedTrainStep:
         if lengths is not None:
             self.static_lengths = seqlens_tensor(lengths, example.shape[0], example.shape[1], self.static_x.device).clone()
             args = (self.static_x, self.static_lengths)
+        self.static_y = self.mix = None
+        self.mixup_alpha, self.generator, self.last_lam = float(mixup_alpha), generator, None
+        if self.mixup_alpha > 0 and labels is None:
+            raise ValueError("mixup_alpha needs labels (the mixed batch is scored against both label sets)")
+        if labels is not None:
+            self.static_y = labels.to("cuda").view(-1).long().clone()
+            if self.static_y.numel() != example.shape[0]:
+                raise ValueError(f"labels must hold {example.shape[0]} entries, got {self.static_y.numel()}")
+            if self.mixup_alpha > 0:
+                # one buffer, one copy per run: [lam, 1 - lam] as fp32 bits, then the permutation; until the first run
+                # the identity at lam = 1 (the warm-up and the capture see a valid draw)
+                B = example.shape[0]
+                self._draw = torch.empty(B + 2, dtype=torch.int32, device=self.static_x.device)
+                self._draw.copy_(self._draw_host(1.0, torch.arange(B)))
+                from .training import MixState
+                self.mix = MixState(self._draw[2:], self._draw[:2].view(torch.float32))
+            args = (self.static_x, self.static_y, self.static_lengths, self.mix)
         self.optimizer = optimizer
         k = self.accumulation_steps = int(accumulation_steps)
         if k < 1:
@@ -174,48 +203,91 @@ class GraphedTrainStep:
                 self.apply_graph.replay()
                 self._micro = 0
 
-    def run(self, x: Optional[torch.Tensor] = None, lengths=None) -> torch.Tensor:
-        if x is not None:
-            self.static_x.copy_(x, non_blocking=True)
+    @staticmethod
+    def _draw_host(lam: float, perm: torch.Tensor) -> torch.Tensor:
+        """The host image of the draw buffer: [lam, 1 - lam] (fp32, 1 - lam taken in double) | perm (int32)."""
+        mix = torch.tensor([lam, 1.0 - lam], dtype=torch.float32).view(torch.int32)
+        return torch.cat([mix, perm.to(torch.int32)])
+
+    def _load(self, y=None, lengths=None):
+        """Copy the labels and lengths given, and a fresh Mixup draw, into the static buffers (no device sync)."""
+        if y is not None:
+            if self.static_y is None:
+                raise ValueError("this step was captured without labels")
+            self.static_y.copy_(y.view(-1), non_blocking=True)
         if lengths is not None:
             if self.static_lengths is None:
                 raise ValueError("this step was captured without lengths")
             B, T = self.static_x.shape[:2]
             self.static_lengths.copy_(seqlens_tensor(lengths, B, T, self.static_x.device), non_blocking=True)
+        if self.mix is not None:
+            from .training import draw_mixup
+            self.last_lam, perm = draw_mixup(self.static_x.shape[0], self.mixup_alpha, self.generator)
+            self._draw.copy_(self._draw_host(self.last_lam, perm), non_blocking=True)
+
+    def run(self, x: Optional[torch.Tensor] = None, lengths=None, *, y: Optional[torch.Tensor] = None) -> torch.Tensor:
+        if x is not None:
+            self.static_x.copy_(x, non_blocking=True)
+        self._load(y, lengths)
         self._replay()
         return self.static_loss
 
+    def _host_parts(self, batch):
+        """A host batch x or (x, y[, lengths]) -> its tensors in the order of self._statics (lengths as int32)."""
+        if isinstance(batch, torch.Tensor):
+            return [batch]
+        parts = [batch[0]]
+        if len(batch) > 1 and batch[1] is not None:
+            if self.static_y is None:
+                raise ValueError("this step was captured without labels")
+            parts.append(batch[1].view(-1))
+        if len(batch) > 2 and batch[2] is not None:
+            if self.static_lengths is None or len(parts) < 2:
+                raise ValueError("lengths in a pipelined batch need a step captured with labels and lengths")
+            parts.append(seqlens_tensor(batch[2], *self.static_x.shape[:2], "cpu"))
+        return parts
+
     def run_pipelined(self, host_batches):
-        """Generator over pinned host batches: yields float(loss) of every step (a device->host read per step, like
-        src/main.py:1123).  The host->device copy of batch i+1 runs on a copy stream while step i replays (double
-        buffered staging + one device-to-device copy into the graph's static input), which is what a data loader
-        with pinned memory does for the reference loop."""
+        """Generator over pinned host batches, each x or (x, y[, lengths]): yields float(loss) of every step (a
+        device->host read per step, like src/main.py:1123).  The host->device copy of batch i+1 runs on a copy stream
+        while step i replays (double buffered staging + one device-to-device copy per tensor into the graph's static
+        buffers), which is what a data loader with pinned memory does for the reference loop.  A Mixup draw is made
+        for every step, as in run()."""
+        statics = [t for t in (self.static_x, self.static_y, self.static_lengths) if t is not None]
         if not hasattr(self, "_copy_stream"):
             self._copy_stream = torch.cuda.Stream()
-            self._stage = [torch.empty_like(self.static_x) for _ in range(2)]
+            self._stage = [[torch.empty_like(t) for t in statics] for _ in range(2)]
             self._ready = [torch.cuda.Event() for _ in range(2)]
             self._consumed = [torch.cuda.Event() for _ in range(2)]
         copy, main = self._copy_stream, torch.cuda.current_stream()
         it = iter(host_batches)
         nxt = next(it, None)
+        count = [0, 0]
+
+        def stage(slot, batch):
+            parts = self._host_parts(batch)
+            for buf, part in zip(self._stage[slot], parts):
+                buf.copy_(part, non_blocking=True)
+            count[slot] = len(parts)
+            self._ready[slot].record(copy)
         if nxt is not None:
             copy.wait_stream(main)
             with torch.cuda.stream(copy):
-                self._stage[0].copy_(nxt, non_blocking=True)
-                self._ready[0].record(copy)
+                stage(0, nxt)
         idx = 0
         while nxt is not None:
             cur = idx & 1
             main.wait_event(self._ready[cur])
-            self.static_x.copy_(self._stage[cur], non_blocking=True)
+            for dst, buf in zip(statics[:count[cur]], self._stage[cur]):
+                dst.copy_(buf, non_blocking=True)
             self._consumed[cur].record(main)
             nxt = next(it, None)
             if nxt is not None:
                 with torch.cuda.stream(copy):
                     if idx > 0:
                         copy.wait_event(self._consumed[1 - cur])
-                    self._stage[1 - cur].copy_(nxt, non_blocking=True)
-                    self._ready[1 - cur].record(copy)
+                    stage(1 - cur, nxt)
+            self._load()
             self._replay()
             yield float(self.static_loss.detach())
             idx += 1

@@ -218,6 +218,38 @@ def mask_frames(x: torch.Tensor, seqlens: torch.Tensor) -> torch.Tensor:
     return MaskFramesFn.apply(x, seqlens)
 
 
+def mixup_frames(x: torch.Tensor, perm: torch.Tensor, mix: torch.Tensor, seqlens: Optional[torch.Tensor] = None,
+                 out: Optional[torch.Tensor] = None):
+    """Mixup of a right-padded batch x (B, T) or (B, T, C), one launch of bimamba_mixup_frames -> (mixed, mixed
+    seqlens or None).  perm: (B,) int32 CUDA permutation; mix: (2,) fp32 CUDA (lam, 1 - lam), each rounded from the
+    host's double.  Without seqlens the bits of `lam * x + (1.0 - lam) * x[perm]`; with seqlens (seqlens_tensor) each
+    term only over its own utterance's frames and the mixed length max(n_b, n_perm[b]).  Capture-safe: lam and perm
+    are read on the device.  `out`: a contiguous tensor like x (not x itself) to write into.  Data only (the input of
+    a training step): x must not require a gradient."""
+    _require_cuda(x, perm, mix)
+    if _wants_grad(x):
+        raise NotImplementedError("mixup_frames mixes the input batch and has no backward: x must not require grad")
+    if perm.dtype != torch.int32 or mix.dtype != torch.float32 or tuple(mix.shape) != (2,):
+        raise TypeError("perm must be int32 and mix a (2,) float32 tensor (lam, 1 - lam)")
+    lib = _lib.load()
+    x = x.detach()
+    x = x if x.is_contiguous() else x.contiguous()
+    Bsz, T = x.shape[0], x.shape[1]
+    C_ = x.shape[2:].numel()
+    if tuple(perm.shape) != (Bsz,):
+        raise ValueError(f"perm must have shape ({Bsz},), got {tuple(perm.shape)}")
+    if out is None:
+        out = torch.empty_like(x)
+    elif out.shape != x.shape or out.dtype != x.dtype or not out.is_contiguous() or out.data_ptr() == x.data_ptr():
+        raise ValueError("out must be a contiguous tensor of x's shape and dtype, other than x")
+    sl_out = None if seqlens is None else torch.empty(Bsz, dtype=torch.int32, device=x.device)
+    with _timed("mixup"):
+        _lib.check(lib.bimamba_mixup_frames(_ptr(x), _ptr(out), _ptr(perm.contiguous()), _ptr(mix.contiguous()),
+                                            _ptr(seqlens), _ptr(sl_out), Bsz, T, C_, _dt(x), _stream()),
+                   "bimamba_mixup_frames")
+    return out, sl_out
+
+
 # ----------------------------------------------------------------------------------------
 # variable-length DualStreamFusion (DualStreamSEMamba.py:601-628 per utterance): interpolation of the projected SincNet
 # branch onto each utterance's WavLM frames, SELayer's masked mean and channel scale.  One launch each way.

@@ -13,7 +13,7 @@ side of it.  Differences from the reference loop, all deliberate:
 from __future__ import annotations
 
 import math
-from typing import Callable, Iterable, Optional, Sequence
+from typing import Callable, Iterable, NamedTuple, Optional, Sequence
 
 import torch
 import torch.nn as nn
@@ -61,21 +61,81 @@ class FGM:
 # ----------------------------------------------------------------------------------------------------------------------
 # Mixup (src/main.py:1038-1046, :1070-1075)
 # ----------------------------------------------------------------------------------------------------------------------
+class MixState(NamedTuple):
+    """The device side of one Mixup draw, as the kernel reads it: perm (B,) int32 and mix (2,) fp32 = (lam, 1 - lam),
+    both weights formed in double on the host and rounded to fp32 (as torch rounds a Python scalar for an fp32/16-bit
+    tensor).  A captured step reads them from static buffers, so every replay mixes with that replay's draw."""
+    perm: torch.Tensor
+    mix: torch.Tensor
+
+
+def mix_record(lam: float, device) -> torch.Tensor:
+    """(2,) fp32 (lam, 1 - lam) on `device`: 1 - lam is taken in double before the rounding, as `(1.0 - lam) * x`."""
+    return torch.tensor([lam, 1.0 - lam], dtype=torch.float32).to(device, non_blocking=True)
+
+
+def draw_mixup(batch: int, alpha: float, generator: Optional[torch.Generator] = None):
+    """The host draw of one Mixup step, in mixup_batch's order -> (lam, permutation as a CPU int64 tensor): lam ~
+    Beta(alpha, alpha) from torch's global generator, then torch.randperm(batch) on `generator` (a CPU generator, or
+    torch's global one)."""
+    lam = float(torch.distributions.Beta(alpha, alpha).sample())
+    return lam, torch.randperm(batch, generator=generator)
+
+
+def _mix_cpu(x, index, lam, lengths):
+    """The CPU form of the kernel's contract (the CPU tests' stand-ins): the same three roundings, by selection."""
+    n = torch.as_tensor(lengths, device=x.device).long().clamp(0, x.size(1))
+    t = torch.arange(x.size(1), device=x.device).view(1, -1, *([1] * (x.dim() - 2)))
+    keep_a, keep_b = t < n.view(-1, *([1] * (x.dim() - 1))), t < n[index].view(-1, *([1] * (x.dim() - 1)))
+    a = torch.where(keep_a, lam * x, torch.zeros((), dtype=x.dtype))
+    c = torch.where(keep_b, (1.0 - lam) * x[index], torch.zeros((), dtype=x.dtype))
+    return a + c, torch.maximum(n, n[index])
+
+
 def mixup_batch(x: torch.Tensor, y: torch.Tensor, alpha: float = 1.0, generator: Optional[torch.Generator] = None,
-                lam: Optional[float] = None):
-    """-> (mixed_x, y_a, y_b, lam): lam ~ Beta(alpha, alpha), one permutation of the batch.  Batches of one sample are
-    returned unchanged with lam = 1 (main.py:1038, :1043-1046)."""
-    if x.size(0) <= 1 or alpha <= 0:
-        return x, y, y, 1.0
+                lam=None, lengths=None, *, index: Optional[torch.Tensor] = None):
+    """-> (mixed_x, y_a, y_b, lam), and with `lengths` (mixed_x, y_a, y_b, lam, mixed_lengths): lam ~ Beta(alpha,
+    alpha) and one permutation of the batch, drawn on the host unless given (`lam`, `index`).  Batches of one sample
+    are returned unchanged with lam = 1 (main.py:1038, :1043-1046).
+
+    CUDA tensors are mixed by one bimamba_mixup_frames launch: without lengths the bits of `lam * x + (1.0 - lam) *
+    x[index]`; with lengths (per-utterance frame counts of the right-padded batch x, as ops.seqlens_tensor takes them)
+    each clip adds only over its own frames, zero-padded, and mixed utterance b has max(n_b, n_index[b]) frames
+    (returned as a (B,) int32 tensor on x's device).  The capture-safe form passes lam as the (2,) device record of
+    mix_record and index as a device int32 tensor (a MixState's fields): nothing is read or drawn on the host, and the
+    returned lam is that record, which mixup_loss takes."""
+    B = x.size(0)
+    if B <= 1 or alpha <= 0:
+        return (x, y, y, 1.0) if lengths is None else (x, y, y, 1.0, lengths)
     if lam is None:
         lam = float(torch.distributions.Beta(alpha, alpha).sample())
-    index = torch.randperm(x.size(0), generator=generator, device=x.device if generator is None else generator.device)
-    index = index.to(x.device)
-    return lam * x + (1.0 - lam) * x[index], y, y[index], lam
+    if index is None:
+        index = torch.randperm(B, generator=generator, device=x.device if generator is None else generator.device)
+    device_lam = isinstance(lam, torch.Tensor)
+    if not x.is_cuda:
+        if device_lam:
+            raise ValueError("a device lam record needs CUDA tensors")
+        index = index.to(x.device)
+        if lengths is None:
+            return lam * x + (1.0 - lam) * x[index], y, y[index], lam
+        mx, ml = _mix_cpu(x, index, lam, lengths)
+        return mx, y, y[index], lam, ml
+    from .ops import mixup_frames, seqlens_tensor
+    perm = index.to(device=x.device, dtype=torch.int32)
+    mix = lam if device_lam else mix_record(lam, x.device)
+    sl = None if lengths is None else seqlens_tensor(lengths, B, x.size(1), x.device)
+    mx, ml = mixup_frames(x, perm, mix, sl)
+    y_b = y[perm]
+    return (mx, y, y_b, lam) if lengths is None else (mx, y, y_b, lam, ml)
 
 
-def mixup_loss(loss_fn: Callable, out, feats, y_a, y_b, lam: float):
-    """lam * L(out, y_a) + (1 - lam) * L(out, y_b) (main.py:1070-1073)."""
+def mixup_loss(loss_fn: Callable, out, feats, y_a, y_b, lam):
+    """lam * L(out, y_a) + (1 - lam) * L(out, y_b) (main.py:1070-1073).  lam: a float; a 0-d device tensor (1 - lam is
+    then taken on the device); or the (2,) record (lam, 1 - lam) of mix_record, whose weights give the bits of the
+    float form, so a captured step with a device draw computes what the eager step computes with the host's float."""
+    if isinstance(lam, torch.Tensor):
+        w_a, w_b = (lam[0], lam[1]) if lam.dim() == 1 else (lam, 1.0 - lam)
+        return w_a * loss_fn(out, feats, y_a) + w_b * loss_fn(out, feats, y_b)
     if lam == 1.0:
         return loss_fn(out, feats, y_a)
     return lam * loss_fn(out, feats, y_a) + (1.0 - lam) * loss_fn(out, feats, y_b)
@@ -158,7 +218,8 @@ class Phase6TrainStep:
         [all-reduce the flat gradient bucket over ranks]  -> scaler.unscale_ -> clip_grad_norm_(3.0) -> scaler.step
         -> scaler.update -> zero grads -> [EMA update] -> [scheduler.step]
 
-    model(x) must return (features, logits) like the reference Model.forward.  `loss_fn(logits, feats, target)`.
+    model(x) must return (features, logits) like the reference Model.forward, and model(x, lengths, mask_padding=True)
+    too when micro-batches carry lengths.  `loss_fn(logits, feats, target)`.
     bucket: a FlatGradBucket(accumulate=True) over the trainable parameters when running data-parallel (its views ARE
     the .grad tensors, so both backward passes of FGM and every micro-batch accumulate into it), else None.
 
@@ -194,28 +255,42 @@ class Phase6TrainStep:
         else:
             self.optimizer.zero_grad(set_to_none=True)
 
-    def _forward_loss(self, x, y_a, y_b, lam):
+    def _forward_loss(self, x, y_a, y_b, lam, lengths=None):
         dev = x.device.type
         with torch.autocast(dev, dtype=self.autocast_dtype, enabled=self.autocast_dtype is not None):
-            feats, out = self.model(x, **self.model_kwargs)
+            if lengths is None:
+                feats, out = self.model(x, **self.model_kwargs)
+            else:
+                feats, out = self.model(x, lengths, mask_padding=True, **self.model_kwargs)
             loss = mixup_loss(self.loss_fn, out, feats, y_a, y_b, lam)
         return loss / self.accumulation_steps
 
     def __call__(self, micro_batches: Iterable, generator: Optional[torch.Generator] = None, lam: Optional[float] = None):
-        """micro_batches: iterable of (x, y) of length accumulation_steps.  Returns the mean (un-divided) clean loss of the
-        micro-batches as a 0-d tensor (no host sync)."""
+        """micro_batches: iterable of (x, y) or (x, y, lengths) of length accumulation_steps.  With lengths (per-utterance
+        frame counts of the right-padded x, see ops.seqlens_tensor) the batch is mixed on its own frames (mixup_batch)
+        and both the clean and FGM's adversarial pass call model(x, mixed_lengths, mask_padding=True).  Returns the mean
+        (un-divided) clean loss of the micro-batches as a 0-d tensor (no host sync)."""
         self.model.train()
         if self.freeze_bn:
             freeze_batch_norm_stats(self.model)
         total = None
-        for x, y in micro_batches:
-            y = y.view(-1).long()
-            mx, y_a, y_b, lam_i = mixup_batch(x, y, self.mixup_alpha, generator, lam) if self.mixup_alpha > 0 else (x, y, y, 1.0)
-            loss = self._forward_loss(mx, y_a, y_b, lam_i)
+        for mb in micro_batches:
+            x, y = mb[0], mb[1].view(-1).long()
+            lengths = mb[2] if len(mb) > 2 else None
+            if lengths is not None and x.is_cuda:
+                from .ops import seqlens_tensor
+                lengths = seqlens_tensor(lengths, x.size(0), x.size(1), x.device)
+            if self.mixup_alpha > 0:
+                mixed = mixup_batch(x, y, self.mixup_alpha, generator, lam, lengths)
+                mx, y_a, y_b, lam_i = mixed[:4]
+                lengths = mixed[4] if lengths is not None else None
+            else:
+                mx, y_a, y_b, lam_i = x, y, y, 1.0
+            loss = self._forward_loss(mx, y_a, y_b, lam_i, lengths)
             self.scaler.scale(loss).backward()                                        # main.py:1077
             if self.fgm is not None:                                                  # main.py:1080-1098
                 self.fgm.attack()
-                adv = self._forward_loss(mx, y_a, y_b, lam_i)
+                adv = self._forward_loss(mx, y_a, y_b, lam_i, lengths)
                 self.scaler.scale(adv).backward()
                 self.fgm.restore()
             total = loss.detach() if total is None else total + loss.detach()
